@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py -- headline benchmark of the LiDAR front-end hot path (see DESIGN.md "Measurement").
 
-  python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference]
+  python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--dump-outputs DIR]
 
 Metric (BASELINE.json): NDT scan-to-map aligns per second, 120 000-point 64-beam sweep against a 1 000 000-point
 local map (configs[0]: DIRECT7, 1.0 m, step 0.1, eps 0.01, max_iter 64), synthetic data (SURVEY.md section 8d).
@@ -21,8 +21,16 @@ under "loop_closure".
 
 --impl reference times the reference's CPU path (the oracle port: the reference cannot be compiled here) on the
 same workload with all host threads.
+
+--dump-outputs DIR writes what the last timed step returned to its caller as DIR/<name>.npy (float32 / float64), so that
+two builds can be compared output for output on identical inputs (the workload is seeded):
+  final_transformation (4x4 f32), fitness_score, transformation_probability, align_counts (iterations, converged,
+  derivative evaluations, line-search trials, computeHessian calls)   the headline path (sweep resident in HBM)
+  e2e_<same names>, e2e_aligned_cloud (n_source x 4 f32)              the e2e path (host buffers)
+--impl reference writes the headline names and aligned_cloud.
 """
 import argparse
+import atexit
 import json
 import os
 import subprocess
@@ -72,6 +80,7 @@ class ClockSampler:
         try:
             self.proc = subprocess.Popen(["nvidia-smi", "-i", str(self.gpu), "--query-gpu=" + self.Q, "--format=csv,noheader,nounits", "-lms", "100"],
                                          stdout=subprocess.PIPE, stderr=subprocess.DEVNULL, text=True)
+            atexit.register(self._kill)  # the sampler must not outlive a benchmark that fails before stop()
             self.thread = threading.Thread(target=self._read, daemon=True)
             self.thread.start()
         except Exception:
@@ -80,6 +89,11 @@ class ClockSampler:
     def _read(self):
         for line in self.proc.stdout:
             self.rows.append([c.strip() for c in line.split(",")])
+
+    def _kill(self):
+        if self.proc and self.proc.poll() is None:
+            self.proc.kill()
+            self.proc.wait()
 
     def stop(self):
         if not self.proc:
@@ -129,6 +143,21 @@ def measured_peak_hbm():
             return float(json.load(f)["hbm_gbs"]), "measured (MEASURED_PEAKS.json hbm_gbs)"
     except Exception:
         return 6650.0, "fallback (B200_PROFILING.md 6.65 TB/s)"
+
+
+def ndt_outputs(ndt, counts, prefix=""):
+    """What the caller of one NDT align receives (the product's and the oracle's NDT share these getters).  `counts`:
+    iterations, converged, derivative evaluations, line-search trials, computeHessian calls."""
+    return {prefix + "final_transformation": np.array(ndt.getFinalTransformation(), np.float32),
+            prefix + "fitness_score": np.array([ndt.getFitnessScore()], np.float64),
+            prefix + "transformation_probability": np.array([ndt.getTransformationProbability()], np.float64),
+            prefix + "align_counts": np.array(counts, np.float64)}
+
+
+def write_outputs(directory, arrays):
+    os.makedirs(directory, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(directory, name + ".npy"), a)
 
 
 def cpu_baseline(target, sweeps, guesses, budget_s=20.0, threads=0):
@@ -183,18 +212,21 @@ def run_reference(args, rank, world):
     t0 = time.perf_counter()
     n.align(guesses[0])
     t_one = time.perf_counter() - t0
-    # bound the whole run to a few minutes: a step is one align; cap the step count by a time budget
-    budget = float(os.environ.get("LGS_REF_BUDGET_S", 150))
     warm = min(args.warmup, 1 if t_one > 5 else args.warmup)
-    steps = int(max(1, min(args.steps, budget / max(t_one, 1e-3))))
+    steps = max(1, args.steps)
     for w in range(max(0, warm - 1)):
         n.setInputSource(sweeps[w % len(sweeps)])
         n.align(guesses[w % len(sweeps)])
     t0 = time.perf_counter()
     for s in range(steps):
         n.setInputSource(sweeps[s % len(sweeps)])
-        n.align(guesses[s % len(sweeps)])
+        aligned = n.align(guesses[s % len(sweeps)])
     dt = time.perf_counter() - t0
+    if args.dump_outputs:
+        st = n.stats
+        out = ndt_outputs(n, (n.nr_iterations, n.converged, st["derivative_evals"], st["line_search_trials"], st["hessian_recomputes"]))
+        out["aligned_cloud"] = aligned
+        write_outputs(args.dump_outputs, out)
     val = steps / dt
     line = {"impl": "reference", "metric": "ndt_scan_to_map_aligns_per_sec", "value": val, "unit": "aligns/s", "n_gpus": args.gpus, "steps": steps,
             "warmup": warm, "ms_per_step": 1e3 * dt / steps, "higher_is_better": True, "scaling": "weak", "vs_baseline": None, "dtype": "f32",
@@ -438,6 +470,7 @@ def main():
     ap.add_argument("--odometry-sweeps", type=int, default=_env_int("LGS_BENCH_ODOMETRY_SWEEPS", 1000), help="configs[2]: sweeps of the GICP odometry run (0 disables)")
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-big-map", action="store_true", help="skip configs[3] (20 M-point map)")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write what the last timed step returned as DIR/<name>.npy (rank 0)")
     args = ap.parse_args()
     rank, world, local_rank = _env_int("RANK", 0), _env_int("WORLD_SIZE", 1), _env_int("LOCAL_RANK", 0)
 
@@ -498,6 +531,10 @@ def main():
         ndt.align(guesses[i % len(guesses)], want_output=True, out=aligned_pinned.numpy())
         return ndt.getFinalTransformation()
 
+    def last_step_outputs(prefix):
+        r = ndt.result
+        return ndt_outputs(ndt, (r.iterations, r.converged, r.evaluations, r.line_search_trials, r.hessian_recomputes), prefix)
+
     def timed(fn, steps, warm):
         for i in range(warm):
             fn(i)
@@ -529,8 +566,15 @@ def main():
     ndt.profile(2)
     per_dev, launches, evals_dev = timed(step_dev, K, W)
     prof = ndt.profile(0)
+    dump = rank == 0 and args.dump_outputs
+    outputs = last_step_outputs("") if dump else {}
     per_host, _, evals_host = timed(step_host, K, W)
+    if dump:
+        outputs.update(last_step_outputs("e2e_"))
+        outputs["e2e_aligned_cloud"] = aligned_pinned.numpy()[:len(sweeps[(K - 1) % len(sweeps)])].copy()
     clocks = sampler.stop() if rank == 0 else None
+    if dump:
+        write_outputs(args.dump_outputs, outputs)
     ms_dev, ms_host = float(per_dev.sum()), float(per_host.sum())
 
     # accuracy sanity of the timed workload (not a parity test: those live in tests/)

@@ -8,6 +8,7 @@ counter-based generator keyed by (seed, frame, ray); returns closer than 1 m or 
 """
 import hashlib
 import os
+import tempfile
 
 import numpy as np
 
@@ -197,7 +198,8 @@ def trajectory_pose(k, spacing=1.0):
 
 
 def _cache_dir():
-    d = os.environ.get("LGS_SYNTH_CACHE", "/tmp/lgs_synth_cache")
+    # one directory per user: the temporary directory is shared, and a cache another account created there is not writable
+    d = os.environ.get("LGS_SYNTH_CACHE") or os.path.join(tempfile.gettempdir(), "lgs_synth_cache_%d" % os.getuid())
     os.makedirs(d, exist_ok=True)
     return d
 
@@ -213,8 +215,11 @@ def _cached(name, params, fn):
             pass
     out = fn()
     tmp = path + ".tmp%d.npz" % os.getpid()
-    np.savez(tmp, **out)
-    os.replace(tmp, path)
+    try:
+        np.savez(tmp, **out)
+        os.replace(tmp, path)
+    except OSError:  # the cache only saves time: a full or read-only disk must not fail the run
+        pass
     return out
 
 
