@@ -273,6 +273,14 @@ class _Registration:
 
     _prefix = ""
 
+    def __init__(self, ctx=None):
+        self.ctx = ctx or default_context()
+        self._L = self.ctx._L
+        h = C.c_void_p()
+        check(self._fn("create")(self.ctx._h, C.byref(h)))
+        self._h = h
+        self._ns = self._nt = 0
+
     def _fn(self, name):
         return getattr(self._L, "lgs_%s_%s" % (self._prefix, name))
 
@@ -335,12 +343,7 @@ class NormalDistributionsTransform(_Registration):
     _prefix = "ndt"
 
     def __init__(self, ctx=None):
-        self.ctx = ctx or default_context()
-        self._L = self.ctx._L
-        h = C.c_void_p()
-        check(self._L.lgs_ndt_create(self.ctx._h, C.byref(h)))
-        self._h = h
-        self._ns = self._nt = 0
+        super().__init__(ctx)
         self._resolution, self._step, self._outlier = 1.0, 0.1, 0.55
 
     def setResolution(self, r): check(self._L.lgs_ndt_set_resolution(self._h, float(r))); self._resolution = float(r)
@@ -436,14 +439,6 @@ class FastGICP(_Registration):
 
     _prefix = "gicp"
 
-    def __init__(self, ctx=None):
-        self.ctx = ctx or default_context()
-        self._L = self.ctx._L
-        h = C.c_void_p()
-        check(self._L.lgs_gicp_create(self.ctx._h, C.byref(h)))
-        self._h = h
-        self._ns = self._nt = 0
-
     def setCorrespondenceRandomness(self, k): check(self._L.lgs_gicp_set_correspondence_randomness(self._h, int(k)))
     def setMaxCorrespondenceDistance(self, d): check(self._L.lgs_gicp_set_max_correspondence_distance(self._h, float(d)))
     def setTransformationEpsilon(self, e): check(self._L.lgs_gicp_set_transformation_epsilon(self._h, float(e)))
@@ -503,14 +498,6 @@ class GeneralizedIterativeClosestPoint(_Registration):
     """pclomp::GeneralizedIterativeClosestPoint (gicp_omp.h:116-270; BFGS), the "GICP" method of LSM:73-96 / GBS:120-141."""
 
     _prefix = "gicp_omp"
-
-    def __init__(self, ctx=None):
-        self.ctx = ctx or default_context()
-        self._L = self.ctx._L
-        h = C.c_void_p()
-        check(self._L.lgs_gicp_omp_create(self.ctx._h, C.byref(h)))
-        self._h = h
-        self._ns = self._nt = 0
 
     def setCorrespondenceRandomness(self, k): check(self._L.lgs_gicp_omp_set_correspondence_randomness(self._h, int(k)))
     def setMaxCorrespondenceDistance(self, d): check(self._L.lgs_gicp_omp_set_max_correspondence_distance(self._h, float(d)))
@@ -600,14 +587,9 @@ class KeyFrameArray:
         cid = np.ascontiguousarray(center_ids, np.int32)
         n = int(sid.size)
         assert cid.size == n
-        g = None
-        if guesses is not None:
-            g = np.ascontiguousarray(np.stack([np.asarray(T, np.float32).reshape(4, 4).ravel(order="F") for T in guesses]))
-        bp = BatchParams(method=method, max_iterations=max_iterations, transformation_epsilon=transformation_epsilon,
-                         max_correspondence_distance=max_correspondence_distance, k_correspondences=k_correspondences,
-                         ndt_resolution=ndt_resolution, ndt_step_size=ndt_step_size, submap_leaf=submap_leaf,
-                         fitness_max_range=fitness_max_range, n_workers=n_workers, max_optimizer_iterations=max_optimizer_iterations,
-                         euclidean_fitness_epsilon=euclidean_fitness_epsilon)
+        g = _pack_guesses(guesses)
+        bp = _batch_params(method, max_iterations, transformation_epsilon, max_correspondence_distance, k_correspondences, ndt_resolution,
+                           ndt_step_size, submap_leaf, fitness_max_range, n_workers, max_optimizer_iterations, euclidean_fitness_epsilon)
         recs = (AlignResult * max(n, 1))()
         vp = lambda a: a.ctypes.data_as(C.c_void_p)
         check(self._L.lgs_batch_align_keyframes(self._h, None, C.byref(bp), n, vp(sid), vp(cid), int(search_key_frame_num),
@@ -623,9 +605,7 @@ class KeyFrameArray:
         cid = np.ascontiguousarray(center_ids, np.int32)
         n = int(sid.size)
         assert cid.size == n
-        g = None
-        if guesses is not None:
-            g = np.ascontiguousarray(np.stack([np.asarray(T, np.float32).reshape(4, 4).ravel(order="F") for T in guesses]))
+        g = _pack_guesses(guesses)
         bp = _batch_params(method, max_iterations, transformation_epsilon, max_correspondence_distance, k_correspondences, ndt_resolution,
                            ndt_step_size, submap_leaf, fitness_max_range, n_workers, max_optimizer_iterations, euclidean_fitness_epsilon)
         recs = (AlignResult * max(n, 1))()
@@ -661,14 +641,6 @@ class IterativeClosestPoint(_Registration):
     """pcl::IterativeClosestPoint<PointXYZI, PointXYZI>, the graph SLAM node's default loop-closure method (GBS:142-151)."""
 
     _prefix = "icp"
-
-    def __init__(self, ctx=None):
-        self.ctx = ctx or default_context()
-        self._L = self.ctx._L
-        h = C.c_void_p()
-        check(self._L.lgs_icp_create(self.ctx._h, C.byref(h)))
-        self._h = h
-        self._ns = self._nt = 0
 
     def setMaxCorrespondenceDistance(self, d): check(self._L.lgs_icp_set_max_correspondence_distance(self._h, float(d)))
     def setMaximumIterations(self, n): check(self._L.lgs_icp_set_maximum_iterations(self._h, int(n)))
@@ -721,19 +693,21 @@ def batch_align(scans, submaps, method=METHOD_GICP, guesses=None, device=0, stre
     mp = (C.c_void_p * n)(*[s.ctypes.data for s in sm])
     ns = (C.c_int64 * n)(*[s.shape[0] for s in sc])
     nm = (C.c_int64 * n)(*[s.shape[0] for s in sm])
-    g = None
-    if guesses is not None:
-        g = np.ascontiguousarray(np.stack([np.asarray(T, np.float32).reshape(4, 4).ravel(order="F") for T in guesses]))
-    bp = BatchParams(method=method, max_iterations=max_iterations, transformation_epsilon=transformation_epsilon,
-                     max_correspondence_distance=max_correspondence_distance, k_correspondences=k_correspondences,
-                     ndt_resolution=ndt_resolution, ndt_step_size=ndt_step_size, submap_leaf=submap_leaf,
-                     fitness_max_range=fitness_max_range, n_workers=n_workers, max_optimizer_iterations=max_optimizer_iterations,
-                     euclidean_fitness_epsilon=euclidean_fitness_epsilon)
+    g = _pack_guesses(guesses)
+    bp = _batch_params(method, max_iterations, transformation_epsilon, max_correspondence_distance, k_correspondences, ndt_resolution, ndt_step_size,
+                       submap_leaf, fitness_max_range, n_workers, max_optimizer_iterations, euclidean_fitness_epsilon)
     recs = (AlignResult * max(n, 1))()
     check(L.lgs_batch_align(int(device), C.c_void_p(stream) if stream else None, C.byref(bp), n, sp, ns, mp, nm, 16,
                             g.ctypes.data_as(C.c_void_p) if g is not None else None, int(pair_id0), recs,
                             C.c_void_p(records_dev) if records_dev else None))
     return [recs[i] for i in range(n)]
+
+
+def _pack_guesses(guesses):
+    """(K, 16) float32 column-major transforms, or None."""
+    if guesses is None:
+        return None
+    return np.ascontiguousarray(np.stack([np.asarray(T, np.float32).reshape(4, 4).ravel(order="F") for T in guesses]))
 
 
 def _batch_params(method, max_iterations, transformation_epsilon, max_correspondence_distance, k_correspondences, ndt_resolution, ndt_step_size,
@@ -850,9 +824,7 @@ def batch_align_dist(comm, scans, submaps, method=METHOD_GICP, guesses=None, max
         sizes = [(a.shape[0], b.shape[0]) for a, b in zip(sc, sm)]
     ns = (C.c_int64 * max(n, 1))(*[int(a) for a, _ in sizes])
     nm = (C.c_int64 * max(n, 1))(*[int(b) for _, b in sizes])
-    g = None
-    if guesses is not None:
-        g = np.ascontiguousarray(np.stack([np.asarray(T, np.float32).reshape(4, 4).ravel(order="F") for T in guesses]))
+    g = _pack_guesses(guesses)
     bp = _batch_params(method, max_iterations, transformation_epsilon, max_correspondence_distance, k_correspondences, ndt_resolution, ndt_step_size,
                        submap_leaf, fitness_max_range, n_workers, max_optimizer_iterations, euclidean_fitness_epsilon)
     recs = (AlignResult * max(n, 1))()

@@ -161,8 +161,16 @@ inline int use_device(const lgs_ctx* c) {
 
 // Upload a host cloud with arbitrary record stride into packed float4 xyzi device storage.
 int upload_cloud(lgs_ctx* ctx, const void* pts, int64_t n, int32_t stride_bytes, DevBuf* dst);
-// Copy an already packed device cloud into dst (device to device).
-int adopt_cloud_dev(lgs_ctx* ctx, const float* pts_dev, int64_t n, DevBuf* dst);
+// The input of every registration set_source / set_target entry point, validated on the host before anything is copied:
+// host records of stride_bytes each (as upload_cloud) or, on_device, a packed float4 xyzi device array (copied device to
+// device; stride_bytes unused).  pts may be null only when n == 0.
+int load_cloud(lgs_ctx* ctx, const void* pts, int64_t n, int32_t stride_bytes, bool on_device, DevBuf* dst);
+
+// dst = T * src as pcl::transformPointCloud (intensity kept); T column-major
+int transform_cloud(lgs_ctx* ctx, const float4* src, int64_t n, const float* T, float4* dst);
+// The aligned source cloud of align(output, guess): T * src through the device buffer scratch into out_host (n x 4 floats),
+// waited for.  Nothing to do when n == 0.
+int write_aligned_cloud(lgs_ctx* ctx, const float4* src, int64_t n, const float* T, DevBuf* scratch, float* out_host);
 
 // Next mailbox token + kernel argument; mailbox_wait spins until the kernel has published k records with that token
 // (checking the stream for errors now and then) and copies the values to out.

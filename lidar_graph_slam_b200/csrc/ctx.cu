@@ -1,4 +1,4 @@
-// Context, error reporting and cloud upload (host AoS records -> packed float4 xyzi in HBM).
+// Context, error reporting, cloud upload (host AoS records -> packed float4 xyzi in HBM) and the aligned output cloud.
 #include <atomic>
 
 #include <cstdlib>
@@ -53,10 +53,44 @@ int upload_cloud(lgs_ctx* ctx, const void* pts, int64_t n, int32_t stride, DevBu
   return LGS_OK;
 }
 
-int adopt_cloud_dev(lgs_ctx* ctx, const float* pts_dev, int64_t n, DevBuf* dst) {
+int load_cloud(lgs_ctx* ctx, const void* pts, int64_t n, int32_t stride_bytes, bool on_device, DevBuf* dst) {
+  LGS_TRY(use_device(ctx));
+  if (!on_device) return upload_cloud(ctx, pts, n, stride_bytes, dst);
   LGS_REQUIRE(n >= 0, "negative point count");
+  LGS_REQUIRE(n == 0 || pts != nullptr, "null cloud");
   LGS_TRY(dst->reserve(static_cast<size_t>(n > 0 ? n : 1) * 16));
-  if (n) LGS_CUDA(cudaMemcpyAsync(dst->p, pts_dev, static_cast<size_t>(n) * 16, cudaMemcpyDeviceToDevice, ctx->stream));
+  if (n) LGS_CUDA(cudaMemcpyAsync(dst->p, pts, static_cast<size_t>(n) * 16, cudaMemcpyDeviceToDevice, ctx->stream));
+  return LGS_OK;
+}
+
+struct Mat4f {  // a transform passed by value (64 bytes of kernel parameters), column-major
+  float m[16];
+};
+
+__global__ void __launch_bounds__(256) transform_cloud_kernel(const float4* __restrict__ src, int64_t n, Mat4f T, float4* __restrict__ dst) {
+  const int64_t i = blockIdx.x * static_cast<int64_t>(blockDim.x) + threadIdx.x;
+  if (i >= n) return;
+  const float4 p = src[i];
+  const float3 t = transform_pcl(T.m, p.x, p.y, p.z);
+  dst[i] = make_float4(t.x, t.y, t.z, p.w);
+}
+
+int transform_cloud(lgs_ctx* ctx, const float4* src, int64_t n, const float* T, float4* dst) {
+  if (n == 0) return LGS_OK;
+  Mat4f m;
+  memcpy(m.m, T, sizeof(m.m));
+  transform_cloud_kernel<<<grid_for(n, 256), 256, 0, ctx->stream>>>(src, n, m, dst);
+  ctx->launches++;
+  LGS_CUDA(cudaGetLastError());
+  return LGS_OK;
+}
+
+int write_aligned_cloud(lgs_ctx* ctx, const float4* src, int64_t n, const float* T, DevBuf* scratch, float* out_host) {
+  if (n == 0) return LGS_OK;
+  LGS_TRY(scratch->reserve(static_cast<size_t>(n) * 16));
+  LGS_TRY(transform_cloud(ctx, src, n, T, scratch->as<float4>()));
+  LGS_CUDA(cudaMemcpyAsync(out_host, scratch->p, static_cast<size_t>(n) * 16, cudaMemcpyDeviceToHost, ctx->stream));
+  LGS_CUDA(cudaStreamSynchronize(ctx->stream));
   return LGS_OK;
 }
 

@@ -338,18 +338,6 @@ __global__ void __launch_bounds__(kLinBlock) gicp_error_kernel(const float4* __r
   lin_block_reduce_and_finish<1>(acc, partials, result, counter, mb);
 }
 
-__global__ void __launch_bounds__(256) gicp_transform_cloud_kernel(const float4* __restrict__ src, int64_t n, const float* __restrict__ Tdev,
-                                                                  float4* __restrict__ out) {
-  __shared__ float T[16];
-  if (threadIdx.x < 16) T[threadIdx.x] = Tdev[threadIdx.x];
-  __syncthreads();
-  int64_t i = blockIdx.x * static_cast<int64_t>(blockDim.x) + threadIdx.x;
-  if (i >= n) return;
-  float4 p = src[i];
-  float3 t = transform_pcl(T, p.x, p.y, p.z);
-  out[i] = make_float4(t.x, t.y, t.z, p.w);
-}
-
 }  // namespace lgs
 
 // =============================================================================================
@@ -552,8 +540,7 @@ int step_lm(lgs_gicp* g, double* x0, double* delta, bool* ok) {
   return LGS_OK;
 }
 
-int set_cloud(lgs_gicp* g, std::shared_ptr<GicpCloud>* slot, const void* pts, const float* pts_dev, int64_t n, int32_t stride) {
-  LGS_TRY(use_device(g->ctx));
+int set_cloud(lgs_gicp* g, std::shared_ptr<GicpCloud>* slot, const void* pts, int64_t n, int32_t stride, bool on_device) {
   // a bundle nobody else holds (no swap partner, no exported alias) is recycled with its device buffers: steady-state
   // calls never reach cudaMalloc / cudaFree, which would serialise every stream of the device
   std::shared_ptr<GicpCloud> c;
@@ -566,10 +553,7 @@ int set_cloud(lgs_gicp* g, std::shared_ptr<GicpCloud>* slot, const void* pts, co
   } else {
     c = std::make_shared<GicpCloud>();
   }
-  if (pts_dev)
-    LGS_TRY(adopt_cloud_dev(g->ctx, pts_dev, n, &c->pts));
-  else
-    LGS_TRY(upload_cloud(g->ctx, pts, n, stride, &c->pts));
+  LGS_TRY(load_cloud(g->ctx, pts, n, stride, on_device, &c->pts));
   c->n = n;
   *slot = c;
   return LGS_OK;
@@ -660,19 +644,19 @@ int lgs_gicp_set_initial_lambda_factor(lgs_gicp* g, double f) { LGS_REQUIRE(g, "
 
 int lgs_gicp_set_source(lgs_gicp* g, const void* pts, int64_t n, int32_t stride) {
   LGS_REQUIRE(g, "null");
-  return set_cloud(g, &g->source, pts, nullptr, n, stride);
+  return set_cloud(g, &g->source, pts, n, stride, false);
 }
 int lgs_gicp_set_target(lgs_gicp* g, const void* pts, int64_t n, int32_t stride) {
   LGS_REQUIRE(g, "null");
-  return set_cloud(g, &g->target, pts, nullptr, n, stride);
+  return set_cloud(g, &g->target, pts, n, stride, false);
 }
 int lgs_gicp_set_source_dev(lgs_gicp* g, const float* pts_dev, int64_t n) {
-  LGS_REQUIRE(g && (pts_dev || n == 0), "null");
-  return set_cloud(g, &g->source, nullptr, pts_dev ? pts_dev : reinterpret_cast<const float*>(g), n, 16);
+  LGS_REQUIRE(g, "null");
+  return set_cloud(g, &g->source, pts_dev, n, 16, true);
 }
 int lgs_gicp_set_target_dev(lgs_gicp* g, const float* pts_dev, int64_t n) {
-  LGS_REQUIRE(g && (pts_dev || n == 0), "null");
-  return set_cloud(g, &g->target, nullptr, pts_dev ? pts_dev : reinterpret_cast<const float*>(g), n, 16);
+  LGS_REQUIRE(g, "null");
+  return set_cloud(g, &g->target, pts_dev, n, 16, true);
 }
 int lgs_gicp_swap_source_and_target(lgs_gicp* g) {  // FG:50-57: clouds, trees and covariances travel together
   LGS_REQUIRE(g, "null");
@@ -686,19 +670,7 @@ int lgs_gicp_align(lgs_gicp* g, const float* guess16, lgs_align_result* res, flo
   LGS_NVTX("lgs_gicp_align");
   LGS_REQUIRE(g && res, "null argument");
   LGS_TRY(gicp_align_impl(g, guess16, res));
-  if (out_cloud && g->source->n) {  // LSQ:77-78
-    cudaStream_t st = g->ctx->stream;
-    const int64_t n = g->source->n;
-    LGS_TRY(g->out_cloud.reserve(static_cast<size_t>(n) * 16 + 64));
-    float* Tdev = reinterpret_cast<float*>(g->out_cloud.as<char>() + static_cast<size_t>(n) * 16);
-    LGS_TRY(g->ctx->pin_up.reserve(64));
-    memcpy(g->ctx->pin_up.p, g->final_T, 64);
-    LGS_CUDA(cudaMemcpyAsync(Tdev, g->ctx->pin_up.p, 64, cudaMemcpyHostToDevice, st));
-    gicp_transform_cloud_kernel<<<grid_for(n, 256), 256, 0, st>>>(g->source->pts.as<float4>(), n, Tdev, g->out_cloud.as<float4>());
-    g->ctx->launches++;
-    LGS_CUDA(cudaMemcpyAsync(out_cloud, g->out_cloud.p, static_cast<size_t>(n) * 16, cudaMemcpyDeviceToHost, st));
-    LGS_CUDA(cudaStreamSynchronize(st));
-  }
+  if (out_cloud) LGS_TRY(write_aligned_cloud(g->ctx, g->source->pts.as<float4>(), g->source->n, g->final_T, &g->out_cloud, out_cloud));  // LSQ:77-78
   return LGS_OK;
 }
 

@@ -257,17 +257,15 @@ struct PgicpPose {
   int pad;
   unsigned long long token;
 };
-constexpr int kPgWords = static_cast<int>(sizeof(PgicpPose) / 8);
-static_assert(sizeof(PgicpPose) % 8 == 0, "commands are copied as 64-bit words");
-using PgicpCmdHost = CmdHost<kPgWords>;
-using PgicpCmdDev = CmdDev<kPgWords>;
+using PgicpSession = ResidentSession<PgicpPose>;
+constexpr int kPgWords = PgicpSession::kWords;
 constexpr int kFunResident = 4;  // CTAs of the persistent grid per SM (all of them must be co-resident)
 
 __global__ void __launch_bounds__(kFunBlock, kFunResident) pgicp_persistent_kernel(const float4* __restrict__ out_cloud, const float4* __restrict__ tgt, int n,
                                                                                   const int* __restrict__ corr, const float* __restrict__ mahal,
                                                                                   Fix128* __restrict__ partials, unsigned* __restrict__ counter,
-                                                                                  MailboxRecord* mailbox, const PgicpCmdHost* __restrict__ cmd_host,
-                                                                                  PgicpCmdDev* __restrict__ cmd_dev, unsigned long long first_seq) {
+                                                                                  MailboxRecord* mailbox, const PgicpSession::Host* __restrict__ cmd_host,
+                                                                                  PgicpSession::Dev* __restrict__ cmd_dev, unsigned long long first_seq) {
   __shared__ __align__(16) PgicpPose pose;
   __shared__ int give_up;
   if (threadIdx.x == 0) give_up = 0;
@@ -286,14 +284,6 @@ __global__ void __launch_bounds__(kFunBlock, kFunResident) pgicp_persistent_kern
       pgicp_functor_body<2>(out_cloud, tgt, n, pose.T, corr, mahal, partials, counter, mb);
     __syncthreads();
   }
-}
-
-__global__ void __launch_bounds__(256) pgicp_transform_kernel(const float4* __restrict__ src, int64_t n, PgicpParams P, float4* __restrict__ out) {
-  const int64_t i = blockIdx.x * static_cast<int64_t>(blockDim.x) + threadIdx.x;
-  if (i >= n) return;
-  const float4 p = src[i];
-  const float3 t = transform_pcl(P.T, p.x, p.y, p.z);
-  out[i] = make_float4(t.x, t.y, t.z, p.w);
 }
 
 }  // namespace lgs
@@ -315,26 +305,10 @@ struct lgs_gicp_omp {
   float base_T[16], T[16], prev_T[16], final_T[16], guess[16];
   int n_corr = 0;
   int f_calls = 0, df_calls = 0, fdf_calls = 0, inner_total = 0;
-  // persistent functor evaluator (between two update_correspondences calls of one align)
-  bool allow_session = false, session_active = false, session_broken = false;
-  int session_device = -1;
-  PgicpCmdHost* cmd_host = nullptr;  // mapped pinned memory
-  DevBuf cmd_dev;
-  unsigned long long cmd_seq = 0;
+  PgicpSession session{PgicpPose{{}, -1, 0, 0}};  // persistent functor evaluator (between two update_correspondences calls of one align)
 };
 
 namespace {
-
-void identity16f(float* T) {
-  for (int i = 0; i < 16; i++) T[i] = (i % 5 == 0) ? 1.0f : 0.0f;
-}
-
-void mul4f(const float* A, const float* B, float* C) {  // column-major, ((a0 b0 + a1 b1) + a2 b2) + a3 b3
-  float R[16];
-  for (int c = 0; c < 4; c++)
-    for (int r = 0; r < 4; r++) R[c * 4 + r] = ((A[r] * B[c * 4] + A[4 + r] * B[c * 4 + 1]) + A[8 + r] * B[c * 4 + 2]) + A[12 + r] * B[c * 4 + 3];
-  memcpy(C, R, sizeof(R));
-}
 
 // applyState (GO:518-529): t <- [Rz(x5) Ry(x4) Rx(x3) * t.linear | t.translation + x0..2], the rotation composed through
 // f32 quaternions as Eigen's AngleAxisf products do
@@ -391,31 +365,6 @@ void r_derivative(const double* x, const double* R, double* g) {
 // one row of partial sums per CTA goes through the last-CTA pass: no more CTAs than SMs (a 30 000-point cloud is 1.6 points per thread)
 int fun_grid(int64_t n) { return std::max(1, std::min(grid_for(n, kFunBlock), kNumSMs)); }
 
-void end_session(lgs_gicp_omp* g) {
-  if (!g->session_active) return;
-  PgicpPose quit;
-  memset(&quit, 0, sizeof(quit));
-  quit.mode = -1;
-  persist_send<kPgWords>(g->cmd_host, ++g->cmd_seq, &quit);
-  g->session_active = false;
-  persist_release(g->session_device);
-}
-
-// everything the session needs that may allocate or synchronise, before the grid becomes resident
-int prepare_session(lgs_gicp_omp* g) {
-  if (!g->cmd_host) {
-    void* p = nullptr;
-    LGS_CUDA(cudaHostAlloc(&p, sizeof(PgicpCmdHost), cudaHostAllocMapped | cudaHostAllocPortable));
-    memset(p, 0, sizeof(PgicpCmdHost));
-    g->cmd_host = static_cast<PgicpCmdHost*>(p);
-  }
-  if (!g->cmd_dev.p) {
-    LGS_TRY(g->cmd_dev.reserve(sizeof(PgicpCmdDev)));
-    LGS_CUDA(cudaMemsetAsync(g->cmd_dev.p, 0, sizeof(PgicpCmdDev), g->ctx->stream));
-  }
-  return LGS_OK;
-}
-
 // one functor evaluation on the device: mode 0 -> f; 1 -> g; 2 -> f and g
 int functor_eval(lgs_gicp_omp* g, const double* x, int mode, double* f, double* grad) {
   lgs_ctx* ctx = g->ctx;
@@ -433,40 +382,22 @@ int functor_eval(lgs_gicp_omp* g, const double* x, int mode, double* f, double* 
   const int grid = fun_grid(n);
   double h[kMailboxRecords];
   const int K = mode == 0 ? 1 : (mode == 1 ? 12 : 13);
-  const bool want_session = g->allow_session && !g->session_broken && persist_env_enabled() && grid <= kNumSMs * kFunResident;
-  if (!want_session) end_session(g);
-  if (want_session && !g->session_active) {
-    LGS_TRY(prepare_session(g));
-    if (persist_try_acquire(ctx->device)) {
-      void* dv = nullptr;
-      LGS_CUDA(cudaHostGetDevicePointer(&dv, g->cmd_host, 0));
-      pgicp_persistent_kernel<<<grid, kFunBlock, 0, ctx->stream>>>(out, tgt, n, g->corr.as<int>(), g->mahal.as<float>(), partials, counter, mb.r,
-                                                                 static_cast<const PgicpCmdHost*>(dv), g->cmd_dev.as<PgicpCmdDev>(), g->cmd_seq + 1);
-      ctx->launches++;
-      cudaError_t le = cudaGetLastError();
-      if (le != cudaSuccess) {
-        persist_release(ctx->device);
-        set_error("pgicp_persistent_kernel launch failed: %s", cudaGetErrorString(le));
-        return LGS_ERR_CUDA;
-      }
-      g->session_active = true;
-      g->session_device = ctx->device;
-    }
-  }
-  if (g->session_active) {
+  LGS_TRY(g->session.open(ctx, grid <= kNumSMs * kFunResident, [&](const PgicpSession::Host* host, PgicpSession::Dev* dev, unsigned long long first_seq) {
+    pgicp_persistent_kernel<<<grid, kFunBlock, 0, ctx->stream>>>(out, tgt, n, g->corr.as<int>(), g->mahal.as<float>(), partials, counter, mb.r, host, dev,
+                                                               first_seq);
+  }));
+  if (g->session.active) {
     PgicpPose pose;
     memcpy(pose.T, P.T, sizeof(pose.T));
     pose.mode = mode;
     pose.pad = 0;
     pose.token = mb.token;
-    persist_send<kPgWords>(g->cmd_host, ++g->cmd_seq, &pose);
+    g->session.send(pose);
     const int rc = mailbox_wait(ctx, mb, K, h);
     if (rc != LGS_OK) {
-      // the grid gave up (command time-out): if the stream is healthy, go on with one launch per evaluation
-      end_session(g);
-      if (cudaStreamSynchronize(ctx->stream) != cudaSuccess || cudaGetLastError() != cudaSuccess) return rc;
-      g->session_broken = true;
-      if (cudaMemsetAsync(counter, 0, sizeof(unsigned), ctx->stream) != cudaSuccess) return rc;
+      // the grid gave up (command time-out): the functor only reads, so if the stream is healthy this evaluation runs
+      // again with a plain launch, and so do the ones after it
+      if (!g->session.recover(ctx, counter)) return rc;
       (mode == 0 ? g->f_calls : mode == 1 ? g->df_calls : g->fdf_calls)--;
       return functor_eval(g, x, mode, f, grad);
     }
@@ -844,18 +775,11 @@ int ensure_ready(lgs_gicp_omp* g) {
 }
 
 // output = guess * source (GO:398)
-int transform_source(lgs_gicp_omp* g, const float* T, float4* dst) {
-  PgicpParams P;
-  memcpy(P.T, T, sizeof(P.T));
-  pgicp_transform_kernel<<<grid_for(g->source->n, 256), 256, 0, g->ctx->stream>>>(g->source->pts.as<float4>(), g->source->n, P, dst);
-  g->ctx->launches++;
-  LGS_CUDA(cudaGetLastError());
-  return LGS_OK;
-}
+int transform_source(lgs_gicp_omp* g) { return transform_cloud(g->ctx, g->source->pts.as<float4>(), g->source->n, g->guess, g->output.as<float4>()); }
 
 // the correspondence / Mahalanobis half of one outer iteration (GO:404-474); sets g->n_corr
 int update_correspondences(lgs_gicp_omp* g) {
-  end_session(g);  // the correspondence / Mahalanobis kernels need the SMs; the next functor call opens a new run
+  g->session.close();  // the correspondence / Mahalanobis kernels need the SMs; the next functor call opens a new run
   lgs_ctx* ctx = g->ctx;
   PgicpParams P;
   memcpy(P.T, g->T, sizeof(P.T));
@@ -881,16 +805,12 @@ int update_correspondences(lgs_gicp_omp* g) {
   return LGS_OK;
 }
 
-int set_cloud(lgs_gicp_omp* g, std::shared_ptr<GicpCloud>* slot, const void* pts, const float* pts_dev, int64_t n, int32_t stride) {
-  LGS_TRY(use_device(g->ctx));
+int set_cloud(lgs_gicp_omp* g, std::shared_ptr<GicpCloud>* slot, const void* pts, int64_t n, int32_t stride, bool on_device) {
   if (!*slot) *slot = std::make_shared<GicpCloud>();
   GicpCloud& c = **slot;
   c.nn_ready = false;
   c.covs_ready = false;  // GO.h:155,168: a new cloud drops its covariances
-  if (pts_dev)
-    LGS_TRY(adopt_cloud_dev(g->ctx, pts_dev, n, &c.pts));
-  else
-    LGS_TRY(upload_cloud(g->ctx, pts, n, stride, &c.pts));
+  LGS_TRY(load_cloud(g->ctx, pts, n, stride, on_device, &c.pts));
   c.n = n;
   return LGS_OK;
 }
@@ -910,11 +830,7 @@ int lgs_gicp_omp_create(lgs_ctx* ctx, lgs_gicp_omp** out) {
 
 void lgs_gicp_omp_destroy(lgs_gicp_omp* g) {
   if (!g) return;
-  end_session(g);
-  cudaSetDevice(g->ctx->device);
-  cudaStreamSynchronize(g->ctx->stream);
-  if (g->cmd_host) cudaFreeHost(g->cmd_host);
-  g->cmd_dev.release();
+  g->session.release(g->ctx);
   g->source.reset();
   g->target.reset();
   for (DevBuf* b : {&g->output, &g->corr, &g->mahal, &g->partials, &g->state, &g->out_cloud}) b->release();
@@ -935,35 +851,26 @@ int lgs_gicp_omp_set_maximum_optimizer_iterations(lgs_gicp_omp* g, int32_t n) { 
 
 int lgs_gicp_omp_set_source(lgs_gicp_omp* g, const void* pts, int64_t n, int32_t stride) {
   LGS_REQUIRE(g, "null");
-  return set_cloud(g, &g->source, pts, nullptr, n, stride);
+  return set_cloud(g, &g->source, pts, n, stride, false);
 }
 int lgs_gicp_omp_set_target(lgs_gicp_omp* g, const void* pts, int64_t n, int32_t stride) {
   LGS_REQUIRE(g, "null");
-  return set_cloud(g, &g->target, pts, nullptr, n, stride);
+  return set_cloud(g, &g->target, pts, n, stride, false);
 }
 int lgs_gicp_omp_set_source_dev(lgs_gicp_omp* g, const float* pts_dev, int64_t n) {
-  LGS_REQUIRE(g && (pts_dev || n == 0), "null");
-  return set_cloud(g, &g->source, nullptr, pts_dev ? pts_dev : reinterpret_cast<const float*>(g), n, 16);
+  LGS_REQUIRE(g, "null");
+  return set_cloud(g, &g->source, pts_dev, n, 16, true);
 }
 int lgs_gicp_omp_set_target_dev(lgs_gicp_omp* g, const float* pts_dev, int64_t n) {
-  LGS_REQUIRE(g && (pts_dev || n == 0), "null");
-  return set_cloud(g, &g->target, nullptr, pts_dev ? pts_dev : reinterpret_cast<const float*>(g), n, 16);
+  LGS_REQUIRE(g, "null");
+  return set_cloud(g, &g->target, pts_dev, n, 16, true);
 }
 
 // pcl::Registration::align + computeTransformation (GO:370-516)
-static int gicp_omp_align_body(lgs_gicp_omp* g, const float* guess16, lgs_align_result* res, float* out_cloud);
-
 int lgs_gicp_omp_align(lgs_gicp_omp* g, const float* guess16, lgs_align_result* res, float* out_cloud) {
   LGS_NVTX("lgs_gicp_omp_align");
   LGS_REQUIRE(g && res, "null argument");
-  g->allow_session = true;
-  const int rc = gicp_omp_align_body(g, guess16, res, out_cloud);
-  end_session(g);  // every exit path releases the resident grid
-  g->allow_session = false;
-  return rc;
-}
-
-static int gicp_omp_align_body(lgs_gicp_omp* g, const float* guess16, lgs_align_result* res, float* out_cloud) {
+  SessionScope scope(g->session);
   memset(res, 0, sizeof(*res));
   LGS_TRY(use_device(g->ctx));
   LGS_TRY(ensure_ready(g));
@@ -971,7 +878,7 @@ static int gicp_omp_align_body(lgs_gicp_omp* g, const float* guess16, lgs_align_
   identity16f(g->guess);
   if (guess16) memcpy(g->guess, guess16, sizeof(g->guess));
   for (float* T : {g->base_T, g->T, g->prev_T, g->final_T}) identity16f(T);
-  LGS_TRY(transform_source(g, g->guess, g->output.as<float4>()));
+  LGS_TRY(transform_source(g));
   bool converged = false;
   int nr_iterations = 0;
   while (!converged) {
@@ -993,7 +900,7 @@ static int gicp_omp_align_body(lgs_gicp_omp* g, const float* guess16, lgs_align_
       memcpy(g->prev_T, g->T, sizeof(g->T));
     }
   }
-  end_session(g);
+  g->session.close();  // before the output cloud's kernel
   mul4f(g->prev_T, g->guess, g->final_T);  // GO:512
   memcpy(res->T, g->final_T, sizeof(g->final_T));
   res->iterations = nr_iterations;
@@ -1001,14 +908,7 @@ static int gicp_omp_align_body(lgs_gicp_omp* g, const float* guess16, lgs_align_
   res->evaluations = g->fdf_calls + g->df_calls;
   res->line_search_trials = g->f_calls;
   res->hessian_recomputes = g->inner_total;
-  if (out_cloud) {  // GO:515
-    cudaStream_t st = g->ctx->stream;
-    const int64_t n = g->source->n;
-    LGS_TRY(g->out_cloud.reserve(static_cast<size_t>(n) * 16));
-    LGS_TRY(transform_source(g, g->final_T, g->out_cloud.as<float4>()));
-    LGS_CUDA(cudaMemcpyAsync(out_cloud, g->out_cloud.p, static_cast<size_t>(n) * 16, cudaMemcpyDeviceToHost, st));
-    LGS_CUDA(cudaStreamSynchronize(st));
-  }
+  if (out_cloud) LGS_TRY(write_aligned_cloud(g->ctx, g->source->pts.as<float4>(), g->source->n, g->final_T, &g->out_cloud, out_cloud));  // GO:515
   return LGS_OK;
 }
 
@@ -1048,7 +948,7 @@ int lgs_gicp_omp_functor(lgs_gicp_omp* g, const float* guess16, const float* tra
   memcpy(g->guess, guess16, sizeof(g->guess));
   memcpy(g->T, transformation16, sizeof(g->T));
   identity16f(g->base_T);
-  LGS_TRY(transform_source(g, g->guess, g->output.as<float4>()));
+  LGS_TRY(transform_source(g));
   LGS_TRY(update_correspondences(g));
   out15[14] = g->n_corr;
   double f_dummy = 0;

@@ -117,17 +117,15 @@ struct IcpPose {
   int use_seed;
   unsigned long long token;
 };
-constexpr int kIcpWords = static_cast<int>(sizeof(IcpPose) / 8);
-static_assert(sizeof(IcpPose) % 8 == 0, "commands are copied as 64-bit words");
-using IcpCmdHost = CmdHost<kIcpWords>;
-using IcpCmdDev = CmdDev<kIcpWords>;
+using IcpSession = ResidentSession<IcpPose>;
+constexpr int kIcpWords = IcpSession::kWords;
 constexpr int kIcpResident = 4;  // CTAs per SM of the persistent grid (all co-resident)
 
 __global__ void __launch_bounds__(kIcpBlock, kIcpResident) icp_persistent_kernel(const __grid_constant__ NNView tv, const float4* __restrict__ tgt,
                                                                                 float4* __restrict__ cloud, int* __restrict__ nn_prev, int n, double max_dist2,
                                                                                 double* __restrict__ partials, unsigned* __restrict__ counter,
-                                                                                MailboxRecord* mailbox, const IcpCmdHost* __restrict__ cmd_host,
-                                                                                IcpCmdDev* __restrict__ cmd_dev, unsigned long long first_seq) {
+                                                                                MailboxRecord* mailbox, const IcpSession::Host* __restrict__ cmd_host,
+                                                                                IcpSession::Dev* __restrict__ cmd_dev, unsigned long long first_seq) {
   __shared__ __align__(16) IcpPose pose;
   __shared__ IcpParams P;
   __shared__ int give_up;
@@ -149,14 +147,6 @@ __global__ void __launch_bounds__(kIcpBlock, kIcpResident) icp_persistent_kernel
     icp_step_body(tv, tgt, cloud, nn_prev, n, P, partials, counter, mb);
     __syncthreads();
   }
-}
-
-__global__ void __launch_bounds__(256) icp_transform_kernel(const float4* __restrict__ src, int64_t n, IcpParams P, float4* __restrict__ out) {
-  const int64_t i = blockIdx.x * static_cast<int64_t>(blockDim.x) + threadIdx.x;
-  if (i >= n) return;
-  const float4 p = src[i];
-  const float3 t = transform_pcl(P.T, p.x, p.y, p.z);
-  out[i] = make_float4(t.x, t.y, t.z, p.w);
 }
 
 }  // namespace lgs
@@ -186,27 +176,13 @@ struct lgs_icp {
   // closure, GBS:145-148).  lgs_icp_reset_convergence_criteria gives the state of a freshly constructed object.
   double crit_prev_mse = std::numeric_limits<double>::max();
   int crit_state = 0, crit_similar = 0;
-  // persistent evaluator (inside lgs_icp_align only)
-  bool allow_session = false, session_active = false, session_broken = false;
-  int session_device = -1;
-  IcpCmdHost* cmd_host = nullptr;  // mapped pinned memory
-  DevBuf cmd_dev;
-  unsigned long long cmd_seq = 0;
+  IcpSession session{IcpPose{{}, -1, 0, 0}};  // persistent evaluator (inside lgs_icp_align only)
 };
 
 namespace {
 
 enum { kNotConverged = 0, kIterations = 1, kTransform = 2, kAbsMse = 3, kRelMse = 4, kNoCorrespondences = 5 };
 
-void identity16f(float* T) {
-  for (int i = 0; i < 16; i++) T[i] = (i % 5 == 0) ? 1.0f : 0.0f;
-}
-void mul4f(const float* A, const float* B, float* C) {
-  float R[16];
-  for (int c = 0; c < 4; c++)
-    for (int r = 0; r < 4; r++) R[c * 4 + r] = ((A[r] * B[c * 4] + A[4 + r] * B[c * 4 + 1]) + A[8 + r] * B[c * 4 + 2]) + A[12 + r] * B[c * 4 + 3];
-  memcpy(C, R, sizeof(R));
-}
 float det3f(const float* m) {
   return m[0] * (m[4] * m[8] - m[5] * m[7]) - m[1] * (m[3] * m[8] - m[5] * m[6]) + m[2] * (m[3] * m[7] - m[4] * m[6]);
 }
@@ -286,30 +262,6 @@ int ensure_ready(lgs_icp* g) {
   return LGS_OK;
 }
 
-void end_session(lgs_icp* g) {
-  if (!g->session_active) return;
-  IcpPose quit;
-  memset(&quit, 0, sizeof(quit));
-  quit.apply = -1;
-  persist_send<kIcpWords>(g->cmd_host, ++g->cmd_seq, &quit);
-  g->session_active = false;
-  persist_release(g->session_device);
-}
-
-int prepare_session(lgs_icp* g) {  // whatever allocates or synchronises, before the grid becomes resident
-  if (!g->cmd_host) {
-    void* p = nullptr;
-    LGS_CUDA(cudaHostAlloc(&p, sizeof(IcpCmdHost), cudaHostAllocMapped | cudaHostAllocPortable));
-    memset(p, 0, sizeof(IcpCmdHost));
-    g->cmd_host = static_cast<IcpCmdHost*>(p);
-  }
-  if (!g->cmd_dev.p) {
-    LGS_TRY(g->cmd_dev.reserve(sizeof(IcpCmdDev)));
-    LGS_CUDA(cudaMemsetAsync(g->cmd_dev.p, 0, sizeof(IcpCmdDev), g->ctx->stream));
-  }
-  return LGS_OK;
-}
-
 // transforms the working cloud by T (unless null) and returns the 17 sums of the correspondences found after it
 int step(lgs_icp* g, const float* T, double* sums) {
   lgs_ctx* ctx = g->ctx;
@@ -323,44 +275,23 @@ int step(lgs_icp* g, const float* T, double* sums) {
   LGS_TRY(mailbox_next(ctx, &mb));
   const int grid = step_grid(g->n_source);
   const int n = static_cast<int>(g->n_source);
-  const bool want_session = g->allow_session && !g->session_broken && persist_env_enabled() && grid <= kNumSMs * kIcpResident;
-  if (!want_session) end_session(g);
-  if (want_session && !g->session_active) {
-    LGS_TRY(prepare_session(g));
-    if (persist_try_acquire(ctx->device)) {
-      void* dv = nullptr;
-      LGS_CUDA(cudaHostGetDevicePointer(&dv, g->cmd_host, 0));
-      icp_persistent_kernel<<<grid, kIcpBlock, 0, ctx->stream>>>(g->nn.view(), g->target.as<float4>(), g->cloud.as<float4>(), g->nn_prev.as<int>(), n, P.max_dist2,
-                                                               g->partials.as<double>(), g->state.as<unsigned>(), mb.r, static_cast<const IcpCmdHost*>(dv),
-                                                               g->cmd_dev.as<IcpCmdDev>(), g->cmd_seq + 1);
-      ctx->launches++;
-      cudaError_t le = cudaGetLastError();
-      if (le != cudaSuccess) {
-        persist_release(ctx->device);
-        set_error("icp_persistent_kernel launch failed: %s", cudaGetErrorString(le));
-        return LGS_ERR_CUDA;
-      }
-      g->session_active = true;
-      g->session_device = ctx->device;
-    }
-  }
-  if (g->session_active) {
+  LGS_TRY(g->session.open(ctx, grid <= kNumSMs * kIcpResident, [&](const IcpSession::Host* host, IcpSession::Dev* dev, unsigned long long first_seq) {
+    icp_persistent_kernel<<<grid, kIcpBlock, 0, ctx->stream>>>(g->nn.view(), g->target.as<float4>(), g->cloud.as<float4>(), g->nn_prev.as<int>(), n, P.max_dist2,
+                                                             g->partials.as<double>(), g->state.as<unsigned>(), mb.r, host, dev, first_seq);
+  }));
+  if (g->session.active) {
     IcpPose pose;
     memcpy(pose.T, P.T, sizeof(pose.T));
     pose.apply = P.apply;
     pose.use_seed = P.use_seed;
     pose.token = mb.token;
-    persist_send<kIcpWords>(g->cmd_host, ++g->cmd_seq, &pose);
+    g->session.send(pose);
     const int rc = mailbox_wait(ctx, mb, kIcpSums, sums);
     if (rc == LGS_OK) return LGS_OK;
     // The grid gave up (command time-out).  It may have transformed part of the working cloud already, so this align
-    // cannot be continued with plain launches: report it; the next align starts from the source cloud with plain launches.
-    end_session(g);
-    if (cudaStreamSynchronize(ctx->stream) == cudaSuccess && cudaGetLastError() == cudaSuccess) {
-      g->session_broken = true;
-      cudaMemsetAsync(g->state.p, 0, sizeof(unsigned), ctx->stream);
+    // cannot be continued with plain launches: lgs_icp_align runs it again from the source cloud.
+    if (g->session.recover(ctx, g->state.as<unsigned>()))
       set_error("IterativeClosestPoint: the resident evaluator timed out waiting for the host; call align again (plain launches from now on)");
-    }
     return rc;
   }
   icp_step_kernel<<<grid, kIcpBlock, 0, ctx->stream>>>(g->nn.view(), g->target.as<float4>(), g->cloud.as<float4>(), g->nn_prev.as<int>(), n, P, g->partials.as<double>(),
@@ -370,12 +301,8 @@ int step(lgs_icp* g, const float* T, double* sums) {
   return mailbox_wait(ctx, mb, kIcpSums, sums);
 }
 
-int set_cloud(lgs_icp* g, DevBuf* dst, int64_t* cnt, const void* pts, const float* pts_dev, int64_t n, int32_t stride) {
-  LGS_TRY(use_device(g->ctx));
-  if (pts_dev)
-    LGS_TRY(adopt_cloud_dev(g->ctx, pts_dev, n, dst));
-  else
-    LGS_TRY(upload_cloud(g->ctx, pts, n, stride, dst));
+int set_cloud(lgs_icp* g, DevBuf* dst, int64_t* cnt, const void* pts, int64_t n, int32_t stride, bool on_device) {
+  LGS_TRY(load_cloud(g->ctx, pts, n, stride, on_device, dst));
   *cnt = n;
   return LGS_OK;
 }
@@ -394,11 +321,7 @@ int lgs_icp_create(lgs_ctx* ctx, lgs_icp** out) {
 
 void lgs_icp_destroy(lgs_icp* g) {
   if (!g) return;
-  end_session(g);
-  cudaSetDevice(g->ctx->device);
-  cudaStreamSynchronize(g->ctx->stream);
-  if (g->cmd_host) cudaFreeHost(g->cmd_host);
-  g->cmd_dev.release();
+  g->session.release(g->ctx);
   for (DevBuf* b : {&g->source, &g->target, &g->target_copy, &g->cloud, &g->nn_prev, &g->partials, &g->state, &g->out_cloud}) b->release();
   g->nn.release();
   delete g;
@@ -419,42 +342,38 @@ int lgs_icp_reset_convergence_criteria(lgs_icp* g) {
 
 int lgs_icp_set_source(lgs_icp* g, const void* pts, int64_t n, int32_t stride) {
   LGS_REQUIRE(g, "null");
-  return set_cloud(g, &g->source, &g->n_source, pts, nullptr, n, stride);
+  return set_cloud(g, &g->source, &g->n_source, pts, n, stride, false);
 }
 int lgs_icp_set_source_dev(lgs_icp* g, const float* pts_dev, int64_t n) {
-  LGS_REQUIRE(g && (pts_dev || n == 0), "null");
-  return set_cloud(g, &g->source, &g->n_source, nullptr, pts_dev ? pts_dev : reinterpret_cast<const float*>(g), n, 16);
+  LGS_REQUIRE(g, "null");
+  return set_cloud(g, &g->source, &g->n_source, pts_dev, n, 16, true);
 }
 int lgs_icp_set_target(lgs_icp* g, const void* pts, int64_t n, int32_t stride) {
   LGS_REQUIRE(g, "null");
   g->nn_ready = false;
-  return set_cloud(g, &g->target, &g->n_target, pts, nullptr, n, stride);
+  return set_cloud(g, &g->target, &g->n_target, pts, n, stride, false);
 }
 int lgs_icp_set_target_dev(lgs_icp* g, const float* pts_dev, int64_t n) {
-  LGS_REQUIRE(g && (pts_dev || n == 0), "null");
+  LGS_REQUIRE(g, "null");
   g->nn_ready = false;
-  return set_cloud(g, &g->target, &g->n_target, nullptr, pts_dev ? pts_dev : reinterpret_cast<const float*>(g), n, 16);
+  return set_cloud(g, &g->target, &g->n_target, pts_dev, n, 16, true);
 }
 
 // pcl::Registration::align + IterativeClosestPoint::computeTransformation
-static int icp_align_body(lgs_icp* g, const float* guess16, lgs_align_result* res, float* out_cloud);
+static int icp_align(lgs_icp* g, const float* guess16, lgs_align_result* res, float* out_cloud);
 
 int lgs_icp_align(lgs_icp* g, const float* guess16, lgs_align_result* res, float* out_cloud) {
   LGS_NVTX("lgs_icp_align");
   LGS_REQUIRE(g && res, "null argument");
-  g->allow_session = true;
-  int rc = icp_align_body(g, guess16, res, out_cloud);
-  end_session(g);  // every exit path releases the resident grid
-  if (rc != LGS_OK && g->session_broken && g->allow_session) {
-    // the resident grid timed out mid-align (see step()): run the whole align again with plain launches
-    g->allow_session = false;
-    rc = icp_align_body(g, guess16, res, out_cloud);
-  }
-  g->allow_session = false;
+  const bool was_broken = g->session.broken;
+  const int rc = icp_align(g, guess16, res, out_cloud);
+  // the resident grid timed out mid-align (see step()): run the whole align again, with plain launches now
+  if (rc != LGS_OK && g->session.broken && !was_broken) return icp_align(g, guess16, res, out_cloud);
   return rc;
 }
 
-static int icp_align_body(lgs_icp* g, const float* guess16, lgs_align_result* res, float* out_cloud) {
+static int icp_align(lgs_icp* g, const float* guess16, lgs_align_result* res, float* out_cloud) {
+  SessionScope scope(g->session);
   memset(res, 0, sizeof(*res));
   LGS_TRY(use_device(g->ctx));
   LGS_TRY(ensure_ready(g));
@@ -498,7 +417,7 @@ static int icp_align_body(lgs_icp* g, const float* guess16, lgs_align_result* re
     g->last_mse = sums[1] / sums[0];
     converged = crit.check(nr_iterations, T, g->last_mse);
   } while (crit.state == kNotConverged);
-  end_session(g);
+  g->session.close();  // before the output cloud's kernel
   g->convergence_state = crit.state;
   g->crit_prev_mse = crit.prev_mse;
   g->crit_state = crit.state;
@@ -509,17 +428,7 @@ static int icp_align_body(lgs_icp* g, const float* guess16, lgs_align_result* re
   res->evaluations = nr_iterations;
   res->line_search_trials = crit.state;
   res->trans_probability = g->last_mse;
-  if (out_cloud) {
-    IcpParams P;
-    memcpy(P.T, g->final_T, sizeof(P.T));
-    P.apply = 1;
-    P.max_dist2 = 0;
-    LGS_TRY(g->out_cloud.reserve(static_cast<size_t>(g->n_source) * 16));
-    icp_transform_kernel<<<grid_for(g->n_source, 256), 256, 0, st>>>(g->source.as<float4>(), g->n_source, P, g->out_cloud.as<float4>());
-    g->ctx->launches++;
-    LGS_CUDA(cudaMemcpyAsync(out_cloud, g->out_cloud.p, static_cast<size_t>(g->n_source) * 16, cudaMemcpyDeviceToHost, st));
-    LGS_CUDA(cudaStreamSynchronize(st));
-  }
+  if (out_cloud) LGS_TRY(write_aligned_cloud(g->ctx, g->source.as<float4>(), g->n_source, g->final_T, &g->out_cloud, out_cloud));
   return LGS_OK;
 }
 

@@ -6,6 +6,7 @@
 #pragma once
 #include <cfloat>
 #include <cmath>
+#include <cstring>
 
 #if defined(__CUDACC__)
 #define LGS_HD __host__ __device__ __forceinline__
@@ -383,4 +384,17 @@ LGS_HD void ldlt_solve6(const double* Ain, const double* b, double* x) {
 }
 
 }  // namespace m
+
+// Host 4x4 transforms, column-major.  mul4f keeps Matrix4f's f32 order ((a0 b0 + a1 b1) + a2 b2) + a3 b3: the registration
+// results built from it are compared bit for bit with the reference.  C may alias A or B.
+inline void identity16f(float* T) {
+  for (int i = 0; i < 16; i++) T[i] = (i % 5 == 0) ? 1.0f : 0.0f;
+}
+inline void mul4f(const float* A, const float* B, float* C) {
+  float R[16];
+  for (int c = 0; c < 4; c++)
+    for (int r = 0; r < 4; r++) R[c * 4 + r] = ((A[r] * B[c * 4] + A[4 + r] * B[c * 4 + 1]) + A[8 + r] * B[c * 4 + 2]) + A[12 + r] * B[c * 4 + 3];
+  memcpy(C, R, sizeof(R));
+}
+
 }  // namespace lgs

@@ -366,7 +366,6 @@ __device__ __forceinline__ void block_reduce_and_finish(double (&acc)[K], double
 
 }  // namespace lgs
 
-#include "persist.cuh"
 #include "ndt_opt.cuh"
 #include "ndt_deriv.cuh"
 
@@ -405,14 +404,6 @@ __global__ void __launch_bounds__(kEvalBlock) ndt_score_kernel(const float4* __r
     }
   }
   block_reduce_and_finish<1>(acc, partials, result, counter, mb);
-}
-
-__global__ void __launch_bounds__(256) transform_cloud_kernel(const float4* __restrict__ src, int64_t n, EvalParams P, float4* __restrict__ out) {
-  int64_t i = blockIdx.x * static_cast<int64_t>(blockDim.x) + threadIdx.x;
-  if (i >= n) return;
-  float4 p = src[i];
-  float3 t = transform_pcl(P.T, p.x, p.y, p.z);
-  out[i] = make_float4(t.x, t.y, t.z, p.w);
 }
 
 }  // namespace lgs
@@ -485,10 +476,6 @@ struct lgs_ndt {
 namespace {
 
 constexpr uint64_t kDenseCellLimit = uint64_t(1) << 26;  // 64 Mi cells (256 MiB of int32) before switching to the hash
-
-void identity16(float* T) {
-  for (int i = 0; i < 16; i++) T[i] = (i % 5 == 0) ? 1.0f : 0.0f;
-}
 
 // NDT.h:214-231 (ndt_opt.cuh holds the arithmetic, shared with the device-resident optimiser)
 void pose_to_matrix(const double x[6], float* T) {
@@ -1092,7 +1079,7 @@ int lgs_ndt_create(lgs_ctx* ctx, lgs_ndt** out) {
   LGS_REQUIRE(ctx && out, "null argument");
   lgs_ndt* n = new lgs_ndt;
   n->ctx = ctx;
-  identity16(n->final_T);
+  identity16f(n->final_T);
   memset(&n->P, 0, sizeof(n->P));
   compute_gauss(n);
   *out = n;
@@ -1154,16 +1141,14 @@ static int after_target(lgs_ndt* n) {
 int lgs_ndt_set_target(lgs_ndt* n, const void* pts, int64_t cnt, int32_t stride) {
   LGS_NVTX("lgs_ndt_set_target");
   LGS_REQUIRE(n, "null");
-  LGS_TRY(use_device(n->ctx));
-  LGS_TRY(upload_cloud(n->ctx, pts, cnt, stride, &n->target));
+  LGS_TRY(load_cloud(n->ctx, pts, cnt, stride, false, &n->target));
   n->n_target = cnt;
   return after_target(n);
 }
 int lgs_ndt_set_target_dev(lgs_ndt* n, const float* pts_dev, int64_t cnt) {
   LGS_NVTX("lgs_ndt_set_target_dev");
   LGS_REQUIRE(n, "null");
-  LGS_TRY(use_device(n->ctx));
-  LGS_TRY(adopt_cloud_dev(n->ctx, pts_dev, cnt, &n->target));
+  LGS_TRY(load_cloud(n->ctx, pts_dev, cnt, 16, true, &n->target));
   n->n_target = cnt;
   return after_target(n);
 }
@@ -1191,16 +1176,14 @@ int lgs_ndt_set_target_keyframes(lgs_ndt* n, lgs_keyframes* kf, const int32_t* i
 
 int lgs_ndt_set_source(lgs_ndt* n, const void* pts, int64_t cnt, int32_t stride) {
   LGS_REQUIRE(n, "null");
-  LGS_TRY(use_device(n->ctx));
-  LGS_TRY(upload_cloud(n->ctx, pts, cnt, stride, &n->source));
+  LGS_TRY(load_cloud(n->ctx, pts, cnt, stride, false, &n->source));
   n->n_source = cnt;
   n->have_source = true;
   return LGS_OK;
 }
 int lgs_ndt_set_source_dev(lgs_ndt* n, const float* pts_dev, int64_t cnt) {
   LGS_REQUIRE(n, "null");
-  LGS_TRY(use_device(n->ctx));
-  LGS_TRY(adopt_cloud_dev(n->ctx, pts_dev, cnt, &n->source));
+  LGS_TRY(load_cloud(n->ctx, pts_dev, cnt, 16, true, &n->source));
   n->n_source = cnt;
   n->have_source = true;
   return LGS_OK;
@@ -1222,7 +1205,7 @@ int lgs_ndt_align(lgs_ndt* n, const float* guess16, lgs_align_result* res, float
   n->align_launches = 0;
   compute_gauss(n);
   float guess[16];
-  identity16(guess);
+  identity16f(guess);
   if (guess16) memcpy(guess, guess16, sizeof(guess));  // NDT:95-101; the evaluation transforms by the guess on the fly
   double p0[6];
   matrix_to_pose(guess, p0);  // NDT:103-111
@@ -1246,15 +1229,7 @@ int lgs_ndt_align(lgs_ndt* n, const float* guess16, lgs_align_result* res, float
     fprintf(stderr, "[lgs ndt] align %.1f us (%s): %d evaluations (%d trials, %d f64 Hessians), %d iterations\n",
             std::chrono::duration<double, std::micro>(std::chrono::steady_clock::now() - t0).count(), on_device ? "one resident launch" : "host-stepped",
             res->evaluations, res->line_search_trials, res->hessian_recomputes, res->iterations);
-  if (out_cloud && n->n_source) {
-    cudaStream_t st = n->ctx->stream;
-    LGS_TRY(n->out_cloud.reserve(static_cast<size_t>(n->n_source) * 16));
-    memcpy(n->P.T, n->final_T, sizeof(float) * 16);
-    transform_cloud_kernel<<<grid_for(n->n_source, 256), 256, 0, st>>>(n->source.as<float4>(), n->n_source, n->P, n->out_cloud.as<float4>());
-    n->ctx->launches++;
-    LGS_CUDA(cudaMemcpyAsync(out_cloud, n->out_cloud.p, static_cast<size_t>(n->n_source) * 16, cudaMemcpyDeviceToHost, st));
-    LGS_CUDA(cudaStreamSynchronize(st));
-  }
+  if (out_cloud) LGS_TRY(write_aligned_cloud(n->ctx, n->source.as<float4>(), n->n_source, n->final_T, &n->out_cloud, out_cloud));
   return LGS_OK;
 }
 
