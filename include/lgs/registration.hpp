@@ -217,6 +217,22 @@ class NormalDistributionsTransform : public Registration {
     return s;
   }
   lgs_ndt* handle() const { return h_; }
+  // No counterpart in the reference: align this source from every guess in one resident launch per wave
+  // (lgs_ndt_align_many).  Record k is bit-identical to align(output, guesses[k]); afterwards result() is the last guess's.
+  // fitness_max_range < 0: no fitness, else records[k].fitness = getFitnessScore(fitness_max_range) at record k's transform.
+  std::vector<lgs_align_result> alignGuesses(const std::vector<Matrix4f>& guesses, double fitness_max_range = -1.0) {
+    ok_ = true;
+    std::vector<lgs_ndt*> hs(guesses.size(), h_);
+    std::vector<float> packed(guesses.size() * 16);
+    for (size_t k = 0; k < guesses.size(); k++) std::copy(guesses[k].begin(), guesses[k].end(), packed.begin() + 16 * k);
+    std::vector<lgs_align_result> out(guesses.size());
+    check(lgs_ndt_align_many(hs.data(), static_cast<int32_t>(hs.size()), packed.data(), fitness_max_range < 0 ? nullptr : &fitness_max_range,
+                             out.data(), nullptr));
+    if (ok_ && !out.empty()) result_ = out.back();
+    return out;
+  }
+  friend std::vector<lgs_align_result> alignMany(const std::vector<NormalDistributionsTransform*>& ndts, const std::vector<Matrix4f>& guesses,
+                                                 double fitness_max_range);
 
  private:
   std::shared_ptr<Context> ctx_;
@@ -224,6 +240,28 @@ class NormalDistributionsTransform : public Registration {
   float resolution_ = 1.0f;
   double step_ = 0.1, outlier_ = 0.55;
 };
+
+// No counterpart in the reference: ndts[i]->align(guesses[i]) for every i in one resident launch per wave (lgs_ndt_align_many);
+// the objects may repeat and must share one Context.  guesses: empty (identity) or one per object.  Each object's result()
+// becomes that of its last occurrence.  On failure every object records the error (hasConverged() false, lastError()).
+inline std::vector<lgs_align_result> alignMany(const std::vector<NormalDistributionsTransform*>& ndts, const std::vector<Matrix4f>& guesses = {},
+                                               double fitness_max_range = -1.0) {
+  std::vector<lgs_ndt*> hs;
+  for (auto* x : ndts) hs.push_back(x->h_);
+  std::vector<float> packed(guesses.size() * 16);
+  for (size_t k = 0; k < guesses.size(); k++) std::copy(guesses[k].begin(), guesses[k].end(), packed.begin() + 16 * k);
+  std::vector<lgs_align_result> out(ndts.size());
+  const int rc = (!guesses.empty() && guesses.size() != ndts.size())
+                     ? LGS_ERR_INVALID
+                     : lgs_ndt_align_many(hs.data(), static_cast<int32_t>(hs.size()), guesses.empty() ? nullptr : packed.data(),
+                                          fitness_max_range < 0 ? nullptr : &fitness_max_range, out.data(), nullptr);
+  for (size_t i = 0; i < ndts.size(); i++) {
+    ndts[i]->ok_ = true;
+    ndts[i]->check(rc);
+    if (rc == LGS_OK) ndts[i]->result_ = out[i];
+  }
+  return out;
+}
 
 enum class RegularizationMethod { NONE = LGS_REG_NONE, MIN_EIG, NORMALIZED_MIN_EIG, PLANE, FROBENIUS };
 

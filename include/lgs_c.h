@@ -198,6 +198,15 @@ int lgs_ndt_set_target_keyframes(lgs_ndt* ndt, lgs_keyframes* kf, const int32_t*
 /* align (pcl::Registration::align + NDT:80-171, LSM:165, GBS:318).  guess may be NULL (identity).
  * out_cloud: NULL or capacity n_source packed xyzi records = source transformed by the final T. */
 int lgs_ndt_align(lgs_ndt* ndt, const float* guess16, lgs_align_result* result, float* out_cloud);
+/* No counterpart in the reference (ndt_omp runs one align per call): N aligns in one resident launch (per wave).  Record i is
+ * bit-identical to lgs_ndt_align(ndts[i], guess i) run alone, and each handle ends in the state its last occurrence leaves;
+ * handles may repeat; all on one context.  guesses16: N x 16 col-major floats or NULL (identity).  fitness_max_range:
+ * NULL = no fitness, else records[i].fitness = getFitnessScore(*fitness_max_range) at record i's transform.
+ * out_clouds: NULL or N pointers (each NULL or capacity n_source of ndts[i]).  records[i].pair_id = i.  n = 0 does nothing.
+ * LGS_NDT_MANY_MAX_GROUPS (environment, read on every call): at most this many aligns per launch (default 1:
+ * measured, grouped aligns were slower than consecutive ones; see DESIGN section 7). */
+int lgs_ndt_align_many(lgs_ndt* const* ndts, int32_t n, const float* guesses16, const double* fitness_max_range,
+                       lgs_align_result* records, float* const* out_clouds);
 /* getFitnessScore(max_range) (PCL registration.hpp, GBS:321): exact 1-NN mean squared distance */
 int lgs_ndt_fitness(lgs_ndt* ndt, double max_range, double* fitness);
 /* calculateScore (NDT:934-982) of the source transformed by T */

@@ -88,6 +88,7 @@ SYMBOLS = {
     "lgs_ndt_set_source_dev": (_i32, [_vp, _vp, _i64]),
     "lgs_ndt_set_target_keyframes": (_i32, [_vp, _vp, _vp, _i32, C.POINTER(_i32)]),
     "lgs_ndt_align": (_i32, [_vp, _vp, C.POINTER(AlignResult), _vp]),
+    "lgs_ndt_align_many": (_i32, [_vp, _i32, _vp, _vp, C.POINTER(AlignResult), _vp]),
     "lgs_ndt_fitness": (_i32, [_vp, _f64, C.POINTER(_f64)]),
     "lgs_ndt_calculate_score": (_i32, [_vp, _vp, C.POINTER(_f64)]),
     "lgs_ndt_grid_info_get": (_i32, [_vp, C.POINTER(NdtGridInfo)]),

@@ -401,6 +401,11 @@ class NormalDistributionsTransform(_Registration):
         self._nt = -1
         return nv.value
 
+    def align_guesses(self, guesses, fitness_max_range=None):
+        """One map, many seeds: align this source from every 4x4 guess in one resident launch per wave (ndt_align_many).
+        Record k is bit-identical to align(guesses[k]); afterwards the object holds the last guess's result."""
+        return ndt_align_many([self] * len(guesses), guesses, fitness_max_range)
+
     def align_breakdown(self):
         """SM cycles CTA 0 spent per phase of the last device-resident align (lgs_ndt_align_breakdown)."""
         out = np.zeros(16)
@@ -655,6 +660,33 @@ class IterativeClosestPoint(_Registration):
         sums, T, ok = np.zeros(17), np.zeros(16, np.float32), C.c_int32()
         check(self._L.lgs_icp_step(self._h, vp(gc), vp(sums), vp(T), C.byref(ok)))
         return bool(ok.value), sums, T.reshape(4, 4, order="F").copy()
+
+
+def ndt_align_many(ndts, guesses=None, fitness_max_range=None, want_output=False):
+    """Aligns N NDT problems in one resident launch per wave (lgs_ndt_align_many): ndts[i] from guesses[i] (4x4, or identity
+    when guesses is None).  Handles may repeat and must share one Context.  Each record is bit-identical to ndts[i].align(
+    guesses[i]) run alone, and every object ends with the result and final transformation of its last occurrence, as after
+    those calls in order.  fitness_max_range: records[i].fitness = getFitnessScore(fitness_max_range) at record i's
+    transform.  Returns the list of records, or (records, aligned clouds) when want_output."""
+    n = len(ndts)
+    if guesses is not None and len(guesses) != n:
+        raise ValueError("need one guess per problem")
+    L = _lib.load()
+    hs = (C.c_void_p * max(n, 1))(*[x._h.value for x in ndts])
+    g = _pack_guesses(guesses) if n else None
+    recs = (AlignResult * max(n, 1))()
+    fmr = C.c_double(float(fitness_max_range)) if fitness_max_range is not None else None
+    outs = [np.empty((max(x._ns, 1), 4), np.float32) for x in ndts] if want_output else None
+    op = (C.c_void_p * max(n, 1))(*[o.ctypes.data for o in outs]) if want_output else None
+    check(L.lgs_ndt_align_many(hs, n, g.ctypes.data_as(C.c_void_p) if g is not None else None, C.byref(fmr) if fmr is not None else None,
+                               recs, op))
+    out = [recs[i] for i in range(n)]
+    for x, r in zip(ndts, out):
+        x.result = r
+        x.final_transformation = _result_T(r)
+    if want_output:
+        return out, [o[: x._ns] for o, x in zip(outs, ndts)]
+    return out
 
 
 def knn(pts, queries, k, ctx=None):

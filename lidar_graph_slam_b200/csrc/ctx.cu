@@ -229,6 +229,7 @@ void lgs_ctx_destroy(lgs_ctx* c) {
   c->vg_out.release();
   c->vg_vidx.release();
   c->vg_rank.release();
+  c->ndt_many.release();
   if (c->mbox) cudaFreeHost(c->mbox);
   if (c->own_stream) cudaStreamDestroy(c->stream);
   delete c;

@@ -810,6 +810,7 @@ struct DeviceCaps {
   bool ready = false;
   int num_sms = 0;
   int align_ctas_per_sm[2] = {0, 0};  // ndt_align_kernel<D7 = false / true>
+  int group_ctas_per_sm[2] = {0, 0};  // ndt_align_group_kernel<D7 = false / true>
 };
 int device_caps(lgs_ctx* ctx, const DeviceCaps** out) {
   static DeviceCaps caps[64];
@@ -824,12 +825,16 @@ int device_caps(lgs_ctx* ctx, const DeviceCaps** out) {
     LGS_CUDA(cudaFuncSetAttribute(ndt_derivatives_kernel<2, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem));
     LGS_CUDA(cudaFuncSetAttribute(ndt_align_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem));
     LGS_CUDA(cudaFuncSetAttribute(ndt_align_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem));
+    LGS_CUDA(cudaFuncSetAttribute(ndt_align_group_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem));
+    LGS_CUDA(cudaFuncSetAttribute(ndt_align_group_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem));
     LGS_CUDA(cudaDeviceGetAttribute(&c.num_sms, cudaDevAttrMultiProcessorCount, ctx->device));
     int coop = 0;
     LGS_CUDA(cudaDeviceGetAttribute(&coop, cudaDevAttrCooperativeLaunch, ctx->device));
     if (coop) {
       LGS_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&c.align_ctas_per_sm[0], ndt_align_kernel<false>, kDerivThreads, sizeof(DerivSmem)));
       LGS_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&c.align_ctas_per_sm[1], ndt_align_kernel<true>, kDerivThreads, sizeof(DerivSmem)));
+      LGS_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&c.group_ctas_per_sm[0], ndt_align_group_kernel<false>, kDerivThreads, sizeof(DerivSmem)));
+      LGS_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&c.group_ctas_per_sm[1], ndt_align_group_kernel<true>, kDerivThreads, sizeof(DerivSmem)));
     }
     c.ready = true;
   }
@@ -995,6 +1000,28 @@ int align_host_stepped(lgs_ndt* n, const double p0[6], const float T0[16], Align
   return LGS_OK;
 }
 
+// Evaluating CTAs of a device-resident align of n (one per round of 32 points at most, one CTA per SM, the optimiser's SM
+// excluded).  G also fixes which points each CTA adds and in what order the rows are summed: every launch form of the align
+// must use this G to produce the same bits.
+int align_eval_ctas(const lgs_ndt* n, const DeviceCaps* caps) {
+  return std::max(1, std::min(std::min(kNumSMs, caps->num_sms) - 1, static_cast<int>((n->n_source + 31) / 32)));
+}
+
+// The inputs of a device-resident align of n from guess T0 (pose p0): the first command in n->P (NDT:119: the guess and the
+// tables of its pose; the machine on the device builds the same one) and the machine's arguments.
+void align_launch_inputs(lgs_ndt* n, const double p0[6], const float T0[16], NdtAlignArgs* args) {
+  fill_eval_constants(n);
+  memcpy(n->P.T, T0, sizeof(float) * 16);
+  angle_derivatives(p0, &n->P);
+  memcpy(args->p0, p0, sizeof(args->p0));
+  memcpy(args->T0, T0, sizeof(args->T0));
+  args->step_size = n->step_size;
+  args->trans_eps = n->trans_eps;
+  args->n_in = static_cast<double>(n->n_source);
+  args->max_iter = n->max_iter;
+  args->exact_solve = exact_solve_requested(n) ? 1 : 0;
+}
+
 // the whole align as one cooperative launch of ndt_align_kernel; *used = false when the device cannot hold the grid
 int align_on_device(lgs_ndt* n, const double p0[6], const float T0[16], AlignOutcome* out, bool* used) {
   *used = false;
@@ -1004,23 +1031,12 @@ int align_on_device(lgs_ndt* n, const double p0[6], const float T0[16], AlignOut
   LGS_TRY(device_caps(ctx, &caps));
   const bool d7 = n->search == LGS_NDT_DIRECT7;
   const int ns = static_cast<int>(n->n_source);
-  // evaluating CTAs (one per round of 32 points at most) + the optimiser CTA, one CTA per SM
-  const int grid = std::max(1, std::min(std::min(kNumSMs, caps->num_sms) - 1, (ns + 31) / 32)) + 1;
+  const int grid = align_eval_ctas(n, caps) + 1;  // + the optimiser CTA
   if (caps->num_sms < 2 || caps->align_ctas_per_sm[d7 ? 1 : 0] * caps->num_sms < grid) return LGS_OK;  // the grid must be co-resident
   LGS_TRY(ensure_reduction_buffers(n, grid));
   if (!n->align_dev.p) LGS_TRY(n->align_dev.reserve(sizeof(NdtAlignDev)));
-  fill_eval_constants(n);
-  // the first command (NDT:119): the guess and the tables of its pose; the machine on the device builds the same one
-  memcpy(n->P.T, T0, sizeof(float) * 16);
-  angle_derivatives(p0, &n->P);
   NdtAlignArgs args;
-  memcpy(args.p0, p0, sizeof(args.p0));
-  memcpy(args.T0, T0, sizeof(args.T0));
-  args.step_size = n->step_size;
-  args.trans_eps = n->trans_eps;
-  args.n_in = static_cast<double>(n->n_source);
-  args.max_iter = n->max_iter;
-  args.exact_solve = exact_solve_requested(n) ? 1 : 0;
+  align_launch_inputs(n, p0, T0, &args);
   Mailbox mb;
   LGS_TRY(mailbox_next(ctx, &mb));
   LGS_CUDA(cudaMemsetAsync(n->align_dev.p, 0, 48, st));  // seq, the arrival counter, the trace words
@@ -1068,6 +1084,116 @@ int align_on_device(lgs_ndt* n, const double p0[6], const float T0[16], AlignOut
     n->prof_align_terms += h[30];
   }
   *used = true;
+  return LGS_OK;
+}
+
+// getFitnessScore(max_range) of n's source under T (the 1-NN structure over the target is built on first use)
+int fitness_at(lgs_ndt* n, const float* T, double max_range, double* fitness) {
+  LGS_TRY(ensure_target_cloud(n));
+  if (!n->nn_ready) {
+    LGS_TRY(n->nn.build(n->ctx, n->target.as<float4>(), n->n_target));
+    n->nn_ready = true;
+  }
+  return nn_fitness(n->ctx, n->nn, n->source.as<float4>(), n->n_source, T, max_range, fitness);
+}
+
+// ---- several aligns in one launch (lgs_ndt_align_many) --------------------------------------------------------------
+// Groups per ndt_align_group_kernel launch (a wave), unless LGS_NDT_MANY_MAX_GROUPS says otherwise (read on every call).
+// 1: measured on a B200 (DESIGN section 7), every grouping of 2 to 16 problems was slower than the same aligns one after
+// another - a group's aligns end at different evaluation counts, and the SMs of the groups that finish first idle.
+constexpr int kManyDefaultGroups = 1;
+int many_max_groups() {
+  const char* e = getenv("LGS_NDT_MANY_MAX_GROUPS");
+  const int v = e && e[0] ? atoi(e) : 0;
+  return v > 0 ? v : kManyDefaultGroups;
+}
+
+struct ManyProblem {
+  int i;  // index in the caller's list
+  lgs_ndt* n;
+  double p0[6];
+  float T0[16];
+  int G;  // evaluating CTAs of the same align alone (align_eval_ctas)
+};
+
+constexpr size_t kManyRowsPerGroup = static_cast<size_t>(kNumSMs) * (kRow + 8);  // doubles: G <= kNumSMs - 1 rows (+ trace words)
+inline size_t round_up_256(size_t b) { return (b + 255) & ~size_t(255); }
+
+// One cooperative launch of ndt_align_group_kernel<d7> for probs[0..k): group sizes roughly proportional to G with
+// 1 <= g <= G and sum(g + 1) <= capacity; record r of problem j lands in out[j * kAlignResultRecords + r].
+int run_many_wave(lgs_ctx* ctx, bool d7, int capacity, const ManyProblem* probs, int k, double* out) {
+  cudaStream_t st = ctx->stream;
+  if (k == 1) {  // a lone problem: lgs_ndt_align's own launch, without the descriptor and record copies
+    lgs_ndt* n = probs[0].n;
+    AlignOutcome o;
+    bool used = false;
+    LGS_TRY(align_on_device(n, probs[0].p0, probs[0].T0, &o, &used));
+    LGS_REQUIRE(used, "the align grid does not fit the device");
+    std::fill(out, out + kAlignResultRecords, 0.0);
+    for (int r = 0; r < 16; r++) out[r] = static_cast<double>(o.T[r]);
+    out[23] = o.trans_probability;
+    out[24] = o.iterations;
+    out[25] = o.converged;
+    out[26] = o.evals;
+    out[27] = o.trials;
+    out[28] = o.hess;
+    out[29] = n->last_terms;
+    out[30] = n->terms_total;
+    for (int r = 0; r < 16; r++) out[32 + r] = n->align_trace[r];
+    return LGS_OK;
+  }
+  const size_t desc_b = round_up_256(sizeof(NdtGroupDesc) * k), dev_b = round_up_256(sizeof(NdtAlignDev) * k);
+  const size_t rec_b = round_up_256(sizeof(double) * kAlignResultRecords * k), rows_b = sizeof(double) * kManyRowsPerGroup * k;
+  // an earlier call may still have a copy out of the pinned staging blocks in flight on this stream (keyframes.cu does the same)
+  LGS_CUDA(cudaStreamSynchronize(st));
+  LGS_TRY(ctx->ndt_many.reserve(desc_b + dev_b + rec_b + rows_b));
+  LGS_TRY(ctx->pin_up.reserve(sizeof(NdtGroupDesc) * k));
+  LGS_TRY(ctx->pin.reserve(sizeof(double) * kAlignResultRecords * k));
+  char* base = ctx->ndt_many.as<char>();
+  NdtGroupDesc* descs = reinterpret_cast<NdtGroupDesc*>(base);
+  NdtAlignDev* devs = reinterpret_cast<NdtAlignDev*>(base + desc_b);
+  double* recs = reinterpret_cast<double*>(base + desc_b + dev_b);
+  double* rows = reinterpret_cast<double*>(base + desc_b + dev_b + rec_b);
+  int64_t sum_G = 0;
+  for (int j = 0; j < k; j++) sum_G += probs[j].G;
+  const int64_t spare = capacity - 2 * k;  // evaluating CTAs beyond the one every group has
+  NdtGroupDesc* h = ctx->pin_up.as<NdtGroupDesc>();
+  int cta = 0;
+  for (int j = 0; j < k; j++) {
+    lgs_ndt* n = probs[j].n;
+    NdtGroupDesc& d = h[j];
+    align_launch_inputs(n, probs[j].p0, probs[j].T0, &d.args);
+    d.P0 = n->P;
+    d.ct = make_cell_table(n);
+    d.src = n->source.as<float4>();
+    d.recs = n->recs.as<VoxelRec>();
+    d.vmean = n->ex_mean.as<double>();
+    d.vicov = n->ex_icov.as<double>();
+    d.partials = rows + kManyRowsPerGroup * j;
+    d.dev = devs + j;
+    d.record = recs + static_cast<size_t>(kAlignResultRecords) * j;
+    d.n = static_cast<int>(n->n_source);
+    d.G = probs[j].G;
+    d.g = static_cast<int>(std::min<int64_t>(probs[j].G, 1 + spare * probs[j].G / sum_G));
+    d.cta0 = cta;
+    cta += d.g + 1;
+  }
+  LGS_CUDA(cudaMemcpyAsync(descs, h, sizeof(NdtGroupDesc) * k, cudaMemcpyHostToDevice, st));
+  LGS_CUDA(cudaMemsetAsync(devs, 0, sizeof(NdtAlignDev) * k, st));
+  const NdtGroupDesc* descs_arg = descs;
+  int k_arg = k;
+  u64 one2 = 0x3f8000003f800000ull;  // (1.0f, 1.0f): see ndt_deriv.cuh
+  void* kargs[] = {&descs_arg, &k_arg, &one2};
+  const void* fn = d7 ? reinterpret_cast<const void*>(ndt_align_group_kernel<true>) : reinterpret_cast<const void*>(ndt_align_group_kernel<false>);
+  cudaError_t le = cudaLaunchCooperativeKernel(fn, dim3(cta), dim3(kDerivThreads), kargs, sizeof(DerivSmem), st);
+  if (le != cudaSuccess) {
+    set_error("ndt_align_group_kernel cooperative launch failed: %s", cudaGetErrorString(le));
+    return LGS_ERR_CUDA;
+  }
+  ctx->launches++;
+  LGS_CUDA(cudaMemcpyAsync(ctx->pin.p, recs, sizeof(double) * kAlignResultRecords * k, cudaMemcpyDeviceToHost, st));
+  LGS_CUDA(cudaStreamSynchronize(st));
+  memcpy(out, ctx->pin.p, sizeof(double) * kAlignResultRecords * k);
   return LGS_OK;
 }
 
@@ -1241,12 +1367,98 @@ int lgs_ndt_fitness(lgs_ndt* n, double max_range, double* fitness) {
     return LGS_ERR_STATE;
   }
   LGS_TRY(use_device(n->ctx));
-  LGS_TRY(ensure_target_cloud(n));
-  if (!n->nn_ready) {
-    LGS_TRY(n->nn.build(n->ctx, n->target.as<float4>(), n->n_target));
-    n->nn_ready = true;
+  return fitness_at(n, n->final_T, max_range, fitness);
+}
+
+// N aligns as if lgs_ndt_align(ndts[i], guess i, &records[i], out_clouds[i]) ran for i = 0 .. n - 1 in turn.  The problems a
+// lone align would run in one ndt_align_kernel launch go to ndt_align_group_kernel launches (one per wave of at most
+// many_max_groups() problems of one search-method class); every other problem runs through lgs_ndt_align itself.
+int lgs_ndt_align_many(lgs_ndt* const* ndts, int32_t count, const float* guesses16, const double* fitness_max_range, lgs_align_result* records,
+                       float* const* out_clouds) {
+  LGS_NVTX("lgs_ndt_align_many");
+  LGS_REQUIRE(count >= 0, "negative count");
+  if (count == 0) return LGS_OK;
+  LGS_REQUIRE(ndts && records, "null argument");
+  for (int32_t i = 0; i < count; i++) LGS_REQUIRE(ndts[i], "null handle");
+  lgs_ctx* ctx = ndts[0]->ctx;
+  for (int32_t i = 0; i < count; i++) LGS_REQUIRE(ndts[i]->ctx == ctx, "all handles must belong to one context");
+  for (int32_t i = 0; i < count; i++) {
+    if (!ndts[i]->have_target || !ndts[i]->have_source) {
+      set_error("lgs_ndt_align_many: handle %d: setInputTarget and setInputSource must be called first", i);
+      return LGS_ERR_STATE;
+    }
   }
-  return nn_fitness(n->ctx, n->nn, n->source.as<float4>(), n->n_source, n->final_T, max_range, fitness);
+  LGS_TRY(use_device(ctx));
+  const DeviceCaps* caps = nullptr;
+  LGS_TRY(device_caps(ctx, &caps));
+  std::vector<lgs_ndt*> prepared;
+  for (int32_t i = 0; i < count; i++) {
+    lgs_ndt* n = ndts[i];
+    if (std::find(prepared.begin(), prepared.end(), n) != prepared.end()) continue;
+    prepared.push_back(n);
+    if (!n->grid_ready) LGS_TRY(build_grid(n));
+    compute_gauss(n);
+  }
+  // route: a problem joins a group launch exactly when lgs_ndt_align would run it as one ndt_align_kernel launch
+  std::vector<ManyProblem> cls[2];  // DIRECT1 / DIRECT26, DIRECT7: D7 is a template parameter of the kernel
+  std::vector<int> slot(count, -1);  // problem i's place in its class, -1: runs through lgs_ndt_align
+  for (int32_t i = 0; i < count; i++) {
+    lgs_ndt* n = ndts[i];
+    const int c = n->search == LGS_NDT_DIRECT7 ? 1 : 0;
+    const int G = align_eval_ctas(n, caps);
+    const bool nothing_to_evaluate = n->n_source == 0 || n->refused || n->n_valid == 0;
+    const bool fits = caps->num_sms >= 2 && caps->align_ctas_per_sm[c] * caps->num_sms >= G + 1 && caps->group_ctas_per_sm[c] * caps->num_sms >= 2;
+    if (nothing_to_evaluate || n->profiling != 0 || !device_align_env_enabled() || !fits) continue;
+    ManyProblem p;
+    p.i = i;
+    p.n = n;
+    identity16f(p.T0);
+    if (guesses16) memcpy(p.T0, guesses16 + 16 * static_cast<size_t>(i), sizeof(p.T0));
+    matrix_to_pose(p.T0, p.p0);
+    p.G = G;
+    slot[i] = static_cast<int>(cls[c].size());
+    cls[c].push_back(p);
+  }
+  std::vector<double> rec[2];
+  for (int c = 0; c < 2; c++) {
+    rec[c].resize(cls[c].size() * kAlignResultRecords);
+    const int capacity = caps->group_ctas_per_sm[c] * caps->num_sms;
+    const int M = std::max(1, std::min(many_max_groups(), capacity / 2));
+    for (size_t w0 = 0; w0 < cls[c].size(); w0 += M) {
+      const int k = static_cast<int>(std::min(cls[c].size() - w0, static_cast<size_t>(M)));
+      LGS_TRY(run_many_wave(ctx, c == 1, capacity, cls[c].data() + w0, k, rec[c].data() + w0 * kAlignResultRecords));
+    }
+  }
+  // publish in the caller's order: each handle ends in the state of its last occurrence
+  for (int32_t i = 0; i < count; i++) {
+    lgs_ndt* n = ndts[i];
+    lgs_align_result* res = records + i;
+    float* out_cloud = out_clouds ? out_clouds[i] : nullptr;
+    if (slot[i] < 0) {
+      float guess[16];
+      identity16f(guess);
+      if (guesses16) memcpy(guess, guesses16 + 16 * static_cast<size_t>(i), sizeof(guess));
+      LGS_TRY(lgs_ndt_align(n, guess, res, out_cloud));
+    } else {
+      const double* h = rec[n->search == LGS_NDT_DIRECT7 ? 1 : 0].data() + static_cast<size_t>(slot[i]) * kAlignResultRecords;
+      memset(res, 0, sizeof(*res));
+      for (int k = 0; k < 16; k++) res->T[k] = n->final_T[k] = static_cast<float>(h[k]);
+      res->trans_probability = h[23];
+      res->iterations = static_cast<int>(h[24]);
+      res->converged = static_cast<int>(h[25]);
+      res->evaluations = n->evals = static_cast<int>(h[26]);
+      res->line_search_trials = n->trials = static_cast<int>(h[27]);
+      res->hessian_recomputes = n->hess_recomputes = static_cast<int>(h[28]);
+      n->last_terms = h[29];
+      n->terms_total = h[30];
+      for (int k = 0; k < 16; k++) n->align_trace[k] = h[32 + k];
+      n->align_launches = 1;
+      if (out_cloud) LGS_TRY(write_aligned_cloud(ctx, n->source.as<float4>(), n->n_source, n->final_T, &n->out_cloud, out_cloud));
+    }
+    if (fitness_max_range) LGS_TRY(fitness_at(n, res->T, *fitness_max_range, &res->fitness));
+    res->pair_id = i;
+  }
+  return LGS_OK;
 }
 
 int lgs_ndt_calculate_score(lgs_ndt* n, const float* T16, double* score) {
