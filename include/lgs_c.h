@@ -360,6 +360,12 @@ int lgs_icp_step(lgs_icp* icp, const float* guess16, double* sums17, float* T16,
 /* exact k-NN of `queries` in `pts` (the search behind FG:133 and FG:254); idx/d2 are m x k, ascending */
 int lgs_knn(lgs_ctx* ctx, const void* pts, int64_t n, int32_t stride_bytes, const void* queries, int64_t m, int32_t qstride_bytes,
             int32_t k, int32_t* idx, float* d2);
+/* parity hook for the exact 1-NN of the correspondence searches (FG:133, ICP) and of getFitnessScore: idx/d2 are m
+ * entries.  seeds (m entries, or NULL for the unseeded search) start query t from indexed point seeds[t], as the
+ * correspondence searches start from the previous iteration's neighbour; a seed outside [0, n) means none.  The result
+ * does not depend on the seed.  An empty cloud gives idx -1 and d2 +inf.  d2 may be NULL. */
+int lgs_nn_search1(lgs_ctx* ctx, const void* pts, int64_t n, int32_t stride_bytes, const void* queries, int64_t m, int32_t qstride_bytes,
+                   const int32_t* seeds, int32_t* idx, float* d2);
 
 /* parity hook for the device radix sort that orders points by voxel (the std::sort of pcl::VoxelGrid::applyFilter
  * and the std::map iteration order of VGC:218-263): stable sort of n (key, value) pairs by the low `bits` key bits,

@@ -152,6 +152,7 @@ SYMBOLS = {
     "lgs_icp_fitness": (_i32, [_vp, _f64, C.POINTER(_f64)]),
     "lgs_icp_step": (_i32, [_vp, _vp, _vp, _vp, C.POINTER(_i32)]),
     "lgs_knn": (_i32, [_vp, _vp, _i64, _i32, _vp, _i64, _i32, _i32, _vp, _vp]),
+    "lgs_nn_search1": (_i32, [_vp, _vp, _i64, _i32, _vp, _i64, _i32, _vp, _vp, _vp]),
     "lgs_sort_pairs": (_i32, [_vp, _vp, _vp, _i64, _i32]),
     "lgs_keyframes_create": (_i32, [_vp, C.POINTER(_vp)]),
     "lgs_keyframes_destroy": (None, [_vp]),

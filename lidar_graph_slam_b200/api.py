@@ -700,6 +700,25 @@ def knn(pts, queries, k, ctx=None):
     return idx[:m], d2[:m]
 
 
+def nn_search1(pts, queries, seeds=None, ctx=None):
+    """Exact 1-NN of `queries` in `pts` by the search of the correspondence steps (FG:133, ICP), started from seeds[t] (an
+    index into pts; outside [0, n) = no seed) or unseeded when seeds is None.  Returns (idx (m,) int32, d2 (m,) f32);
+    idx -1 and d2 +inf for an empty cloud."""
+    ctx = ctx or default_context()
+    a, pa, n, sa = _host_cloud(pts)
+    q, pq, m, sq = _host_cloud(queries)
+    s = None
+    if seeds is not None:
+        s = np.ascontiguousarray(seeds, dtype=np.int32).ravel()
+        if s.size != m:
+            raise ValueError("need one seed per query")
+    idx = np.empty(max(m, 1), np.int32)
+    d2 = np.empty(max(m, 1), np.float32)
+    vp = lambda x: x.ctypes.data_as(C.c_void_p)
+    check(ctx._L.lgs_nn_search1(ctx._h, pa, n, sa, pq, m, sq, vp(s) if s is not None else None, vp(idx), vp(d2)))
+    return idx[:m], d2[:m]
+
+
 def sort_pairs(keys, vals, bits=32, ctx=None):
     """Stable device radix sort of (uint32 key, uint32 value) pairs by the low `bits` key bits (parity hook for the
     sort that orders points by voxel).  Returns sorted copies."""

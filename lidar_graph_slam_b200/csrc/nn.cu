@@ -322,6 +322,32 @@ __global__ void __launch_bounds__(kKnnBlock) nn_knn_list_kernel(NNView v, const 
   }
 }
 
+// the 1-NN of the correspondence searches (gicp_correspondence_kernel, icp_step_body) with their seed handling: seeds[t]
+// outside [0, n) means no seed, otherwise the search starts from that point of the original (unsorted) cloud `pts`.
+// seeds == nullptr: the unseeded search of getFitnessScore and pclomp GICP.
+__global__ void __launch_bounds__(kKnnBlock) nn_search1_kernel(NNView v, const float4* __restrict__ pts, const float4* __restrict__ queries, int m,
+                                                              const int* __restrict__ seeds, int* __restrict__ out_idx, float* __restrict__ out_d2) {
+  const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
+  for (int t = blockIdx.x * kKnnWarps + warp; t < m; t += gridDim.x * kKnnWarps) {
+    const float4 q = __ldg(queries + t);
+    float d2;
+    int id;
+    if (seeds) {
+      int seed = seeds[t];
+      if (seed >= v.n) seed = -1;
+      float seed_d = 0.f;
+      if (seed >= 0) seed_d = nn_dist2(q.x, q.y, q.z, __ldg(pts + seed));
+      nn_search1_warp_seeded(v, q.x, q.y, q.z, lane, seed_d, seed, d2, id);
+    } else {
+      nn_search1_warp(v, q.x, q.y, q.z, lane, d2, id);
+    }
+    if (lane == 0) {
+      out_idx[t] = id;
+      if (out_d2) out_d2[t] = d2;
+    }
+  }
+}
+
 static int knn_grid(int64_t m) { return static_cast<int>(std::max<int64_t>(1, std::min<int64_t>((m + kKnnWarps - 1) / kKnnWarps, kNumSMs * 64))); }
 
 int nn_self_knn(lgs_ctx* ctx, const NNIndex& index, int k, int* out_idx_dev, float* out_d2_dev) {
@@ -387,6 +413,56 @@ extern "C" int lgs_knn(lgs_ctx* ctx, const void* pts, int64_t n, int32_t stride_
   } while (false);
   cloud.release();
   q.release();
+  oi.release();
+  od.release();
+  index.release();
+  return rc;
+}
+
+extern "C" int lgs_nn_search1(lgs_ctx* ctx, const void* pts, int64_t n, int32_t stride_bytes, const void* queries, int64_t m, int32_t qstride_bytes,
+                              const int32_t* seeds, int32_t* idx, float* d2) {
+  using namespace lgs;
+  LGS_REQUIRE(ctx && idx, "null argument");
+  LGS_TRY(use_device(ctx));
+  DevBuf cloud, q, s, oi, od;
+  NNIndex index;
+  int rc = LGS_OK;
+  do {
+    if ((rc = upload_cloud(ctx, pts, n, stride_bytes, &cloud)) != LGS_OK) break;
+    if ((rc = upload_cloud(ctx, queries, m, qstride_bytes, &q)) != LGS_OK) break;
+    if (m == 0) break;
+    if (n == 0) {  // nothing indexed: no neighbour, at infinite distance
+      for (int64_t t = 0; t < m; t++) {
+        idx[t] = -1;
+        if (d2) d2[t] = std::numeric_limits<float>::infinity();
+      }
+      break;
+    }
+    if ((rc = index.build(ctx, cloud.as<float4>(), n)) != LGS_OK) break;
+    if ((rc = oi.reserve(static_cast<size_t>(m) * 4)) != LGS_OK) break;
+    if ((rc = od.reserve(static_cast<size_t>(m) * 4)) != LGS_OK) break;
+    if (seeds) {
+      if ((rc = s.reserve(static_cast<size_t>(m) * 4)) != LGS_OK) break;
+      cudaMemcpyAsync(s.p, seeds, static_cast<size_t>(m) * 4, cudaMemcpyHostToDevice, ctx->stream);
+    }
+    nn_search1_kernel<<<knn_grid(m), kKnnBlock, 0, ctx->stream>>>(index.view(), cloud.as<float4>(), q.as<float4>(), static_cast<int>(m),
+                                                                  seeds ? s.as<int>() : nullptr, oi.as<int>(), od.as<float>());
+    ctx->launches++;
+    if (cudaGetLastError() != cudaSuccess) {
+      set_error("lgs_nn_search1: launch failed");
+      rc = LGS_ERR_CUDA;
+      break;
+    }
+    cudaMemcpyAsync(idx, oi.p, static_cast<size_t>(m) * 4, cudaMemcpyDeviceToHost, ctx->stream);
+    if (d2) cudaMemcpyAsync(d2, od.p, static_cast<size_t>(m) * 4, cudaMemcpyDeviceToHost, ctx->stream);
+    if (cudaStreamSynchronize(ctx->stream) != cudaSuccess) {
+      set_error("lgs_nn_search1: stream synchronize failed");
+      rc = LGS_ERR_CUDA;
+    }
+  } while (false);
+  cloud.release();
+  q.release();
+  s.release();
   oi.release();
   od.release();
   index.release();
