@@ -465,6 +465,52 @@ class KeyFrameArray {
   lgs_keyframes* h_ = nullptr;
 };
 
+// the flat frame list of lgs_odometry_run*
+struct OdometryInput {
+  std::vector<int32_t> n_frames;
+  std::vector<const void*> frames;
+  std::vector<int64_t> n_points;
+  explicit OdometryInput(const std::vector<std::vector<PointCloud>>& sequences) {
+    for (const auto& seq : sequences) {
+      n_frames.push_back(static_cast<int32_t>(seq.size()));
+      for (const auto& c : seq) {
+        frames.push_back(c.data());
+        n_points.push_back(static_cast<int64_t>(c.size()));
+      }
+    }
+  }
+};
+
+// Offline odometry (lgs_odometry_run): the scan matcher's key-frame loop over each recorded sequence of sensor-frame sweeps.
+// keyframes: empty, or one entry per sequence (nullptr or an empty array on ctx's device, which the run fills).  Returns the
+// records in (sequence, frame) order; throws std::runtime_error with lgs_last_error() when the call is refused or fails.
+inline std::vector<lgs_odometry_frame> odometry(const std::vector<std::vector<PointCloud>>& sequences, const lgs_odometry_params& params,
+                                                const std::vector<Matrix4f>& initial_poses = {}, const std::vector<KeyFrameArray*>& keyframes = {},
+                                                std::shared_ptr<Context> ctx = defaultContext()) {
+  const OdometryInput in(sequences);
+  std::vector<lgs_keyframes*> kf;
+  for (KeyFrameArray* k : keyframes) kf.push_back(k ? k->handle() : nullptr);
+  std::vector<lgs_odometry_frame> out(in.frames.size());
+  const int rc = lgs_odometry_run(ctx->get(), &params, static_cast<int32_t>(sequences.size()), in.n_frames.data(), in.frames.data(), in.n_points.data(),
+                                  sizeof(PointXYZI), initial_poses.empty() ? nullptr : initial_poses[0].data(), kf.empty() ? nullptr : kf.data(),
+                                  out.data());
+  if (rc != LGS_OK) throw std::runtime_error(lgs_last_error());
+  return out;
+}
+
+// lgs_odometry_run_dist (collective over comm, on ctx's device): every rank passes the same sequence list; of the sequences this
+// rank does not own only the cloud sizes are read.  Returns every record on every rank.
+inline std::vector<lgs_odometry_frame> odometryDist(lgs_comm* comm, const std::vector<std::vector<PointCloud>>& sequences, const lgs_odometry_params& params,
+                                                    const std::vector<Matrix4f>& initial_poses = {}, lgs_odometry_dist_info* info = nullptr,
+                                                    std::shared_ptr<Context> ctx = defaultContext()) {
+  const OdometryInput in(sequences);
+  std::vector<lgs_odometry_frame> out(in.frames.size());
+  const int rc = lgs_odometry_run_dist(ctx->get(), comm, &params, static_cast<int32_t>(sequences.size()), in.n_frames.data(), in.frames.data(),
+                                       in.n_points.data(), sizeof(PointXYZI), initial_poses.empty() ? nullptr : initial_poses[0].data(), out.data(), info);
+  if (rc != LGS_OK) throw std::runtime_error(lgs_last_error());
+  return out;
+}
+
 }  // namespace lgs
 
 #ifdef LGS_HAVE_PCL

@@ -484,6 +484,90 @@ int lgs_batch_align_dist(lgs_comm* comm, const lgs_batch_params* params, int64_t
                          const int64_t* n_scan, const void* const* submaps, const int64_t* n_submap, int32_t stride_bytes,
                          const float* guesses16, lgs_align_result* records_all, lgs_batch_dist_info* info);
 
+/* ------------------------------------------------------------------------------------------- */
+/* offline odometry: the scan matcher's key-frame loop (LSM:122-250) over whole recorded sequences */
+/*   per frame: range crop + VoxelGrid + optional SOR in the sensor frame (the prefilter node),   */
+/*   base_from_sensor (LSM:127-131), then frame 0 = key frame 0 and target; frame k > 0 =         */
+/*   setInputSource + align(pose after frame k-1) (LSM:162-165), dropped when not converged       */
+/*   (LSM:167-170); a key frame when |t(T) - t(T_kf)| >= keyframe_displacement (LSM:183), and    */
+/*   then the target = the newest max_scan_accumulate_num key frames, newest first (LSM:187-212). */
+/*   DESIGN.md section 8 records the contract.                                                   */
+typedef struct lgs_odometry_params {
+  int32_t method;                     /* LGS_METHOD_NDT / _GICP / _GICP_OMP (the scan matcher's three, LSM:37-97); ICP is refused */
+  int32_t max_iterations;             /* fields up to max_optimizer_iterations mean what they mean in lgs_batch_params; a value */
+  double transformation_epsilon;      /* <= 0 takes the scan-matcher YAML default (SURVEY Appendix C): NDT resolution 2.0,      */
+  double max_correspondence_distance; /* step 0.1, eps 0.01, 64 iterations; GICP k 20, max correspondence distance 2.0, eps     */
+  int32_t k_correspondences;          /* 0.01, 64 iterations; pclomp GICP 20 BFGS iterations                                  */
+  float ndt_resolution;
+  double ndt_step_size;
+  int32_t max_optimizer_iterations;
+  int32_t max_scan_accumulate_num;    /* key frames in the target window, >= 1 (lidar_scan_matcher.param.yaml: 20) */
+  double keyframe_displacement;       /* metres (param.yaml: 1.0); <= 0 takes 1.0 */
+  double range_min;                   /* keep iff range_min < |p| (PPF:102-112); < 0 disables; needs leaf > 0 (the crop is a VoxelGrid stage) */
+  float leaf;                         /* VoxelGrid leaf (PPF:114-121); <= 0 disables */
+  int32_t sor_mean_k;                 /* StatisticalOutlierRemoval mean_k (PPF:132-140), <= 31; <= 0 disables */
+  double sor_stddev_mul;
+  float base_from_sensor[16];         /* column-major extrinsic (LSM:127-131); all zeros = identity */
+} lgs_odometry_params;
+
+/* One per input frame, in (sequence, frame) order.  Fixed 112 bytes: the distributed run moves it as bytes. */
+typedef struct lgs_odometry_frame {
+  float T[16];               /* pose after the frame (map from base), column-major */
+  double trans_probability;  /* the align's getTransformationProbability (NDT), else 0 */
+  double accum_distance;     /* path length over the key frames so far (LSM:193) */
+  int32_t sequence, frame;
+  int32_t converged;         /* hasConverged(); frame 0 is 1 */
+  int32_t iterations;        /* the align's iteration count; 0 for frame 0 */
+  int32_t evaluations;       /* derivative evaluations (NDT) / linearize or functor calls (GICP) */
+  int32_t keyframe_id;       /* id of the key frame this frame became, -1 if none */
+  int64_t n_source;          /* points after the prefilter */
+} lgs_odometry_frame;
+#ifdef __cplusplus
+static_assert(sizeof(lgs_odometry_frame) == 112, "lgs_odometry_frame is 112 bytes");
+#else
+_Static_assert(sizeof(lgs_odometry_frame) == 112, "lgs_odometry_frame is 112 bytes");
+#endif
+
+/* n_seq sequences; sequence s has n_frames[s] frames.  frames / n_points list the frames of all sequences flat, sequence
+ * after sequence; records receives one record per frame in the same order.  Host form: records of stride_bytes as every host
+ * cloud of this header; frame k+1 is uploaded through pinned staging on a copy stream while frame k aligns.  Device form:
+ * packed xyzi device clouds on ctx's device, read on ctx's stream.  initial_poses: n_seq x 16 column-major or NULL (identity).
+ * keyframes: NULL or n_seq entries, each NULL (the run uses scratch) or an EMPTY array on ctx's device that the run fills
+ * with the sequence's key frames, their poses, accum_distance and f64 positions (ready for detect_loop /
+ * lgs_batch_align_keyframes).  Every sequence starts from fresh registration objects; sequences run one after another.
+ * Every argument is checked before anything runs: a rejected call launches nothing. */
+int lgs_odometry_run(lgs_ctx* ctx, const lgs_odometry_params* params, int32_t n_seq, const int32_t* n_frames, const void* const* frames,
+                     const int64_t* n_points, int32_t stride_bytes, const float* initial_poses, lgs_keyframes* const* keyframes,
+                     lgs_odometry_frame* records);
+int lgs_odometry_run_dev(lgs_ctx* ctx, const lgs_odometry_params* params, int32_t n_seq, const int32_t* n_frames, const float* const* frames_dev,
+                         const int64_t* n_points, const float* initial_poses, lgs_keyframes* const* keyframes, lgs_odometry_frame* records);
+
+/* measurement hook: with LGS_ODOMETRY_PROFILE=1 in the environment the runs of this thread time their stages with CUDA events;
+ * out4 = {frames, prefilter ms (upload + range crop + VoxelGrid + SOR + extrinsic), align ms (setInputSource + align),
+ * key-frame ms (push + target update)} summed since the last call, which clears them. */
+int lgs_odometry_profile(double* out4);
+
+typedef struct lgs_odometry_dist_info {
+  int32_t rank, world;
+  int64_t n_local_sequences;
+  int64_t n_local_frames;
+  int64_t n_received;   /* records that came back from the gather (= all frames on success) */
+  int64_t gather_bytes; /* bytes received by this rank in the ncclAllGather */
+  double run_ms;        /* host wall time of this rank's own sequences */
+  double gather_ms;     /* ncclAllGather + D2H + placement */
+} lgs_odometry_dist_info;
+
+/* Collective over comm (on ctx's device): every rank passes the same n_seq, n_frames and n_points; the sequences are dealt by
+ * lgs_batch_partition over each sequence's total point count; frames of sequences a rank does not own are not read and may
+ * be NULL.  Each rank runs its share as lgs_odometry_run would (scratch key frames) and ONE ncclAllGather returns every
+ * record to every rank in records_all, bit-identical to a one-rank run. */
+int lgs_odometry_run_dist(lgs_ctx* ctx, lgs_comm* comm, const lgs_odometry_params* params, int32_t n_seq, const int32_t* n_frames,
+                          const void* const* frames, const int64_t* n_points, int32_t stride_bytes, const float* initial_poses,
+                          lgs_odometry_frame* records_all, lgs_odometry_dist_info* info);
+int lgs_odometry_run_dist_dev(lgs_ctx* ctx, lgs_comm* comm, const lgs_odometry_params* params, int32_t n_seq, const int32_t* n_frames,
+                              const float* const* frames_dev, const int64_t* n_points, const float* initial_poses,
+                              lgs_odometry_frame* records_all, lgs_odometry_dist_info* info);
+
 /* The per-worker device state of lgs_batch_align (stream, registration objects, staging buffers) is kept in a
  * process-wide pool between calls, the way the reference keeps one registration_ object per node for its lifetime
  * (graph_based_slam.hpp:108).  This frees it (call with no batch in flight, e.g. at node shutdown). */

@@ -54,6 +54,25 @@ class BatchDistInfo(C.Structure):
                 ("verify_ms", C.c_double), ("gather_ms", C.c_double)]
 
 
+class OdometryParams(C.Structure):
+    _fields_ = [("method", C.c_int32), ("max_iterations", C.c_int32), ("transformation_epsilon", C.c_double),
+                ("max_correspondence_distance", C.c_double), ("k_correspondences", C.c_int32), ("ndt_resolution", C.c_float),
+                ("ndt_step_size", C.c_double), ("max_optimizer_iterations", C.c_int32), ("max_scan_accumulate_num", C.c_int32),
+                ("keyframe_displacement", C.c_double), ("range_min", C.c_double), ("leaf", C.c_float), ("sor_mean_k", C.c_int32),
+                ("sor_stddev_mul", C.c_double), ("base_from_sensor", C.c_float * 16)]
+
+
+class OdometryFrame(C.Structure):
+    _fields_ = [("T", C.c_float * 16), ("trans_probability", C.c_double), ("accum_distance", C.c_double), ("sequence", C.c_int32),
+                ("frame", C.c_int32), ("converged", C.c_int32), ("iterations", C.c_int32), ("evaluations", C.c_int32),
+                ("keyframe_id", C.c_int32), ("n_source", C.c_int64)]
+
+
+class OdometryDistInfo(C.Structure):
+    _fields_ = [("rank", C.c_int32), ("world", C.c_int32), ("n_local_sequences", C.c_int64), ("n_local_frames", C.c_int64),
+                ("n_received", C.c_int64), ("gather_bytes", C.c_int64), ("run_ms", C.c_double), ("gather_ms", C.c_double)]
+
+
 # every symbol include/lgs_c.h declares: name -> (restype, argtypes)
 _vp, _i32, _i64, _f32, _f64 = C.c_void_p, C.c_int32, C.c_int64, C.c_float, C.c_double
 SYMBOLS = {
@@ -166,6 +185,11 @@ SYMBOLS = {
     "lgs_keyframes_detect_loop": (_i32, [_vp, _i32, _f64, _f64, _vp, _i32, C.POINTER(_i32), C.POINTER(_i32)]),
     "lgs_batch_align_keyframes": (_i32, [_vp, _vp, C.POINTER(BatchParams), _i64, _vp, _vp, _i32, _vp, _i32, _vp, _vp]),
     "lgs_batch_align": (_i32, [_i32, _vp, C.POINTER(BatchParams), _i64, _vp, _vp, _vp, _vp, _i32, _vp, _i32, _vp, _vp]),
+    "lgs_odometry_run": (_i32, [_vp, C.POINTER(OdometryParams), _i32, _vp, _vp, _vp, _i32, _vp, _vp, _vp]),
+    "lgs_odometry_run_dev": (_i32, [_vp, C.POINTER(OdometryParams), _i32, _vp, _vp, _vp, _vp, _vp, _vp]),
+    "lgs_odometry_profile": (_i32, [_vp]),
+    "lgs_odometry_run_dist": (_i32, [_vp, _vp, C.POINTER(OdometryParams), _i32, _vp, _vp, _vp, _i32, _vp, _vp, C.POINTER(OdometryDistInfo)]),
+    "lgs_odometry_run_dist_dev": (_i32, [_vp, _vp, C.POINTER(OdometryParams), _i32, _vp, _vp, _vp, _vp, _vp, C.POINTER(OdometryDistInfo)]),
     "lgs_batch_release": (None, []),
     "lgs_comm_get_unique_id": (_i32, [_vp]),
     "lgs_comm_init_rank": (_i32, [_vp, _i32, _i32, _i32, C.POINTER(_vp)]),

@@ -13,7 +13,8 @@ import ctypes as C
 import numpy as np
 
 from . import _lib
-from ._lib import AlignResult, BatchDistInfo, BatchParams, NdtGridInfo, Pc2Layout, SorInfo, VoxelGridInfo, check
+from ._lib import (AlignResult, BatchDistInfo, BatchParams, NdtGridInfo, OdometryDistInfo, OdometryFrame, OdometryParams, Pc2Layout, SorInfo,
+                   VoxelGridInfo, check)
 
 NDT_KDTREE, NDT_DIRECT26, NDT_DIRECT7, NDT_DIRECT1 = 0, 1, 2, 3
 REG_NONE, REG_MIN_EIG, REG_NORMALIZED_MIN_EIG, REG_PLANE, REG_FROBENIUS = 0, 1, 2, 3, 4
@@ -882,6 +883,147 @@ def batch_align_dist(comm, scans, submaps, method=METHOD_GICP, guesses=None, max
     info = BatchDistInfo()
     check(L.lgs_batch_align_dist(comm._h, C.byref(bp), n, sp, ns, mp, nm, 16, g.ctypes.data_as(C.c_void_p) if g is not None else None, recs, C.byref(info)))
     return [recs[i] for i in range(n)], _dist_info(info)
+
+
+# lgs_odometry_frame as a numpy record (T is column-major: T.reshape(4, 4, order="F") is the 4x4 pose)
+ODOMETRY_FRAME = np.dtype([("T", "<f4", (16,)), ("trans_probability", "<f8"), ("accum_distance", "<f8"), ("sequence", "<i4"), ("frame", "<i4"),
+                           ("converged", "<i4"), ("iterations", "<i4"), ("evaluations", "<i4"), ("keyframe_id", "<i4"), ("n_source", "<i8")])
+
+
+def odometry_poses(records):
+    """The (N, 4, 4) float32 poses of odometry records."""
+    return np.ascontiguousarray(records["T"].reshape(-1, 4, 4).transpose(0, 2, 1))
+
+
+def _odometry_params(method, keyframe_displacement, max_scan_accumulate_num, range_min, leaf, sor_mean_k, sor_stddev_mul, base_from_sensor,
+                     max_iterations, transformation_epsilon, max_correspondence_distance, k_correspondences, ndt_resolution, ndt_step_size,
+                     max_optimizer_iterations):
+    p = OdometryParams(method=method, max_iterations=max_iterations, transformation_epsilon=transformation_epsilon,
+                       max_correspondence_distance=max_correspondence_distance, k_correspondences=k_correspondences, ndt_resolution=ndt_resolution,
+                       ndt_step_size=ndt_step_size, max_optimizer_iterations=max_optimizer_iterations, max_scan_accumulate_num=max_scan_accumulate_num,
+                       keyframe_displacement=keyframe_displacement, range_min=-1.0 if range_min is None else float(range_min),
+                       leaf=0.0 if leaf is None else float(leaf), sor_mean_k=sor_mean_k, sor_stddev_mul=sor_stddev_mul)
+    E = np.eye(4, dtype=np.float32) if base_from_sensor is None else np.asarray(base_from_sensor, np.float32).reshape(4, 4)
+    p.base_from_sensor[:] = [float(v) for v in E.ravel(order="F")]
+    return p
+
+
+class _OdometryInput:
+    """The flat frame list of lgs_odometry_run*: host clouds (numpy, one record width for all) or packed xyzi CUDA tensors.
+    Sequences that are None (allowed for the distributed run) contribute their frame counts from `n_points`."""
+
+    def __init__(self, sequences, n_points=None, ctx=None):
+        self.n_seq = len(sequences)
+        self.n_frames, self.sizes, ptrs, self._keep = [], [], [], []
+        self.device = None
+        stride = None
+        for s, seq in enumerate(sequences):
+            if seq is None:
+                if n_points is None:
+                    raise ValueError("sequence %d is None: pass n_points" % s)
+                self.n_frames.append(len(n_points[s]))
+                self.sizes += [int(v) for v in n_points[s]]
+                ptrs += [None] * len(n_points[s])
+                continue
+            self.n_frames.append(len(seq))
+            for cloud in seq:
+                if _is_torch(cloud):
+                    if self.device is False:
+                        raise ValueError("a call takes host clouds or CUDA tensors, not both")
+                    p, n = _dev_cloud(cloud, ctx)
+                    self.device = True
+                    self._keep.append(cloud)
+                    ptrs.append(p.value)
+                else:
+                    if self.device is True:
+                        raise ValueError("a call takes host clouds or CUDA tensors, not both")
+                    a, p, n, st = _host_cloud(cloud)
+                    if stride not in (None, st):
+                        raise ValueError("all host clouds of a call need the same record width")
+                    self.device, stride = False, st
+                    self._keep.append(a)
+                    ptrs.append(p.value)
+                self.sizes.append(int(n))
+        if n_points is not None:
+            want = [int(v) for seq in n_points for v in seq]
+            if want != self.sizes:
+                raise ValueError("n_points does not match the clouds")
+        self.device = bool(self.device)
+        self.stride = stride or 16
+        self.total = len(self.sizes)
+        self.nf = (C.c_int32 * max(self.n_seq, 1))(*self.n_frames)
+        self.np = (C.c_int64 * max(self.total, 1))(*self.sizes)
+        self.ptrs = (C.c_void_p * max(self.total, 1))(*ptrs)
+
+
+def _initial_poses(initial_poses, n_seq):
+    if initial_poses is None:
+        return None
+    if len(initial_poses) != n_seq:
+        raise ValueError("need one initial pose per sequence")
+    return _pack_guesses(initial_poses)
+
+
+def odometry(sequences, method=METHOD_NDT, keyframe_displacement=1.0, max_scan_accumulate_num=20, range_min=1.0, leaf=0.1, sor_mean_k=0,
+             sor_stddev_mul=1.0, base_from_sensor=None, initial_poses=None, keyframes=None, max_iterations=0, transformation_epsilon=0.0,
+             max_correspondence_distance=0.0, k_correspondences=0, ndt_resolution=0.0, ndt_step_size=0.0, max_optimizer_iterations=0, ctx=None):
+    """Offline odometry (lgs_odometry_run / _dev): the scan matcher's key-frame loop (LSM:122-250) over each sequence of sweeps in
+    the sensor frame.  sequences: a list of sequences, each a list (or a stacked array / tensor) of clouds, all numpy host clouds
+    or all CUDA (N, 4) tensors.  leaf / range_min None disable the VoxelGrid / range crop (the crop needs the VoxelGrid);
+    sor_mean_k 0 disables the outlier filter.  Registration settings left at 0 take the scan-matcher YAML defaults.
+    keyframes: None or one entry per sequence, each None or an empty KeyFrameArray on the same context, which the run fills.
+    Returns a numpy structured array (ODOMETRY_FRAME) with one record per frame, in (sequence, frame) order."""
+    ctx = ctx or default_context()
+    inp = _OdometryInput(sequences, ctx=ctx)
+    p = _odometry_params(method, keyframe_displacement, max_scan_accumulate_num, range_min, leaf, sor_mean_k, sor_stddev_mul, base_from_sensor,
+                         max_iterations, transformation_epsilon, max_correspondence_distance, k_correspondences, ndt_resolution, ndt_step_size,
+                         max_optimizer_iterations)
+    g = _initial_poses(initial_poses, inp.n_seq)
+    gp = g.ctypes.data_as(C.c_void_p) if g is not None else None
+    kfs = None
+    if keyframes is not None:
+        if len(keyframes) != inp.n_seq:
+            raise ValueError("need one keyframes entry per sequence")
+        kfs = (C.c_void_p * max(inp.n_seq, 1))(*[None if k is None else k._h.value for k in keyframes])
+    recs = np.zeros(max(inp.total, 1), ODOMETRY_FRAME)
+    rp = recs.ctypes.data_as(C.c_void_p)
+    if inp.device:
+        check(ctx._L.lgs_odometry_run_dev(ctx._h, C.byref(p), inp.n_seq, inp.nf, inp.ptrs, inp.np, gp, kfs, rp))
+    else:
+        check(ctx._L.lgs_odometry_run(ctx._h, C.byref(p), inp.n_seq, inp.nf, inp.ptrs, inp.np, inp.stride, gp, kfs, rp))
+    return recs[: inp.total]
+
+
+def odometry_dist(comm, sequences, n_points=None, method=METHOD_NDT, keyframe_displacement=1.0, max_scan_accumulate_num=20, range_min=1.0, leaf=0.1,
+                  sor_mean_k=0, sor_stddev_mul=1.0, base_from_sensor=None, initial_poses=None, max_iterations=0, transformation_epsilon=0.0,
+                  max_correspondence_distance=0.0, k_correspondences=0, ndt_resolution=0.0, ndt_step_size=0.0, max_optimizer_iterations=0, ctx=None):
+    """lgs_odometry_run_dist / _dev (collective over `comm`, ctx on comm's device): every rank passes the same sequence list;
+    a sequence this rank does not own may be None when n_points (per sequence, the point count of every frame) is given.
+    Returns (records of every frame of every sequence, info dict)."""
+    ctx = ctx or default_context()
+    inp = _OdometryInput(sequences, n_points, ctx=ctx)
+    p = _odometry_params(method, keyframe_displacement, max_scan_accumulate_num, range_min, leaf, sor_mean_k, sor_stddev_mul, base_from_sensor,
+                         max_iterations, transformation_epsilon, max_correspondence_distance, k_correspondences, ndt_resolution, ndt_step_size,
+                         max_optimizer_iterations)
+    g = _initial_poses(initial_poses, inp.n_seq)
+    gp = g.ctypes.data_as(C.c_void_p) if g is not None else None
+    recs = np.zeros(max(inp.total, 1), ODOMETRY_FRAME)
+    rp = recs.ctypes.data_as(C.c_void_p)
+    info = OdometryDistInfo()
+    if inp.device:
+        check(ctx._L.lgs_odometry_run_dist_dev(ctx._h, comm._h, C.byref(p), inp.n_seq, inp.nf, inp.ptrs, inp.np, gp, rp, C.byref(info)))
+    else:
+        check(ctx._L.lgs_odometry_run_dist(ctx._h, comm._h, C.byref(p), inp.n_seq, inp.nf, inp.ptrs, inp.np, inp.stride, gp, rp, C.byref(info)))
+    return recs[: inp.total], dict(rank=info.rank, world=info.world, n_local_sequences=info.n_local_sequences, n_local_frames=info.n_local_frames,
+                                   n_received=info.n_received, gather_bytes=info.gather_bytes, run_ms=info.run_ms, gather_ms=info.gather_ms)
+
+
+def odometry_profile():
+    """lgs_odometry_profile: with LGS_ODOMETRY_PROFILE=1 set before the runs, the CUDA-event split of this thread's odometry frames
+    since the last call (which clears it)."""
+    out = np.zeros(4)
+    check(_lib.load().lgs_odometry_profile(out.ctypes.data_as(C.c_void_p)))
+    return dict(frames=int(out[0]), prefilter_ms=out[1], align_ms=out[2], keyframe_ms=out[3])
 
 
 def batch_release():

@@ -416,7 +416,16 @@ int run_dist(lgs_comm* comm, int device, const int64_t* sizes, int64_t n_pairs, 
   LGS_TRY(run_batch(S));
   const auto t1 = std::chrono::steady_clock::now();
   int64_t got = 0;
-  LGS_TRY(comm_all_gather_records(comm, st, cap, n_pairs, records_all, &got));
+  LGS_TRY(comm_all_gather(comm, st, cap, sizeof(lgs_align_result), [&](const void* p) {
+    const lgs_align_result* r = static_cast<const lgs_align_result*>(p);
+    if (r->pair_id < 0) return 0;  // unused slot of a rank with fewer pairs
+    if (r->pair_id >= n_pairs) {
+      set_error("gathered record carries pair id %d outside [0, %lld)", r->pair_id, static_cast<long long>(n_pairs));
+      return LGS_ERR_STATE;
+    }
+    records_all[r->pair_id] = *r;
+    return 1;
+  }, &got));
   const auto t2 = std::chrono::steady_clock::now();
   if (info) {
     info->rank = comm->rank;

@@ -162,6 +162,8 @@ inline int use_device(const lgs_ctx* c) {
 
 // Upload a host cloud with arbitrary record stride into packed float4 xyzi device storage.
 int upload_cloud(lgs_ctx* ctx, const void* pts, int64_t n, int32_t stride_bytes, DevBuf* dst);
+// The repack half of upload_cloud: n records of stride_bytes already in device memory -> packed float4 xyzi, on ctx's stream.
+int repack_cloud(lgs_ctx* ctx, const void* raw_dev, int64_t n, int32_t stride_bytes, float4* dst);
 // The input of every registration set_source / set_target entry point, validated on the host before anything is copied:
 // host records of stride_bytes each (as upload_cloud) or, on_device, a packed float4 xyzi device array (copied device to
 // device; stride_bytes unused).  pts may be null only when n == 0.

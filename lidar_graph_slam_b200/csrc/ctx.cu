@@ -46,8 +46,13 @@ int upload_cloud(lgs_ctx* ctx, const void* pts, int64_t n, int32_t stride, DevBu
   }
   LGS_TRY(ctx->raw.reserve(static_cast<size_t>(n) * stride));
   LGS_CUDA(cudaMemcpyAsync(ctx->raw.p, pts, static_cast<size_t>(n) * stride, cudaMemcpyHostToDevice, ctx->stream));
+  return repack_cloud(ctx, ctx->raw.p, n, stride, dst->as<float4>());
+}
+
+int repack_cloud(lgs_ctx* ctx, const void* raw_dev, int64_t n, int32_t stride, float4* dst) {
+  if (n == 0) return LGS_OK;
   int ioff = stride >= 20 ? 16 : -1;
-  repack_kernel<<<grid_for(n, 256), 256, 0, ctx->stream>>>(ctx->raw.as<unsigned char>(), n, stride, ioff, dst->as<float4>());
+  repack_kernel<<<grid_for(n, 256), 256, 0, ctx->stream>>>(static_cast<const unsigned char*>(raw_dev), n, stride, ioff, dst);
   ctx->launches++;
   LGS_CUDA(cudaGetLastError());
   return LGS_OK;

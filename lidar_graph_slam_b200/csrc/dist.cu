@@ -1,7 +1,7 @@
-// Multi-GPU plumbing of the loop-closure batch (SURVEY section 8e): one process per GPU, candidate pairs dealt to the
-// ranks by size with no data-path collective, and ONE ncclAllGather of the fixed 96-byte result records over
-// NVLink / NVSwitch.  The records are written into the send buffer by the last kernel of each pair (nn.cu), so nothing
-// is staged between the verification and the collective.
+// Multi-GPU plumbing of the loop-closure batch and of offline odometry (SURVEY section 8e): one process per GPU, work
+// items (candidate pairs, sequences) dealt to the ranks by size with no data-path collective, and ONE ncclAllGather of
+// fixed-size result records over NVLink / NVSwitch.  The batch's 96-byte records are written into the send buffer by the
+// last kernel of each pair (nn.cu), so nothing is staged between the verification and the collective.
 //
 // NCCL is bound at run time (dlopen): a process that already holds a libnccl (PyTorch ships its own) keeps using that
 // one, a plain C++ host gets the system library, and a single-GPU user of liblgs_b200.so needs no NCCL at all.
@@ -96,26 +96,21 @@ void partition_pairs(const int64_t* sizes, int64_t n_total, int rank, int world,
   std::sort(mine->begin(), mine->end());
 }
 
-int comm_all_gather_records(lgs_comm* c, cudaStream_t st, int64_t cap, int64_t n_total, lgs_align_result* records_all, int64_t* n_received) {
+int comm_all_gather(lgs_comm* c, cudaStream_t st, int64_t cap, size_t record_bytes, const std::function<int(const void*)>& place, int64_t* n_received) {
   NcclApi* api = nullptr;
   LGS_TRY(require_nccl(&api));
-  const size_t bytes = static_cast<size_t>(cap) * sizeof(lgs_align_result);
+  const size_t bytes = static_cast<size_t>(cap) * record_bytes;
   LGS_TRY(c->recv.reserve(bytes * c->world));
   LGS_TRY(c->host.reserve(bytes * c->world));
   LGS_NCCL(api, api->AllGather(c->send.p, c->recv.p, bytes, ncclInt8, static_cast<ncclComm_t>(c->comm), st));
   LGS_CUDA(cudaMemcpyAsync(c->host.p, c->recv.p, bytes * c->world, cudaMemcpyDeviceToHost, st));
   LGS_CUDA(cudaStreamSynchronize(st));
-  const lgs_align_result* h = c->host.as<lgs_align_result>();
+  const unsigned char* h = c->host.as<unsigned char>();
   int64_t got = 0;
   for (int64_t i = 0; i < cap * c->world; i++) {
-    const int32_t id = h[i].pair_id;
-    if (id < 0) continue;  // unused slot of a rank with fewer pairs
-    if (id >= n_total) {
-      set_error("gathered record carries pair id %d outside [0, %lld)", id, static_cast<long long>(n_total));
-      return LGS_ERR_STATE;
-    }
-    records_all[id] = h[i];
-    got++;
+    const int r = place(h + static_cast<size_t>(i) * record_bytes);
+    if (r < 0) return r;
+    got += r;
   }
   if (n_received) *n_received = got;
   return LGS_OK;

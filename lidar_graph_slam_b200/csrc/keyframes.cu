@@ -137,6 +137,7 @@ int keyframes_wait_resident(const lgs_keyframes* kf) {
 }
 int64_t keyframes_count(const lgs_keyframes* kf) { return static_cast<int64_t>(kf->frames.size()); }
 int keyframes_device(const lgs_keyframes* kf) { return kf->ctx->device; }
+cudaStream_t keyframes_stream(const lgs_keyframes* kf) { return kf->ctx->stream; }
 const float* keyframes_pose(const lgs_keyframes* kf, int64_t id) { return kf->frames[static_cast<size_t>(id)].pose; }
 int64_t keyframes_points(const lgs_keyframes* kf, int64_t id) { return kf->frames[static_cast<size_t>(id)].n; }
 

@@ -15,6 +15,7 @@ int keyframes_wait_resident(const lgs_keyframes* kf);
 int64_t keyframes_count(const lgs_keyframes* kf);
 int64_t keyframes_points(const lgs_keyframes* kf, int64_t id);  // points of key frame id
 int keyframes_device(const lgs_keyframes* kf);
+cudaStream_t keyframes_stream(const lgs_keyframes* kf);  // the stream pushes copy on (that of the array's context)
 const float* keyframes_pose(const lgs_keyframes* kf, int64_t id);  // column-major 4x4 of key frame id
 
 }  // namespace lgs
