@@ -372,6 +372,27 @@ int lgs_nn_search1(lgs_ctx* ctx, const void* pts, int64_t n, int32_t stride_byte
  * in place in the caller's host arrays */
 int lgs_sort_pairs(lgs_ctx* ctx, uint32_t* keys, uint32_t* vals, int64_t n, int32_t bits);
 
+/* parity hook for the small dense solvers the kernels run per voxel, per point and per Newton step (csrc/math.cuh,
+ * csrc/ndt_opt.cuh): n independent problems, one GPU thread each, f64 in and f64 out, row-major, every output bit as the
+ * device computes it.  in holds n records of LGS_LINALG_IN(op) doubles, out receives n records of LGS_LINALG_OUT(op).
+ *   LGS_LINALG_SVD3        A[9]        -> U[9], S[3], V[9]        svd_jacobi<3, double> (FastGICP / pclomp GICP covariances)
+ *   LGS_LINALG_EIG3        A[9]        -> w[3], Q[9], ok          eig_sym3, lower triangle read (NDT voxel covariances)
+ *   LGS_LINALG_INV3        A[9]        -> A^-1[9]                 inv3
+ *   LGS_LINALG_SVD_SOLVE6  H[36], b[6] -> x[6]                    svd_solve<6> (the JacobiSVD Newton step)
+ *   LGS_LINALG_SCHUR6      H[36], b[6] -> x[6], accepted          schur_solve6 (x as left when declined)
+ *   LGS_LINALG_NEWTON6     H[36], b[6] -> x[6], x_exact[6]        the NDT optimiser's step rule: Schur, else JacobiSVD;
+ *                                                                 then with the exact Newton step on (JacobiSVD only)
+ * Flags are 1.0 / 0.0.  An unknown op, n < 0 or a null pointer with n > 0 is LGS_ERR_INVALID and launches nothing. */
+#define LGS_LINALG_SVD3 0
+#define LGS_LINALG_EIG3 1
+#define LGS_LINALG_INV3 2
+#define LGS_LINALG_SVD_SOLVE6 3
+#define LGS_LINALG_SCHUR6 4
+#define LGS_LINALG_NEWTON6 5
+#define LGS_LINALG_IN(op) ((op) <= LGS_LINALG_INV3 ? 9 : 42)
+#define LGS_LINALG_OUT(op) ((op) == LGS_LINALG_SVD3 ? 21 : (op) == LGS_LINALG_EIG3 ? 13 : (op) == LGS_LINALG_INV3 ? 9 : (op) == LGS_LINALG_SVD_SOLVE6 ? 6 : (op) == LGS_LINALG_SCHUR6 ? 7 : 12)
+int lgs_linalg_batch(lgs_ctx* ctx, int32_t op, int64_t n, const double* in, double* out);
+
 /* ------------------------------------------------------------------------------------------- */
 /* key-frame array + sub-map assembly, device resident                                            */
 /*   replaces the per-key-frame fromROSMsg + transform_point_cloud + `*cloud += ...` loops and the */

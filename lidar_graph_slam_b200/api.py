@@ -731,6 +731,24 @@ def sort_pairs(keys, vals, bits=32, ctx=None):
     return k, v
 
 
+LINALG_SVD3, LINALG_EIG3, LINALG_INV3, LINALG_SVD_SOLVE6, LINALG_SCHUR6, LINALG_NEWTON6 = 0, 1, 2, 3, 4, 5
+LINALG_SHAPES = {0: (9, 21), 1: (9, 13), 2: (9, 9), 3: (42, 6), 4: (42, 7), 5: (42, 12)}  # op -> (input, output) doubles
+
+
+def linalg_batch(op, inputs, ctx=None):
+    """The device's small dense solvers, one problem per GPU thread (parity hook lgs_linalg_batch): inputs (n, 9) for
+    SVD3 / EIG3 / INV3, (n, 42) = H row-major + b for SVD_SOLVE6 / SCHUR6 / NEWTON6.  Returns (n, width) f64 as laid out
+    in lgs_c.h."""
+    ctx = ctx or default_context()
+    if op not in LINALG_SHAPES:
+        raise ValueError("unknown linalg op %r" % (op,))
+    nin, nout = LINALG_SHAPES[op]
+    a = np.ascontiguousarray(inputs, dtype=np.float64).reshape(-1, nin)
+    out = np.empty((a.shape[0], nout))
+    check(ctx._L.lgs_linalg_batch(ctx._h, int(op), a.shape[0], a.ctypes.data_as(C.c_void_p), out.ctypes.data_as(C.c_void_p)))
+    return out
+
+
 def batch_align(scans, submaps, method=METHOD_GICP, guesses=None, device=0, stream=None, pair_id0=0, records_dev=None, max_iterations=100,
                 transformation_epsilon=0.01, max_correspondence_distance=2.0, k_correspondences=20, ndt_resolution=1.0, ndt_step_size=0.1,
                 submap_leaf=0.5, fitness_max_range=-1.0, n_workers=0, max_optimizer_iterations=0, euclidean_fitness_epsilon=0.0):

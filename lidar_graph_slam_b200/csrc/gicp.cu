@@ -72,10 +72,10 @@ __global__ void __launch_bounds__(128) gicp_covariance_kernel(NNView v, const fl
     if (regularization == LGS_REG_PLANE) {
       val[0] = 1; val[1] = 1; val[2] = 1e-3;
     } else if (regularization == LGS_REG_MIN_EIG) {
-      for (int a = 0; a < 3; a++) val[a] = fmax(S[a], 1e-3);
-    } else {
-      const double mx = fmax(S[0], fmax(S[1], S[2]));
-      for (int a = 0; a < 3; a++) val[a] = fmax(S[a] / mx, 1e-3);
+      for (int a = 0; a < 3; a++) val[a] = m::tmax(S[a], 1e-3);
+    } else {  // std::max as the reference's Array max: 0 / 0 of an all-zero covariance stays NaN (fmax would give 1e-3)
+      const double mx = m::tmax(S[0], m::tmax(S[1], S[2]));
+      for (int a = 0; a < 3; a++) val[a] = m::tmax(S[a] / mx, 1e-3);
     }
     double UD[9];
     for (int r = 0; r < 3; r++)

@@ -30,12 +30,15 @@ struct Lim<float> {
   static LGS_HD float tiny() { return FLT_MIN; }
 };
 
+// clears the sign bit, as std::fabs: -0.0 -> +0.0 (a compare-and-negate keeps -0.0, and S / eigenvalues would differ in sign)
+LGS_HD double tabs(double v) { return fabs(v); }
+LGS_HD float tabs(float v) { return fabsf(v); }
+// std::max / std::min (and Eigen's maxi / mini): the first argument unless the second compares larger (smaller), so a NaN
+// second argument is skipped, and maxima are taken left to right as the reference's loops take them
 template <typename T>
-LGS_HD T tabs(T v) { return v < T(0) ? -v : v; }
+LGS_HD T tmax(T a, T b) { return a < b ? b : a; }
 template <typename T>
-LGS_HD T tmax(T a, T b) { return a > b ? a : b; }
-template <typename T>
-LGS_HD T tmin(T a, T b) { return a < b ? a : b; }
+LGS_HD T tmin(T a, T b) { return b < a ? b : a; }
 LGS_HD double tsqrt(double v) { return sqrt(v); }
 LGS_HD float tsqrt(float v) { return sqrtf(v); }
 
@@ -203,7 +206,7 @@ LGS_HD void mul3(const double* a, const double* b, double* c) {
 // in the columns of Q.
 LGS_HD bool eig_sym3(const double* A, double* w, double* Q) {
   double a00 = A[0], a10 = A[3], a11 = A[4], a20 = A[6], a21 = A[7], a22 = A[8];
-  double scale = tmax(tmax(tmax(tabs(a00), tabs(a10)), tmax(tabs(a11), tabs(a20))), tmax(tabs(a21), tabs(a22)));
+  double scale = tmax(tmax(tmax(tmax(tmax(tmax(0.0, tabs(a00)), tabs(a10)), tabs(a11)), tabs(a20)), tabs(a21)), tabs(a22));
   if (scale == 0.0) scale = 1.0;
   a00 /= scale; a10 /= scale; a11 /= scale; a20 /= scale; a21 /= scale; a22 /= scale;
   double d[3], e[2];

@@ -415,9 +415,10 @@ LGS_HD bool schur_solve6(const double* H, const double* b, double* x) {
   return true;
 }
 
-// JacobiSVD with Eigen's rank threshold, as the reference; out of line on the device (rare, large stack frame)
+// JacobiSVD with Eigen's rank threshold, as the reference; out of line on the device (rare, large stack frame).  inline:
+// several translation units include this header.
 #if defined(__CUDACC__)
-__host__ __device__ __noinline__
+__host__ __device__ __noinline__ inline
 #else
 inline
 #endif

@@ -5,6 +5,7 @@
 #include <omp.h>
 #endif
 
+#include "linalg.hpp"
 #include "oracle.hpp"
 
 using namespace lgs_oracle;
@@ -318,6 +319,48 @@ void orc_knn(const float* pts, long n, const float* queries, long m, int k, int*
       d2[i * k + j] = 0;
     }
   }
+}
+
+// ---- the small dense solvers (linalg.hpp), n problems, f64 in and out, row-major ----------------
+//   0 jacobi_svd<3>          A[9]        -> U[9], S[3], V[9]
+//   1 self_adjoint_eigen3    A[9]        -> w[3], Q[9], ok
+//   2 inverse3               A[9]        -> A^-1[9]
+//   3 jacobi_svd_solve<6>    H[36], b[6] -> x[6]
+//  16 jacobi_svd<3, float>   A[9]        -> U[9], S[3], V[9]   (inputs rounded to float, results widened exactly)
+//  17 ldlt_solve6            H[36], b[6] -> x[6]
+// Returns 0, or -1 for an unknown op.
+int orc_linalg_batch(int op, long n, const double* in, double* out) {
+  int nin, nout;
+  switch (op) {
+    case 0: case 16: nin = 9; nout = 21; break;
+    case 1: nin = 9; nout = 13; break;
+    case 2: nin = 9; nout = 9; break;
+    case 3: case 17: nin = 42; nout = 6; break;
+    default: return -1;
+  }
+  for (long t = 0; t < n; t++) {
+    const double* a = in + t * nin;
+    double* o = out + t * nout;
+    if (op == 0) {
+      jacobi_svd<3, double>(a, o, o + 9, o + 12);
+    } else if (op == 1) {
+      o[12] = self_adjoint_eigen3(a, o, o + 3) ? 1.0 : 0.0;
+    } else if (op == 2) {
+      inverse3(a, o);
+    } else if (op == 3) {
+      jacobi_svd_solve<6>(a, a + 36, o);
+    } else if (op == 16) {
+      float af[9], U[9], S[3], V[9];
+      for (int i = 0; i < 9; i++) af[i] = static_cast<float>(a[i]);
+      jacobi_svd<3, float>(af, U, S, V);
+      for (int i = 0; i < 9; i++) o[i] = U[i];
+      for (int i = 0; i < 3; i++) o[9 + i] = S[i];
+      for (int i = 0; i < 9; i++) o[12 + i] = V[i];
+    } else {
+      ldlt_solve6(a, a + 36, o);
+    }
+  }
+  return 0;
 }
 
 double orc_fitness(const float* tgt, long nt, const float* src, long ns, const float* T16, double max_range, int num_threads) {

@@ -104,6 +104,8 @@ def lib():
         L.orc_sor_out_n.argtypes = [vp]
         L.orc_sor_get.argtypes = [vp] * 5
         L.orc_sor_free.argtypes = [vp]
+        L.orc_linalg_batch.restype = C.c_int
+        L.orc_linalg_batch.argtypes = [C.c_int, C.c_long, vp, vp]
         _lib = L
     return _lib
 
@@ -514,6 +516,22 @@ def knn(pts, queries, k, num_threads=0):
     d2 = np.empty((m, k), np.float32)
     lib().orc_knn(_p(pts), pts.shape[0], _p(queries), m, int(k), _p(idx), _p(d2), num_threads or max_threads())
     return idx, d2
+
+
+LINALG_SVD3, LINALG_EIG3, LINALG_INV3, LINALG_SVD_SOLVE6, LINALG_SVD3_F32, LINALG_LDLT6 = 0, 1, 2, 3, 16, 17
+_LINALG_SHAPES = {0: (9, 21), 1: (9, 13), 2: (9, 9), 3: (42, 6), 16: (9, 21), 17: (42, 6)}
+
+
+def linalg_batch(op, inputs):
+    """The solvers of linalg.hpp over a batch: inputs (n, 9) for the 3x3 ops, (n, 42) = H row-major + b for the 6x6
+    ones.  Returns (n, width) f64 in the layout of lgs_linalg_batch (LINALG_SVD3_F32: f32 inputs and results, exactly
+    widened)."""
+    nin, nout = _LINALG_SHAPES[op]
+    a = np.ascontiguousarray(inputs, dtype=np.float64).reshape(-1, nin)
+    out = np.empty((a.shape[0], nout))
+    if lib().orc_linalg_batch(int(op), a.shape[0], _p(a), _p(out)) != 0:
+        raise ValueError("unknown linalg op %d" % op)
+    return out
 
 
 def fitness(target, source, T, max_range=np.finfo(np.float64).max, num_threads=0):
