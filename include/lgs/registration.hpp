@@ -63,21 +63,30 @@ class VoxelGrid {
   void setRangeCrop(double min_distance) { range_min_ = min_distance; }
   void setBoxCrop(const std::array<double, 6>& box) { box_ = box; use_box_ = true; }
   void setInputCloud(const std::shared_ptr<const PointCloud>& cloud) { input_ = cloud; }
+  // the wide VoxelGrid (lgs_voxelgrid_filter_wide): a 64-bit voxel index, so grids beyond INT32_MAX cells are filtered
+  // instead of refused; the per-point index then lands in wideVoxelIndices()
+  void setWideIndices(bool wide) { wide_ = wide; }
   void filter(PointCloud& output) {
     output.clear();
     if (!input_) return;
     const int64_t n = static_cast<int64_t>(input_->size());
     std::vector<float> packed(static_cast<size_t>(n > 0 ? n : 1) * 4);
-    voxel_idx_.assign(static_cast<size_t>(n), -1);
+    voxel_idx_.assign(wide_ ? 0 : static_cast<size_t>(n), -1);
+    voxel_idx64_.assign(wide_ ? static_cast<size_t>(n) : 0, -1);
     member_rank_.assign(static_cast<size_t>(n), -1);
-    ok_ = lgs_voxelgrid_filter(ctx_->get(), input_->data(), n, sizeof(PointXYZI), leaf_.data(), min_pts_, range_min_,
-                               use_box_ ? box_.data() : nullptr, packed.data(), voxel_idx_.data(), member_rank_.data(), &info_) == LGS_OK;
+    if (wide_)
+      ok_ = lgs_voxelgrid_filter_wide(ctx_->get(), input_->data(), n, sizeof(PointXYZI), leaf_.data(), min_pts_, range_min_,
+                                      use_box_ ? box_.data() : nullptr, packed.data(), voxel_idx64_.data(), member_rank_.data(), &info_) == LGS_OK;
+    else
+      ok_ = lgs_voxelgrid_filter(ctx_->get(), input_->data(), n, sizeof(PointXYZI), leaf_.data(), min_pts_, range_min_,
+                                 use_box_ ? box_.data() : nullptr, packed.data(), voxel_idx_.data(), member_rank_.data(), &info_) == LGS_OK;
     if (!ok_) return;
     output.resize(static_cast<size_t>(info_.n_out));
     for (int64_t i = 0; i < info_.n_out; i++)
       output[i] = PointXYZI{packed[4 * i], packed[4 * i + 1], packed[4 * i + 2], 1.0f, packed[4 * i + 3], 0, 0, 0};
   }
   const std::vector<int32_t>& voxelIndices() const { return voxel_idx_; }
+  const std::vector<int64_t>& wideVoxelIndices() const { return voxel_idx64_; }
   const std::vector<int32_t>& memberRanks() const { return member_rank_; }
   const lgs_voxelgrid_info& info() const { return info_; }
   bool ok() const { return ok_; }
@@ -88,9 +97,10 @@ class VoxelGrid {
   int min_pts_ = 0;
   double range_min_ = -1.0;
   std::array<double, 6> box_{};
-  bool use_box_ = false, ok_ = true;
+  bool use_box_ = false, ok_ = true, wide_ = false;
   std::shared_ptr<const PointCloud> input_;
   std::vector<int32_t> voxel_idx_, member_rank_;
+  std::vector<int64_t> voxel_idx64_;
   lgs_voxelgrid_info info_{};
 };
 
@@ -455,6 +465,14 @@ class KeyFrameArray {
   bool assemble(const std::vector<int32_t>& ids, float leaf, const float** cloud_dev, int64_t* n) {
     float* p = nullptr;
     const int rc = lgs_keyframes_assemble(h_, ids.data(), static_cast<int32_t>(ids.size()), leaf, &p, n);
+    *cloud_dev = p;
+    return rc == LGS_OK;
+  }
+  // save_map's map (GBS:469-501, lgs_keyframes_export_map): the key frames `ids` (empty: all of them) at their poses,
+  // then the wide VoxelGrid with `leaf` (<= 0: none); a device cloud valid until the next assemble or export
+  bool exportMap(const std::vector<int32_t>& ids, float leaf, const float** cloud_dev, int64_t* n, lgs_voxelgrid_info* info = nullptr) {
+    float* p = nullptr;
+    const int rc = lgs_keyframes_export_map(h_, ids.empty() ? nullptr : ids.data(), static_cast<int32_t>(ids.size()), leaf, &p, n, info);
     *cloud_dev = p;
     return rc == LGS_OK;
   }

@@ -57,7 +57,7 @@ int64_t lgs_ctx_launch_count(const lgs_ctx* ctx);
 /*   replaces PPF:102-112 (distance_filter), PPF:89-100 (crop), PPF:114-121 (downsample ->        */
 /*   VoxelGrid::setLeafSize/setInputCloud/filter) and the VoxelGrid calls at GBS:311-313,490-493 */
 #define LGS_VG_OK 0
-#define LGS_VG_REFUSED_OVERFLOW 1 /* dx*dy*dz > INT32_MAX: like pcl::VoxelGrid, output = cropped input */
+#define LGS_VG_REFUSED_OVERFLOW 1 /* dx*dy*dz > INT32_MAX (wide grid: its own limits): like pcl::VoxelGrid, output = cropped input */
 
 typedef struct lgs_voxelgrid_info {
   int32_t status;    /* LGS_VG_OK or LGS_VG_REFUSED_OVERFLOW */
@@ -83,6 +83,23 @@ int lgs_voxelgrid_filter(lgs_ctx* ctx, const void* pts, int64_t n, int32_t strid
 int lgs_voxelgrid_filter_dev(lgs_ctx* ctx, const float* pts_dev, int64_t n, const float leaf[3],
                              int32_t min_points_per_voxel, double range_min, const double* box6, float* out_pts_dev,
                              int32_t* out_voxel_idx_dev, int32_t* out_member_rank_dev, lgs_voxelgrid_info* info);
+
+/* Wide VoxelGrid: the same computation with the linear voxel index formed in int64, for grids beyond pcl::VoxelGrid's
+ * INT32_MAX cells (whole maps at save_map resolutions, GBS:469-501; the 32-bit limit is the one restated at VGC:75-84).
+ *   - Wherever lgs_voxelgrid_filter does not refuse (and min_b / max_b fit int32, which that call does not check), the
+ *     result is bit-identical to it: points, n_out, n_kept, min_b,
+ *     max_b, div_b, membership, and the voxel index widened to int64 (-1 for a cropped or non-finite point).
+ *   - Beyond that the per-axis cell index keeps PCL's f32 expression int(floor(x*inv) - float(min_b)), the output is in
+ *     ascending 64-bit index, and the centroids are sequential f32 sums over the members in ascending point index.
+ *   - Refusal (LGS_VG_REFUSED_OVERFLOW, output = cropped input in original order) only when an axis spans >= 2^31 cells,
+ *     when min_b or max_b does not fit int32, or when div_b[0]*div_b[1]*div_b[2] exceeds 2^63 - 1.
+ * Every argument is checked before anything runs (n < 2^31, leaf > 0, pts not NULL when n > 0). */
+int lgs_voxelgrid_filter_wide(lgs_ctx* ctx, const void* pts, int64_t n, int32_t stride_bytes, const float leaf[3],
+                              int32_t min_points_per_voxel, double range_min, const double* box6, float* out_pts,
+                              int64_t* out_voxel_idx, int32_t* out_member_rank, lgs_voxelgrid_info* info);
+int lgs_voxelgrid_filter_wide_dev(lgs_ctx* ctx, const float* pts_dev, int64_t n, const float leaf[3],
+                                  int32_t min_points_per_voxel, double range_min, const double* box6, float* out_pts_dev,
+                                  int64_t* out_voxel_idx_dev, int32_t* out_member_rank_dev, lgs_voxelgrid_info* info);
 
 /* ------------------------------------------------------------------------------------------- */
 /* prefilter, second stage: pcl::StatisticalOutlierRemoval<PointXYZI>                            */
@@ -422,6 +439,14 @@ int lgs_keyframes_detect_loop(lgs_keyframes* kf, int32_t latest_id, double accum
  * pcl::VoxelGrid(leaf) to the result (GBS:311-313).  *out_dev is a packed xyzi device cloud owned by kf, valid
  * until the next assemble call; feed it to lgs_*_set_target_dev / set_source_dev. */
 int lgs_keyframes_assemble(lgs_keyframes* kf, const int32_t* ids, int32_t n_ids, float leaf, float** out_dev, int64_t* n_out);
+/* The map of save_map (GBS:469-501): every key frame (ids == NULL, n_ids == 0; id order) or the listed ones in the order
+ * given, each at its current pose, concatenated as lgs_keyframes_assemble does, then the wide VoxelGrid with `leaf`
+ * (lgs_voxelgrid_filter_wide; leaf <= 0: no grid).  Bit-identical to lgs_voxelgrid_filter_wide_dev(assemble(ids, 0)),
+ * and to lgs_keyframes_assemble(ids, leaf) wherever the 32-bit grid does not refuse (VGC:75-84).  *out_dev is a packed
+ * xyzi device cloud owned by kf, valid until the next assemble or export call.  info (may be NULL) receives the grid's
+ * record.  Every argument is checked before anything runs. */
+int lgs_keyframes_export_map(lgs_keyframes* kf, const int32_t* ids, int32_t n_ids, float leaf, float** out_dev, int64_t* n_out,
+                             lgs_voxelgrid_info* info);
 
 /* ------------------------------------------------------------------------------------------- */
 /* batched loop-closure verification: GBS:297-322 for a list of (scan, submap) pairs              */

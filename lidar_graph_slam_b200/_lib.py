@@ -84,6 +84,8 @@ SYMBOLS = {
     "lgs_ctx_launch_count": (_i64, [_vp]),
     "lgs_voxelgrid_filter": (_i32, [_vp, _vp, _i64, _i32, _vp, _i32, _f64, _vp, _vp, _vp, _vp, C.POINTER(VoxelGridInfo)]),
     "lgs_voxelgrid_filter_dev": (_i32, [_vp, _vp, _i64, _vp, _i32, _f64, _vp, _vp, _vp, _vp, C.POINTER(VoxelGridInfo)]),
+    "lgs_voxelgrid_filter_wide": (_i32, [_vp, _vp, _i64, _i32, _vp, _i32, _f64, _vp, _vp, _vp, _vp, C.POINTER(VoxelGridInfo)]),
+    "lgs_voxelgrid_filter_wide_dev": (_i32, [_vp, _vp, _i64, _vp, _i32, _f64, _vp, _vp, _vp, _vp, C.POINTER(VoxelGridInfo)]),
     "lgs_cloud_from_pointcloud2": (_i32, [_vp, _vp, C.POINTER(Pc2Layout), _vp, C.POINTER(_i64)]),
     "lgs_sor_create": (_i32, [_vp, C.POINTER(_vp)]),
     "lgs_sor_destroy": (None, [_vp]),
@@ -181,6 +183,7 @@ SYMBOLS = {
     "lgs_keyframes_set_pose": (_i32, [_vp, _i32, _vp]),
     "lgs_keyframes_size": (_i32, [_vp, C.POINTER(_i64), C.POINTER(_i64)]),
     "lgs_keyframes_assemble": (_i32, [_vp, _vp, _i32, _f32, C.POINTER(_vp), C.POINTER(_i64)]),
+    "lgs_keyframes_export_map": (_i32, [_vp, _vp, _i32, _f32, C.POINTER(_vp), C.POINTER(_i64), C.POINTER(VoxelGridInfo)]),
     "lgs_keyframes_set_accum_distance": (_i32, [_vp, _i32, _f64]),
     "lgs_keyframes_set_position": (_i32, [_vp, _i32, _vp]),
     "lgs_keyframes_detect_loop": (_i32, [_vp, _i32, _f64, _f64, _vp, _i32, C.POINTER(_i32), C.POINTER(_i32)]),

@@ -157,6 +157,7 @@ class VoxelGrid:
         self._min_pts = 0
         self._range_min = -1.0
         self._box = None
+        self._wide = False
         self._cloud = None
         self.info = None
         self.voxel_idx = None
@@ -181,6 +182,11 @@ class VoxelGrid:
     def setInputCloud(self, cloud):
         self._cloud = cloud
 
+    def setWideIndices(self, flag):
+        """The wide VoxelGrid (lgs_voxelgrid_filter_wide): a 64-bit voxel index, so grids beyond INT32_MAX cells are
+        filtered instead of refused; identical results wherever the 32-bit grid does not refuse.  voxel_idx is int64."""
+        self._wide = bool(flag)
+
     def filter(self, want_membership=True):
         """Returns the downsampled cloud (M, 4).  Per-point voxel_idx / member_rank land in attributes."""
         leaf_p = self._leaf.ctypes.data_as(C.c_void_p)
@@ -190,11 +196,13 @@ class VoxelGrid:
             import torch
             p, n = _dev_cloud(self._cloud, self.ctx)
             out = torch.empty((max(n, 1), 4), dtype=torch.float32, device=self._cloud.device)
-            vidx = torch.empty(max(n, 1), dtype=torch.int32, device=self._cloud.device) if want_membership else None
+            idx_t = torch.int64 if self._wide else torch.int32
+            vidx = torch.empty(max(n, 1), dtype=idx_t, device=self._cloud.device) if want_membership else None
             rank = torch.empty(max(n, 1), dtype=torch.int32, device=self._cloud.device) if want_membership else None
-            check(self._L.lgs_voxelgrid_filter_dev(self.ctx._h, p, n, leaf_p, self._min_pts, self._range_min, box_p, C.c_void_p(out.data_ptr()),
-                                                   C.c_void_p(vidx.data_ptr()) if want_membership else None,
-                                                   C.c_void_p(rank.data_ptr()) if want_membership else None, C.byref(info)))
+            fn = self._L.lgs_voxelgrid_filter_wide_dev if self._wide else self._L.lgs_voxelgrid_filter_dev
+            check(fn(self.ctx._h, p, n, leaf_p, self._min_pts, self._range_min, box_p, C.c_void_p(out.data_ptr()),
+                     C.c_void_p(vidx.data_ptr()) if want_membership else None,
+                     C.c_void_p(rank.data_ptr()) if want_membership else None, C.byref(info)))
             if not self.ctx.shares_torch_stream(self._cloud.device):
                 self.ctx.synchronize()  # outputs are written on the context's stream; torch reads them on its own
             self.info = info
@@ -203,11 +211,12 @@ class VoxelGrid:
             return out[: info.n_out]
         a, p, n, stride = _host_cloud(self._cloud)
         out = np.empty((max(n, 1), 4), np.float32)
-        vidx = np.empty(max(n, 1), np.int32) if want_membership else None
+        vidx = np.empty(max(n, 1), np.int64 if self._wide else np.int32) if want_membership else None
         rank = np.empty(max(n, 1), np.int32) if want_membership else None
-        check(self._L.lgs_voxelgrid_filter(self.ctx._h, p, n, stride, leaf_p, self._min_pts, self._range_min, box_p,
-                                           out.ctypes.data_as(C.c_void_p), vidx.ctypes.data_as(C.c_void_p) if want_membership else None,
-                                           rank.ctypes.data_as(C.c_void_p) if want_membership else None, C.byref(info)))
+        fn = self._L.lgs_voxelgrid_filter_wide if self._wide else self._L.lgs_voxelgrid_filter
+        check(fn(self.ctx._h, p, n, stride, leaf_p, self._min_pts, self._range_min, box_p,
+                 out.ctypes.data_as(C.c_void_p), vidx.ctypes.data_as(C.c_void_p) if want_membership else None,
+                 rank.ctypes.data_as(C.c_void_p) if want_membership else None, C.byref(info)))
         self.info = info
         self.voxel_idx = vidx[:n] if want_membership else None
         self.member_rank = rank[:n] if want_membership else None
@@ -547,6 +556,7 @@ class KeyFrameArray:
         h = C.c_void_p()
         check(self._L.lgs_keyframes_create(self.ctx._h, C.byref(h)))
         self._h = h
+        self.map_info = None
 
     def push(self, cloud, pose):
         _, pp = _mat_to_c(pose)
@@ -633,6 +643,30 @@ class KeyFrameArray:
             t.copy_(_device_view(out.value, n.value, self.ctx.device))
             torch.cuda.current_stream(t.device).synchronize()
         return t
+
+    def export_map(self, ids=None, leaf=0.0):
+        """The map of save_map (GBS:469-501, lgs_keyframes_export_map): every key frame (ids None) or the listed ones at
+        their current poses, concatenated, then the wide VoxelGrid with `leaf` (<= 0: none).  Returns a CUDA float32 tensor
+        (N, 4), a copy of the library's buffer; the grid's record lands in the attribute `map_info`."""
+        import torch
+        a = None if ids is None else np.ascontiguousarray(ids, dtype=np.int32)
+        out, n, info = C.c_void_p(), C.c_int64(), VoxelGridInfo()
+        check(self._L.lgs_keyframes_export_map(self._h, a.ctypes.data_as(C.c_void_p) if a is not None else None, 0 if a is None else int(a.size),
+                                               float(leaf), C.byref(out), C.byref(n), C.byref(info)))
+        self.ctx.synchronize()
+        self.map_info = info
+        t = torch.empty((n.value, 4), dtype=torch.float32, device="cuda:%d" % self.ctx.device)
+        if n.value:
+            t.copy_(_device_view(out.value, n.value, self.ctx.device))
+            torch.cuda.current_stream(t.device).synchronize()
+        return t
+
+    def save_map(self, path, resolution=0.0, ids=None):
+        """The save_map service (GBS:469-501): export_map(ids, resolution) written as a binary PCD.  Returns the point count."""
+        from . import pcd
+        m = self.export_map(ids, resolution).cpu().numpy()
+        pcd.write_pcd(path, m)
+        return int(m.shape[0])
 
     def __del__(self):
         try:

@@ -253,6 +253,47 @@ int lgs_keyframes_assemble(lgs_keyframes* kf, const int32_t* ids, int32_t n_ids,
   return LGS_OK;
 }
 
+// save_map (GBS:469-501): every key frame (ids == NULL) or the listed ones at their current poses, concatenated, then the
+// wide VoxelGrid, which keeps working where pcl::VoxelGrid refuses a whole map
+int lgs_keyframes_export_map(lgs_keyframes* kf, const int32_t* ids, int32_t n_ids, float leaf, float** out_dev, int64_t* n_out,
+                             lgs_voxelgrid_info* info) {
+  LGS_NVTX("lgs_keyframes_export_map");
+  LGS_REQUIRE(kf && out_dev && n_out, "null argument");
+  LGS_REQUIRE(ids ? n_ids >= 0 : n_ids == 0, "ids == NULL takes n_ids = 0");
+  const int32_t n_frames = static_cast<int32_t>(kf->frames.size());
+  std::vector<int32_t> all;
+  if (!ids) {
+    all.resize(static_cast<size_t>(n_frames));
+    for (int32_t i = 0; i < n_frames; i++) all[i] = i;
+    ids = all.data();
+    n_ids = n_frames;
+  }
+  int64_t total = 0;
+  for (int32_t i = 0; i < n_ids; i++) {
+    LGS_REQUIRE(ids[i] >= 0 && ids[i] < n_frames, "key frame id out of range");
+    total += kf->frames[ids[i]].n;
+  }
+  LGS_REQUIRE(total < (int64_t(1) << 31), "map larger than 2^31 points");
+  lgs_ctx* ctx = kf->ctx;
+  LGS_TRY(use_device(ctx));
+  LGS_TRY(keyframes_assemble_into(kf, ctx, ids, n_ids, &kf->poses_dev, &kf->assembled, &total));
+  lgs_voxelgrid_info vi;
+  memset(&vi, 0, sizeof(vi));
+  vi.n_kept = total;
+  vi.n_out = total;
+  *out_dev = kf->assembled.as<float>();
+  if (leaf > 0.0f && total > 0) {
+    LGS_TRY(kf->filtered.reserve(static_cast<size_t>(total) * 16));
+    const float leaf3[3] = {leaf, leaf, leaf};
+    LGS_TRY(voxelgrid_device(ctx, kf->assembled.as<float4>(), total, leaf3, 0, -1.0, nullptr, kf->filtered.as<float4>(), nullptr, nullptr, &vi, true,
+                             nullptr));
+    *out_dev = kf->filtered.as<float>();
+  }
+  *n_out = vi.n_out;
+  if (info) *info = vi;
+  return LGS_OK;
+}
+
 int lgs_keyframes_set_position(lgs_keyframes* kf, int32_t id, const double* xyz) {
   LGS_REQUIRE(kf && xyz, "null argument");
   LGS_REQUIRE(id >= 0 && id < static_cast<int32_t>(kf->frames.size()), "key frame id out of range");

@@ -180,6 +180,30 @@ int radix_sort_pairs(lgs_ctx* ctx, unsigned* keys, unsigned* vals, unsigned* key
   return LGS_OK;
 }
 
+// hi[j] = high word of the key of the index at position j (the second pass's keys)
+__global__ void __launch_bounds__(256) key_high_gather_kernel(const unsigned* __restrict__ perm, const u64_t* __restrict__ keys64, int64_t n,
+                                                             unsigned* __restrict__ hi) {
+  const int64_t j = blockIdx.x * static_cast<int64_t>(blockDim.x) + threadIdx.x;
+  if (j < n) hi[j] = static_cast<unsigned>(keys64[perm[j]] >> 32);
+}
+
+int radix_sort_indices64(lgs_ctx* ctx, const u64_t* keys64, unsigned* keys_lo, unsigned* vals, unsigned* keys_alt, unsigned* vals_alt, int64_t n,
+                         int bits, unsigned** vals_out) {
+  LGS_REQUIRE(bits >= 0 && bits <= 64, "key bits out of range");
+  unsigned *k1, *v1;
+  LGS_TRY(radix_sort_pairs(ctx, keys_lo, vals, keys_alt, vals_alt, n, std::min(bits, 32), &k1, &v1));
+  *vals_out = v1;
+  if (bits <= 32 || n <= 1) return LGS_OK;
+  // the low words are no longer needed: their buffer takes the gathered high words, the other pair is the alt side
+  unsigned* k_other = k1 == keys_lo ? keys_alt : keys_lo;
+  unsigned* v_other = v1 == vals ? vals_alt : vals;
+  key_high_gather_kernel<<<grid_for(n, 256), 256, 0, ctx->stream>>>(v1, keys64, n, k1);
+  ctx->launches++;
+  LGS_CUDA(cudaGetLastError());
+  unsigned* k2;
+  return radix_sort_pairs(ctx, k1, v1, k_other, v_other, n, bits - 32, &k2, vals_out);
+}
+
 int scan_select_prepare(lgs_ctx* ctx, int64_t n, u64_t** status, unsigned** ticket) {
   u64_t* ghist;
   return reserve_sort_tmp(ctx, static_cast<size_t>((n + kScanTile - 1) / kScanTile), ticket, &ghist, status);

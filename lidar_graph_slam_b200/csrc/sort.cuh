@@ -135,6 +135,14 @@ __global__ void __launch_bounds__(kSortThreads) scan_select_kernel(F f, int64_t 
 int radix_sort_pairs(lgs_ctx* ctx, unsigned* keys, unsigned* vals, unsigned* keys_alt, unsigned* vals_alt, int64_t n, int bits,
                      unsigned** keys_out, unsigned** vals_out);
 
+// Stable sort of n indices by a 64-bit key, over the low `bits` (<= 64) key bits: vals holds indices into keys64 and
+// keys_lo[i] the low word of keys64[vals[i]].  Two radix_sort_pairs composed least-significant word first: (low word,
+// index) over min(bits, 32) bits, then the high words gathered through that permutation and (high word, permutation)
+// sorted over bits - 32 bits.  Stability of both keeps equal keys in their input order.  The sorted indices end up in
+// *vals_out (vals or vals_alt); keys_lo and keys_alt are overwritten.
+int radix_sort_indices64(lgs_ctx* ctx, const u64_t* keys64, unsigned* keys_lo, unsigned* vals, unsigned* keys_alt, unsigned* vals_alt, int64_t n,
+                         int bits, unsigned** vals_out);
+
 // reserves and zeroes the look-back scratch for one scan_select launch over n elements
 int scan_select_prepare(lgs_ctx* ctx, int64_t n, u64_t** status, unsigned** ticket);
 
