@@ -227,8 +227,8 @@ class NormalDistributionsTransform : public Registration {
     return s;
   }
   lgs_ndt* handle() const { return h_; }
-  // No counterpart in the reference: align this source from every guess in one resident launch per wave
-  // (lgs_ndt_align_many).  Record k is bit-identical to align(output, guesses[k]); afterwards result() is the last guess's.
+  // No counterpart in the reference: align this source from every guess in turn (lgs_ndt_align_many).  Record k is
+  // bit-identical to align(output, guesses[k]); afterwards result() is the last guess's.
   // fitness_max_range < 0: no fitness, else records[k].fitness = getFitnessScore(fitness_max_range) at record k's transform.
   std::vector<lgs_align_result> alignGuesses(const std::vector<Matrix4f>& guesses, double fitness_max_range = -1.0) {
     ok_ = true;
@@ -251,7 +251,7 @@ class NormalDistributionsTransform : public Registration {
   double step_ = 0.1, outlier_ = 0.55;
 };
 
-// No counterpart in the reference: ndts[i]->align(guesses[i]) for every i in one resident launch per wave (lgs_ndt_align_many);
+// No counterpart in the reference: ndts[i]->align(guesses[i]) for every i in turn, in one call (lgs_ndt_align_many);
 // the objects may repeat and must share one Context.  guesses: empty (identity) or one per object.  Each object's result()
 // becomes that of its last occurrence.  On failure every object records the error (hasConverged() false, lastError()).
 inline std::vector<lgs_align_result> alignMany(const std::vector<NormalDistributionsTransform*>& ndts, const std::vector<Matrix4f>& guesses = {},

@@ -412,7 +412,7 @@ class NormalDistributionsTransform(_Registration):
         return nv.value
 
     def align_guesses(self, guesses, fitness_max_range=None):
-        """One map, many seeds: align this source from every 4x4 guess in one resident launch per wave (ndt_align_many).
+        """One map, many seeds: align this source from every 4x4 guess in turn, in one call (ndt_align_many).
         Record k is bit-identical to align(guesses[k]); afterwards the object holds the last guess's result."""
         return ndt_align_many([self] * len(guesses), guesses, fitness_max_range)
 
@@ -698,7 +698,7 @@ class IterativeClosestPoint(_Registration):
 
 
 def ndt_align_many(ndts, guesses=None, fitness_max_range=None, want_output=False):
-    """Aligns N NDT problems in one resident launch per wave (lgs_ndt_align_many): ndts[i] from guesses[i] (4x4, or identity
+    """Aligns N NDT problems in turn, in one call (lgs_ndt_align_many): ndts[i] from guesses[i] (4x4, or identity
     when guesses is None).  Handles may repeat and must share one Context.  Each record is bit-identical to ndts[i].align(
     guesses[i]) run alone, and every object ends with the result and final transformation of its last occurrence, as after
     those calls in order.  fitness_max_range: records[i].fitness = getFitnessScore(fitness_max_range) at record i's

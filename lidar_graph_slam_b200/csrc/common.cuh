@@ -142,7 +142,6 @@ struct lgs_ctx {
   lgs::PinnedBuf pin;    // small D2H results
   lgs::PinnedBuf pin_up; // small H2D parameter blocks
   lgs::DevBuf vg_in, vg_out, vg_vidx, vg_rank;  // host-facing voxel-grid call: staged cloud + device-side outputs
-  lgs::DevBuf ndt_many;  // lgs_ndt_align_many: group descriptors, hand-over blocks, result records and rows of one launch
   lgs::MailboxHost* mbox = nullptr;             // result mailbox (mapped pinned host memory)
   unsigned long long mbox_token = 0;
   bool polite_wait = false;  // batch workers: yield the core while waiting for a mailbox (several workers may share one)

@@ -1,6 +1,5 @@
-"""lgs_ndt_align_many (-m gpu): N NDT aligns in one resident launch per wave.  Every record must be bit for bit what
-lgs_ndt_align returns for that problem alone, whatever the grouping, and every handle must end in the state the same
-sequence of single aligns leaves."""
+"""lgs_ndt_align_many (-m gpu): N NDT aligns in one call.  Every record must be bit for bit what lgs_ndt_align returns for
+that problem alone, and every handle must end in the state the same sequence of single aligns leaves."""
 import ctypes as C
 
 import numpy as np
@@ -46,23 +45,6 @@ def _key(r):
             r.hessian_recomputes)
 
 
-@pytest.fixture(params=[None, "16", "3"], ids=["default", "groups16", "groups3"])
-def groups(request, monkeypatch):
-    """LGS_NDT_MANY_MAX_GROUPS: the default, every problem of a call in one ndt_align_group_kernel launch, and waves of three
-    (the last wave of a call may hold one problem, which takes the single-align launch)."""
-    if request.param is None:
-        monkeypatch.delenv("LGS_NDT_MANY_MAX_GROUPS", raising=False)
-    else:
-        monkeypatch.setenv("LGS_NDT_MANY_MAX_GROUPS", request.param)
-    return request.param
-
-
-def _launches(groups, k):
-    """ndt_align_* launches of k device-eligible problems of one class."""
-    m = 1 if groups is None else int(groups)
-    return -(-k // m)
-
-
 @pytest.fixture(scope="module")
 def pair(oracle, velodyne_pair):
     return dict(target=oracle.voxel_grid(velodyne_pair["target"], 0.2)["points"], source=oracle.voxel_grid(velodyne_pair["source"], 0.2)["points"],
@@ -71,14 +53,14 @@ def pair(oracle, velodyne_pair):
 
 @pytest.mark.parametrize("exact", [False, True])
 @pytest.mark.parametrize("method", [2, 3, 1])  # DIRECT7, DIRECT1, DIRECT26
-def test_align_guesses_is_bitwise_the_single_aligns(api, pair, method, exact, groups):
+def test_align_guesses_is_bitwise_the_single_aligns(api, pair, method, exact):
     guesses = _guesses(pair["relative"], 1000 + 10 * method + exact, 16)
     many = _ndt(api, pair["target"], pair["source"], method=method, exact=exact)
     one = _ndt(api, pair["target"], pair["source"], method=method, exact=exact)
     ctx = api.default_context()
     before = ctx.launch_count
     recs = many.align_guesses(guesses)
-    assert ctx.launch_count - before == _launches(groups, 16)  # the grouped kernel did run when groups is set
+    assert ctx.launch_count - before == 16  # one ndt_align_kernel launch per align
     assert len(recs) == 16
     for k, (r, guess) in enumerate(zip(recs, guesses)):
         one.align(guess)
@@ -91,7 +73,7 @@ def test_align_guesses_is_bitwise_the_single_aligns(api, pair, method, exact, gr
     assert len({r.iterations for r in recs}) > 3  # the seeds take different paths
 
 
-def test_align_guesses_cfg0_multi_tile(api, groups):
+def test_align_guesses_cfg0_multi_tile(api):
     """BASELINE configs[0]: 120 000 source points (several tiles per CTA) against a 1 000 000-point map."""
     from lidar_graph_slam_b200 import synth
     d = synth.ndt_scan_to_map()
@@ -101,7 +83,7 @@ def test_align_guesses_cfg0_multi_tile(api, groups):
     ctx = api.default_context()
     before = ctx.launch_count
     recs = many.align_guesses(guesses)
-    assert ctx.launch_count - before == _launches(groups, 8)
+    assert ctx.launch_count - before == 8
     for k, (r, guess) in enumerate(zip(recs, guesses)):
         one.align(guess)
         assert _key(r) == _key(one.result), k
@@ -124,7 +106,7 @@ def _mixed_problems(api, pair, velodyne_pair, ctx=None):
     return mk
 
 
-def test_mixed_handles_equal_the_sequential_calls(api, pair, velodyne_pair, groups):
+def test_mixed_handles_equal_the_sequential_calls(api, pair, velodyne_pair):
     mk = _mixed_problems(api, pair, velodyne_pair)
     many = [f() for f in mk]
     seq = [f() for f in mk]
@@ -142,32 +124,6 @@ def test_mixed_handles_equal_the_sequential_calls(api, pair, velodyne_pair, grou
     for h in range(len(mk)):  # post-call state: the last occurrence's
         assert _key(many[h].result) == _key(seq[h].result), h
         assert many[h].getFitnessScore(2.0) == seq[h].getFitnessScore(2.0), h
-
-
-def test_grouping_does_not_change_any_record(api, pair, velodyne_pair, monkeypatch):
-    td, sd = pair["target"], pair["source"]
-    hs = [_ndt(api, td, sd, res=r, method=m) for r, m in ((1.0, 2), (2.0, 2), (1.0, 3), (1.5, 1))]
-    problems = [hs[k % 4] for k in range(8)]
-    g = _guesses(pair["relative"], 5, 8)
-    runs = {}
-    for groups in ("1", "3", None):
-        if groups is None:
-            monkeypatch.delenv("LGS_NDT_MANY_MAX_GROUPS", raising=False)
-        else:
-            monkeypatch.setenv("LGS_NDT_MANY_MAX_GROUPS", groups)
-        runs[groups] = [_key(r) for r in api.ndt_align_many(problems, g)]
-    assert runs["1"] == runs["3"] == runs[None]
-    # 8 device-eligible problems in two classes of 4 (DIRECT7 and DIRECT1/26): one launch per class at 4 groups per wave
-    monkeypatch.setenv("LGS_NDT_MANY_MAX_GROUPS", "4")
-    ctx = api.default_context()
-    before = ctx.launch_count
-    again = [_key(r) for r in api.ndt_align_many(problems, g)]
-    assert ctx.launch_count - before == 2
-    assert again == runs[None]
-    monkeypatch.setenv("LGS_NDT_MANY_MAX_GROUPS", "2")
-    before = ctx.launch_count
-    api.ndt_align_many(problems, g)
-    assert ctx.launch_count - before == 4
 
 
 def test_errors_leave_everything_untouched(api, pair):
@@ -202,7 +158,7 @@ def test_errors_leave_everything_untouched(api, pair):
     assert a.getFitnessScore() == fit_a and b.getFitnessScore() == fit_b
 
 
-def test_align_many_against_the_oracle(api, oracle, pair, groups):
+def test_align_many_against_the_oracle(api, oracle, pair):
     """Four seeds on the bundled Velodyne pair against oracle.NDT at the parity suite's tolerances."""
     g = _ndt(api, pair["target"], pair["source"])
     guesses = _guesses(pair["relative"], 4242, 4)
@@ -224,12 +180,11 @@ def test_align_many_against_the_oracle(api, oracle, pair, groups):
         assert r.trans_probability == pytest.approx(o.trans_probability, rel=1e-5)
 
 
-def test_cpp_shim_align_guesses_and_align_many(api, tmp_path, monkeypatch):
-    """The C++ entry points (NormalDistributionsTransform::alignGuesses, lgs::alignMany) on the GPU, grouped: their records equal
-    the single aligns bitwise."""
+def test_cpp_shim_align_guesses_and_align_many(api, tmp_path):
+    """The C++ entry points (NormalDistributionsTransform::alignGuesses, lgs::alignMany) on the GPU: their records equal the
+    single aligns bitwise."""
     import subprocess
     from test_shim_align_many import build_shim_align_many
     exe = build_shim_align_many(tmp_path)
-    monkeypatch.setenv("LGS_NDT_MANY_MAX_GROUPS", "4")
     out = subprocess.check_output([exe, "--run"]).decode()
     assert "align_many ok" in out, out

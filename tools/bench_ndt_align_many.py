@@ -1,11 +1,11 @@
 """Sequential NDT aligns against lgs_ndt_align_many on one GPU; prints one JSON line.
 
-    python tools/bench_ndt_align_many.py [--reps 5] [--groups 2,4,8,16]
+    python tools/bench_ndt_align_many.py [--reps 5] [--ks 1,2,4,8,16]
 
 For K seeds (random guesses around the true pose) on one map it times K calls of align() and one align_guesses() call of the
 same K guesses, alternately, `reps` times each, and reports aligns/s of both, launches per call and the spread (min / max) over
 the repetitions.  Two workloads: BASELINE configs[0] (120 000-point sweep, 1 000 000-point map) and a loop-closure-sized
-source (every fifth point of it, ~24 000 points).  --groups also times K = 16 under each LGS_NDT_MANY_MAX_GROUPS value.
+source (every fifth point of it, ~24 000 points).
 Every align_guesses record is checked bitwise against its single align.  Needs a CUDA device.
 """
 import argparse
@@ -41,7 +41,6 @@ def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--reps", type=int, default=5)
     ap.add_argument("--ks", default="1,2,4,8,16")
-    ap.add_argument("--groups", default="2,4,8,16")
     args = ap.parse_args()
     from lidar_graph_slam_b200 import api, synth
 
@@ -68,11 +67,7 @@ def main():
             r = fn()
             return time.perf_counter() - t0, ctx.launch_count - l0, r
 
-        def measure(K, label, groups=None):
-            if groups is not None:
-                os.environ["LGS_NDT_MANY_MAX_GROUPS"] = str(groups)
-            else:
-                os.environ.pop("LGS_NDT_MANY_MAX_GROUPS", None)
+        def measure(K):
             gs = seeds[:K]
             seq_t, many_t = [], []
             identical = True
@@ -82,17 +77,14 @@ def main():
                 t, lm, rm = timed(lambda: g.align_guesses(gs))
                 many_t.append(t)
                 identical &= [_key(a) for a in rs] == [_key(b) for b in rm]
-            out["rows"].append(dict(workload=name, n_source=int(len(src)), K=K, max_groups=groups if groups is not None else "default",
+            out["rows"].append(dict(workload=name, n_source=int(len(src)), K=K,
                                     seq_aligns_per_s=K / float(np.median(seq_t)), many_aligns_per_s=K / float(np.median(many_t)),
                                     speedup=float(np.median(seq_t) / np.median(many_t)),
                                     seq_spread_ms=[1e3 * min(seq_t), 1e3 * max(seq_t)], many_spread_ms=[1e3 * min(many_t), 1e3 * max(many_t)],
-                                    seq_launches=ls, many_launches=lm, bit_identical=bool(identical), label=label))
+                                    seq_launches=ls, many_launches=lm, bit_identical=bool(identical)))
 
         for K in [int(k) for k in args.ks.split(",") if k]:
-            measure(K, "ks")
-        for M in [int(m) for m in args.groups.split(",") if m]:
-            measure(16, "groups", M)
-    os.environ.pop("LGS_NDT_MANY_MAX_GROUPS", None)
+            measure(K)
     print(json.dumps(out), flush=True)
 
 
