@@ -409,6 +409,13 @@ int lgs_sort_pairs(lgs_ctx* ctx, uint32_t* keys, uint32_t* vals, int64_t n, int3
 #define LGS_LINALG_OUT(op) ((op) == LGS_LINALG_SVD3 ? 21 : (op) == LGS_LINALG_EIG3 ? 13 : (op) == LGS_LINALG_INV3 ? 9 : (op) == LGS_LINALG_SVD_SOLVE6 ? 6 : (op) == LGS_LINALG_SCHUR6 ? 7 : 12)
 int lgs_linalg_batch(lgs_ctx* ctx, int32_t op, int64_t n, const double* in, double* out);
 
+/* parity hook for the last-CTA reduction behind every sum an evaluation returns (csrc/reduce.cuh): G CTAs take the rows
+ * of rows (G x K, row-major) as their sums and run the grid finish; out receives the K sums it publishes.  Group g of NG
+ * adds rows g, g + NG, g + 2 NG, ... in turn from 0.0, then the NG group sums are added in group order from 0.0.  (K, NG)
+ * is one the kernels use: (1, 1) NDT calculateScore, (1, 2) and (43, 2) FastGICP, (17, 8) ICP, (44, 12), (8, 12) and
+ * (22, 12) the NDT derivatives.  Any other (K, NG), G < 1 or a null pointer is LGS_ERR_INVALID and launches nothing. */
+int lgs_grid_fold_check(lgs_ctx* ctx, const double* rows, int32_t G, int32_t K, int32_t NG, double* out);
+
 /* ------------------------------------------------------------------------------------------- */
 /* key-frame array + sub-map assembly, device resident                                            */
 /*   replaces the per-key-frame fromROSMsg + transform_point_cloud + `*cloud += ...` loops and the */

@@ -176,6 +176,7 @@ SYMBOLS = {
     "lgs_nn_search1": (_i32, [_vp, _vp, _i64, _i32, _vp, _i64, _i32, _vp, _vp, _vp]),
     "lgs_sort_pairs": (_i32, [_vp, _vp, _vp, _i64, _i32]),
     "lgs_linalg_batch": (_i32, [_vp, _i32, _i64, _vp, _vp]),
+    "lgs_grid_fold_check": (_i32, [_vp, _vp, _i32, _i32, _i32, _vp]),
     "lgs_keyframes_create": (_i32, [_vp, C.POINTER(_vp)]),
     "lgs_keyframes_destroy": (None, [_vp]),
     "lgs_keyframes_push": (_i32, [_vp, _vp, _i64, _i32, _vp, C.POINTER(_i32)]),

@@ -783,6 +783,18 @@ def linalg_batch(op, inputs, ctx=None):
     return out
 
 
+def grid_fold_check(rows, groups, ctx=None):
+    """The last-CTA reduction of the kernels (parity hook lgs_grid_fold_check): CTA b of G takes row b of rows (G, K) as
+    its sums; returns the K sums the grid finish publishes when it folds the rows in `groups` groups."""
+    ctx = ctx or default_context()
+    a = np.ascontiguousarray(rows, dtype=np.float64)
+    if a.ndim != 2:
+        raise ValueError("rows must be (G, K)")
+    out = np.empty(a.shape[1])
+    check(ctx._L.lgs_grid_fold_check(ctx._h, a.ctypes.data_as(C.c_void_p), a.shape[0], a.shape[1], int(groups), out.ctypes.data_as(C.c_void_p)))
+    return out
+
+
 def batch_align(scans, submaps, method=METHOD_GICP, guesses=None, device=0, stream=None, pair_id0=0, records_dev=None, max_iterations=100,
                 transformation_epsilon=0.01, max_correspondence_distance=2.0, k_correspondences=20, ndt_resolution=1.0, ndt_step_size=0.1,
                 submap_leaf=0.5, fitness_max_range=-1.0, n_workers=0, max_optimizer_iterations=0, euclidean_fitness_epsilon=0.0):

@@ -14,6 +14,7 @@
 #include <memory>
 
 #include "gicp.cuh"
+#include "reduce.cuh"
 
 namespace lgs {
 
@@ -171,57 +172,8 @@ struct LinParams {
 
 constexpr int kLinBlock = 128;
 
-template <int K>
-__device__ __forceinline__ void lin_block_reduce_and_finish(double (&acc)[K], double* __restrict__ partials, double* __restrict__ result,
-                                                           unsigned* __restrict__ counter, const Mailbox& mb) {
-  __shared__ double sm[kLinBlock / 32][K];
-  __shared__ bool is_last;
-  const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
-#pragma unroll
-  for (int k = 0; k < K; k++) {
-    double v = acc[k];
-#pragma unroll
-    for (int off = 16; off > 0; off >>= 1) v += __shfl_xor_sync(0xffffffffu, v, off);
-    if (lane == 0) sm[warp][k] = v;
-  }
-  __syncthreads();
-  if (threadIdx.x < K) {
-    double v = 0;
-#pragma unroll
-    for (int w = 0; w < kLinBlock / 32; w++) v += sm[w][threadIdx.x];
-    partials[static_cast<size_t>(blockIdx.x) * K + threadIdx.x] = v;
-  }
-  __threadfence();
-  __syncthreads();
-  if (threadIdx.x == 0) is_last = atomicAdd(counter, 1u) == gridDim.x - 1;
-  __syncthreads();
-  if (is_last) {
-    // two groups of 64 threads add the even / odd per-block rows in block order (sixteen loads in flight each), then the
-    // two halves are added: a fixed function of the grid size, so the sums are reproducible run to run
-    __threadfence();
-    static_assert(K <= 64 && kLinBlock == 128, "two groups of 64 threads");
-    __shared__ double half[64];
-    const int kk = threadIdx.x & 63, grp = threadIdx.x >> 6;
-    double v = 0;
-    if (kk < K) {
-      for (unsigned b0 = grp; b0 < gridDim.x; b0 += 32) {  // sixteen loads in flight per round: the pass is L2-latency bound
-        double t[16];
-#pragma unroll
-        for (int u = 0; u < 16; u++) t[u] = b0 + 2 * u < gridDim.x ? __ldcg(partials + static_cast<size_t>(b0 + 2 * u) * K + kk) : 0.0;
-#pragma unroll
-        for (int u = 0; u < 16; u++) v += t[u];
-      }
-    }
-    if (grp == 1 && kk < K) half[kk] = v;
-    __syncthreads();
-    if (grp == 0 && kk < K) {
-      v += half[kk];
-      result[kk] = v;
-    }
-    if (threadIdx.x == 0) *counter = 0;
-    mailbox_publish<K>(mb, v);  // the host reads the sums from mapped pinned memory: no D2H copy, no stream synchronisation
-  }
-}
+// the per-CTA rows are folded in two groups, even rows and odd rows, each with sixteen loads in flight (reduce.cuh)
+constexpr int kLinGroups = 2, kLinLoads = 16;
 
 // error term of one correspondence: e = mean_B - T mean_A ; returns e^T M e and (optionally) accumulates H, b
 template <bool WANT_HB>
@@ -286,7 +238,7 @@ __global__ void __launch_bounds__(kLinBlock) gicp_linearize_kernel(const float4*
                                                                   LinParams P, const double* __restrict__ cov_src,
                                                                   const double* __restrict__ cov_tgt, const int* __restrict__ corr,
                                                                   double* __restrict__ mahal, int want_hb, double* __restrict__ partials,
-                                                                  double* __restrict__ result, unsigned* __restrict__ counter, const Mailbox mb) {
+                                                                  unsigned* __restrict__ counter, const Mailbox mb) {
   double acc[43];
 #pragma unroll
   for (int k = 0; k < 43; k++) acc[k] = 0.0;
@@ -317,13 +269,12 @@ __global__ void __launch_bounds__(kLinBlock) gicp_linearize_kernel(const float4*
     else
       gicp_point_terms<false>(P, a, b, M, acc);
   }
-  lin_block_reduce_and_finish<43>(acc, partials, result, counter, mb);
+  grid_finish<43, kLinBlock, kLinGroups, kLinLoads>(cta_row<kLinBlock>(acc), partials, counter, mb);
 }
 
 __global__ void __launch_bounds__(kLinBlock) gicp_error_kernel(const float4* __restrict__ src, const float4* __restrict__ tgt, int n, LinParams P,
                                                               const int* __restrict__ corr, const double* __restrict__ mahal,
-                                                              double* __restrict__ partials, double* __restrict__ result,
-                                                              unsigned* __restrict__ counter, const Mailbox mb) {
+                                                              double* __restrict__ partials, unsigned* __restrict__ counter, const Mailbox mb) {
   double acc[1] = {0.0};
   for (int i = blockIdx.x * blockDim.x + threadIdx.x; i < n; i += gridDim.x * blockDim.x) {
     const int c = corr[i];
@@ -335,7 +286,7 @@ __global__ void __launch_bounds__(kLinBlock) gicp_error_kernel(const float4* __r
     for (int t = 0; t < 9; t++) M[t] = mahal[static_cast<size_t>(i) * 9 + t];
     gicp_point_terms<false>(P, a, b, M, acc);
   }
-  lin_block_reduce_and_finish<1>(acc, partials, result, counter, mb);
+  grid_finish<1, kLinBlock, kLinGroups, kLinLoads>(cta_row<kLinBlock>(acc), partials, counter, mb);
 }
 
 }  // namespace lgs
@@ -411,9 +362,9 @@ int ensure_ready(lgs_gicp* g) {
   LGS_TRY(g->mahal.reserve(n * 72));
   const int grid = lin_grid(g->source->n);
   LGS_TRY(g->partials.reserve(static_cast<size_t>(grid) * 44 * 8));
-  if (!g->result.p) {
-    LGS_TRY(g->result.reserve(44 * 8 + 64));
-    LGS_CUDA(cudaMemsetAsync(g->result.p, 0, 44 * 8 + 64, g->ctx->stream));
+  if (!g->counter.p) {
+    LGS_TRY(g->counter.reserve(sizeof(unsigned)));
+    LGS_CUDA(cudaMemsetAsync(g->counter.p, 0, sizeof(unsigned), g->ctx->stream));
   }
   return LGS_OK;
 }
@@ -438,8 +389,7 @@ int linearize(lgs_gicp* g, const double* T, double* cost, double* H, double* b) 
   if (n == 0) return LGS_OK;
   LinParams P;
   fill_lin_params(g, T, &P);
-  double* result = g->result.as<double>();
-  unsigned* counter = reinterpret_cast<unsigned*>(result + 44);
+  unsigned* counter = g->counter.as<unsigned>();
   const int cgrid = std::max(1, std::min(grid_for(n, kCorrBlock / 32), kNumSMs * 8));
   Mailbox mb;
   LGS_TRY(mailbox_next(ctx, &mb));
@@ -450,7 +400,7 @@ int linearize(lgs_gicp* g, const double* T, double* cost, double* H, double* b) 
   LGS_TRY(g->target->cover_correspondences(ctx, g->corr.as<int>(), n));
   gicp_linearize_kernel<<<lin_grid(n), kLinBlock, 0, st>>>(g->source->pts.as<float4>(), g->target->pts.as<float4>(), n, P,
                                                           g->source->covs.as<double>(), g->target->covs.as<double>(), g->corr.as<int>(),
-                                                          g->mahal.as<double>(), (H && b) ? 1 : 0, g->partials.as<double>(), result, counter, mb);
+                                                          g->mahal.as<double>(), (H && b) ? 1 : 0, g->partials.as<double>(), counter, mb);
   ctx->launches++;
   LGS_CUDA(cudaGetLastError());
   double h[kMailboxRecords];
@@ -473,12 +423,11 @@ int compute_error(lgs_gicp* g, const double* T, double* cost) {
   if (n == 0) return LGS_OK;
   LinParams P;
   fill_lin_params(g, T, &P);
-  double* result = g->result.as<double>();
-  unsigned* counter = reinterpret_cast<unsigned*>(result + 44);
+  unsigned* counter = g->counter.as<unsigned>();
   Mailbox mb;
   LGS_TRY(mailbox_next(ctx, &mb));
   gicp_error_kernel<<<lin_grid(n), kLinBlock, 0, st>>>(g->source->pts.as<float4>(), g->target->pts.as<float4>(), n, P, g->corr.as<int>(),
-                                                      g->mahal.as<double>(), g->partials.as<double>(), result, counter, mb);
+                                                      g->mahal.as<double>(), g->partials.as<double>(), counter, mb);
   ctx->launches++;
   LGS_CUDA(cudaGetLastError());
   LGS_TRY(mailbox_wait(ctx, mb, 1, cost));
@@ -620,7 +569,7 @@ void lgs_gicp_destroy(lgs_gicp* g) {
   cudaStreamSynchronize(g->ctx->stream);
   g->source.reset();
   g->target.reset();
-  for (DevBuf* b : {&g->corr, &g->nn_prev, &g->mahal, &g->partials, &g->result, &g->out_cloud}) b->release();
+  for (DevBuf* b : {&g->corr, &g->nn_prev, &g->mahal, &g->partials, &g->counter, &g->out_cloud}) b->release();
   delete g;
 }
 

@@ -52,7 +52,7 @@ struct lgs_gicp {
   int lm_max_iterations = 10;
   double lm_init_lambda_factor = 1e-9, lm_lambda = -1.0;
   std::shared_ptr<lgs::GicpCloud> source, target;
-  lgs::DevBuf corr, mahal, partials, result, out_cloud;
+  lgs::DevBuf corr, mahal, partials, counter, out_cloud;  // partials, counter: the last-CTA reduction (reduce.cuh)
   lgs::DevBuf nn_prev;     // nearest target point of every source point at the previous linearisation (search seed)
   bool have_seed = false;  // nn_prev is valid for the current source / target pair
   double final_hessian[36] = {1, 0, 0, 0, 0, 0, 0, 1, 0, 0, 0, 0, 0, 0, 1, 0, 0, 0, 0, 0, 0, 1, 0, 0, 0, 0, 0, 0, 1, 0, 0, 0, 0, 0, 0, 1};

@@ -24,6 +24,7 @@
 #include "fixsum.cuh"
 #include "gicp.cuh"
 #include "persist.cuh"
+#include "reduce.cuh"
 
 namespace lgs {
 
@@ -98,65 +99,9 @@ __global__ void __launch_bounds__(kPCorrBlock) pgicp_correspondence_kernel(NNVie
   }
 }
 
-// Reduction of K per-thread exact sums (fixsum.cuh): warp shuffles, CTA, per-CTA partials, last CTA adds them and
-// publishes the K doubles.  Integer addition: the result does not depend on the order of any of these steps.
-template <int K>
-__device__ __forceinline__ void fun_reduce_and_publish(Fix128 (&acc)[K], Fix128* __restrict__ partials, unsigned* __restrict__ counter,
-                                                      const Mailbox& mb) {
-  __shared__ Fix128 sm[kFunBlock / 32][K];
-  __shared__ bool is_last;
-  const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
-#pragma unroll
-  for (int k = 0; k < K; k++) {
-    Fix128 v = acc[k];
-#pragma unroll
-    for (int off = 16; off > 0; off >>= 1) {
-      Fix128 o;
-      o.lo = __shfl_xor_sync(0xffffffffu, v.lo, off);
-      o.hi = __shfl_xor_sync(0xffffffffu, v.hi, off);
-      fix_add(v, o);
-    }
-    if (lane == 0) sm[warp][k] = v;
-  }
-  __syncthreads();
-  if (threadIdx.x < K) {
-    Fix128 v = sm[0][threadIdx.x];
-#pragma unroll
-    for (int w = 1; w < kFunBlock / 32; w++) fix_add(v, sm[w][threadIdx.x]);
-    partials[static_cast<size_t>(blockIdx.x) * K + threadIdx.x] = v;
-  }
-  __threadfence();
-  __syncthreads();
-  if (threadIdx.x == 0) is_last = atomicAdd(counter, 1u) == gridDim.x - 1;
-  __syncthreads();
-  if (is_last) {
-    // integer sums: any order gives the same bits, so the per-CTA rows are added by eight groups of threads in parallel
-    __threadfence();
-    __shared__ Fix128 fin[kFunBlock / 16][16];
-    static_assert(K <= 16, "one 16-thread group per slice of the rows");
-    const int kk = threadIdx.x & 15, part = threadIdx.x >> 4;
-    Fix128 v = fix_zero();
-    if (kk < K) {
-#pragma unroll 4
-      for (unsigned b = part; b < gridDim.x; b += kFunBlock / 16) {
-        const ulonglong2 t = __ldcg(reinterpret_cast<const ulonglong2*>(partials + static_cast<size_t>(b) * K + kk));
-        Fix128 u;
-        u.lo = t.x;
-        u.hi = static_cast<long long>(t.y);
-        fix_add(v, u);
-      }
-    }
-    fin[part][kk] = v;
-    __syncthreads();
-    v = fix_zero();
-    if (threadIdx.x < K) {
-#pragma unroll
-      for (int p = 0; p < kFunBlock / 16; p++) fix_add(v, fin[p][threadIdx.x]);
-    }
-    if (threadIdx.x == 0) *counter = 0;
-    mailbox_publish<K>(mb, fix_value(v));
-  }
-}
+// The functor sums are reduced through reduce.cuh in integer arithmetic, so no step's order changes the result; the per-CTA
+// rows are folded by eight groups of 16 threads
+constexpr int kFunGroups = 8, kFunLoads = 4;
 
 // M_i = (R C1 R^T + C2)^-1, cast to f32 (GO:439-452); publishes the number of correspondences
 __global__ void __launch_bounds__(kFunBlock) pgicp_mahalanobis_kernel(int n, PgicpParams P, const double* __restrict__ cov_src,
@@ -186,7 +131,7 @@ __global__ void __launch_bounds__(kFunBlock) pgicp_mahalanobis_kernel(int n, Pgi
     for (int t = 0; t < 9; t++) mahal[static_cast<size_t>(i) * 9 + t] = static_cast<float>(inv[t]);
     fix_add(acc[0], 1.0);
   }
-  fun_reduce_and_publish<1>(acc, partials, counter, mb);
+  grid_finish<1, kFunBlock, kFunGroups, kFunLoads>(cta_row<kFunBlock>(acc), partials, counter, mb);
 }
 
 // MODE 0: operator() (f32 arithmetic, GO:245-275)   sums: f
@@ -236,7 +181,7 @@ __device__ __forceinline__ void pgicp_functor_body(const float4* __restrict__ ou
         for (int cc = 0; cc < 3; cc++) fix_add(acc[o + 3 + r * 3 + cc], __dmul_rn(ps[r], temp[cc]));
     }
   }
-  fun_reduce_and_publish<K>(acc, partials, counter, mb);
+  grid_finish<K, kFunBlock, kFunGroups, kFunLoads>(cta_row<kFunBlock>(acc), partials, counter, mb);
 }
 
 template <int MODE>

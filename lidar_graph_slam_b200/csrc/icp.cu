@@ -19,6 +19,7 @@
 #include "math.cuh"
 #include "nn.cuh"
 #include "persist.cuh"
+#include "reduce.cuh"
 
 namespace lgs {
 
@@ -35,7 +36,6 @@ struct IcpParams {
 __device__ __forceinline__ void icp_step_body(const NNView& tv, const float4* __restrict__ tgt, float4* __restrict__ cloud, int* __restrict__ nn_prev, int n,
                                               const IcpParams& P, double* __restrict__ partials, unsigned* __restrict__ counter, const Mailbox& mb) {
   __shared__ double sm[kIcpBlock / 32][kIcpSums];
-  __shared__ bool is_last;
   const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
   double acc = 0.0;  // lane k < 17 owns sum k of this warp
   for (int i = blockIdx.x * (kIcpBlock / 32) + warp; i < n; i += gridDim.x * (kIcpBlock / 32)) {
@@ -69,36 +69,13 @@ __device__ __forceinline__ void icp_step_body(const NNView& tv, const float4* __
   }
   if (lane < kIcpSums) sm[warp][lane] = acc;
   __syncthreads();
+  double v = 0;
   if (threadIdx.x < kIcpSums) {
-    double v = 0;
 #pragma unroll
     for (int w = 0; w < kIcpBlock / 32; w++) v += sm[w][threadIdx.x];
-    partials[static_cast<size_t>(blockIdx.x) * kIcpSums + threadIdx.x] = v;
   }
-  __threadfence();
-  __syncthreads();
-  if (threadIdx.x == 0) is_last = atomicAdd(counter, 1u) == gridDim.x - 1;
-  __syncthreads();
-  if (is_last) {
-    // eight groups of 32 threads each add every eighth per-CTA row in CTA order, then the eight partial sums are added in
-    // group order: a fixed function of the grid size (reproducible), eight times shorter than one serial pass
-    __threadfence();
-    __shared__ double fin[kIcpBlock / 32][kIcpSums];
-    double v = 0;
-    if (lane < kIcpSums) {
-#pragma unroll 4
-      for (unsigned b = warp; b < gridDim.x; b += kIcpBlock / 32) v += __ldcg(partials + static_cast<size_t>(b) * kIcpSums + lane);
-      fin[warp][lane] = v;
-    }
-    __syncthreads();
-    v = 0;
-    if (threadIdx.x < kIcpSums) {
-#pragma unroll
-      for (int w = 0; w < kIcpBlock / 32; w++) v += fin[w][threadIdx.x];
-    }
-    if (threadIdx.x == 0) *counter = 0;
-    mailbox_publish<kIcpSums>(mb, v);
-  }
+  // eight groups of 32 threads fold the per-CTA rows, each with four loads in flight (reduce.cuh)
+  grid_finish<kIcpSums, kIcpBlock, 8, 4>(v, partials, counter, mb);
 }
 
 __global__ void __launch_bounds__(kIcpBlock) icp_step_kernel(const __grid_constant__ NNView tv, const float4* __restrict__ tgt, float4* __restrict__ cloud,

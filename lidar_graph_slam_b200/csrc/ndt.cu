@@ -23,6 +23,7 @@
 #include "keyframes.cuh"
 #include "math.cuh"
 #include "nn.cuh"
+#include "reduce.cuh"
 #include "sort.cuh"
 #include "voxel_common.cuh"
 
@@ -315,54 +316,6 @@ struct EvalParams {
 };
 
 constexpr int kEvalBlock = 128;
-constexpr int kNumAcc = 44;  // score, g[6], H[36], term count
-
-// block-wide sum of K doubles held per thread -> partials[blockIdx][k]; the last block to finish adds the
-// per-block partials in block order (fixed tree => run-to-run reproducible) and writes result[k].
-template <int K>
-__device__ __forceinline__ void block_reduce_and_finish(double (&acc)[K], double* __restrict__ partials, double* __restrict__ result,
-                                                       unsigned* __restrict__ counter, const Mailbox& mb) {
-  __shared__ double sm[kEvalBlock / 32][K];
-  __shared__ bool is_last;
-  const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
-#pragma unroll
-  for (int k = 0; k < K; k++) {
-    double v = acc[k];
-#pragma unroll
-    for (int off = 16; off > 0; off >>= 1) v += __shfl_xor_sync(0xffffffffu, v, off);
-    if (lane == 0) sm[warp][k] = v;
-  }
-  __syncthreads();
-  if (threadIdx.x < K) {
-    double v = 0;
-#pragma unroll
-    for (int w = 0; w < kEvalBlock / 32; w++) v += sm[w][threadIdx.x];
-    partials[static_cast<size_t>(blockIdx.x) * K + threadIdx.x] = v;
-  }
-  __threadfence();
-  __syncthreads();
-  if (threadIdx.x == 0) {
-    unsigned done = atomicAdd(counter, 1u);
-    is_last = (done == gridDim.x - 1);
-  }
-  __syncthreads();
-  if (is_last) {
-    __threadfence();
-    double v = 0;
-    if (threadIdx.x < K) {
-      for (unsigned b0 = 0; b0 < gridDim.x; b0 += 8) {  // eight independent loads in flight, added in block order
-        double t[8];
-#pragma unroll
-        for (int u = 0; u < 8; u++) t[u] = b0 + u < gridDim.x ? __ldcg(partials + static_cast<size_t>(b0 + u) * K + threadIdx.x) : 0.0;
-#pragma unroll
-        for (int u = 0; u < 8; u++) v += t[u];
-      }
-      result[threadIdx.x] = v;
-    }
-    if (threadIdx.x == 0) *counter = 0;  // re-arm for the next launch on this stream
-    mailbox_publish<K>(mb, v);
-  }
-}
 
 }  // namespace lgs
 
@@ -374,7 +327,7 @@ namespace lgs {
 // calculateScore (NDT:934-982)
 __global__ void __launch_bounds__(kEvalBlock) ndt_score_kernel(const float4* __restrict__ src, int n, EvalParams P, CellTable ct,
                                                              const double* __restrict__ vmean, const double* __restrict__ vicov, double gauss_d3,
-                                                             double* __restrict__ partials, double* __restrict__ result, unsigned* __restrict__ counter, const Mailbox mb) {
+                                                             double* __restrict__ partials, unsigned* __restrict__ counter, const Mailbox mb) {
   double acc[1] = {0.0};
   auto s3 = [](double a, double b, double c) { return a + (b + c); };
   for (int i = blockIdx.x * blockDim.x + threadIdx.x; i < n; i += gridDim.x * blockDim.x) {
@@ -403,7 +356,7 @@ __global__ void __launch_bounds__(kEvalBlock) ndt_score_kernel(const float4* __r
       acc[0] += score_inc / cnt;
     }
   }
-  block_reduce_and_finish<1>(acc, partials, result, counter, mb);
+  grid_finish<1, kEvalBlock, 1, 8>(cta_row<kEvalBlock>(acc), partials, counter, mb);  // rows in CTA order
 }
 
 }  // namespace lgs
@@ -432,8 +385,8 @@ struct lgs_ndt {
   int min_b[3] = {0, 0, 0}, max_b[3] = {0, 0, 0}, div_b[3] = {0, 0, 0};
   DevBuf table, hkeys, recs, ex_idx, ex_n, ex_mean, ex_cov, ex_icov, small, vsums;
   unsigned hmask = 0;
-  // reduction scratch
-  DevBuf partials, result;
+  // reduction scratch (reduce.cuh): the per-CTA rows and the arrival counter of the last-CTA pass
+  DevBuf partials, counter;
   // nearest-neighbour structure over the target for getFitnessScore (lazy)
   NNIndex nn;
   bool nn_ready = false;
@@ -854,11 +807,10 @@ void fill_eval_constants(lgs_ndt* n) {
 }
 
 int ensure_reduction_buffers(lgs_ndt* n, int grid) {
-  cudaStream_t st = n->ctx->stream;
   LGS_TRY(n->partials.reserve(static_cast<size_t>(std::max(grid, kNumSMs)) * (kRow + 8) * sizeof(double)));  // rows + LGS_DERIV_TRACE words
-  if (!n->result.p) {
-    LGS_TRY(n->result.reserve(kNumAcc * sizeof(double) + 64));
-    LGS_CUDA(cudaMemsetAsync(n->result.p, 0, kNumAcc * sizeof(double) + 64, st));
+  if (!n->counter.p) {
+    LGS_TRY(n->counter.reserve(sizeof(unsigned)));
+    LGS_CUDA(cudaMemsetAsync(n->counter.p, 0, sizeof(unsigned), n->ctx->stream));
   }
   return LGS_OK;
 }
@@ -880,8 +832,7 @@ int evaluate_launch(lgs_ndt* n, int mode, double* sums) {
   // one CTA per SM (fewer when the cloud has fewer rounds of 32 points than SMs)
   const int dgrid = std::max(1, std::min(kNumSMs, (ns + 31) / 32));
   LGS_TRY(ensure_reduction_buffers(n, dgrid));
-  double* result = n->result.as<double>();
-  unsigned* counter = reinterpret_cast<unsigned*>(result + kNumAcc);
+  unsigned* counter = n->counter.as<unsigned>();
   const CellTable ct = make_cell_table(n);
   const float4* src = n->source.as<float4>();
   const EvalParams& P = n->P;
@@ -899,7 +850,7 @@ int evaluate_launch(lgs_ndt* n, int mode, double* sums) {
     VoxelRec* rc = n->recs.as<VoxelRec>();
     const double *vm = n->ex_mean.as<double>(), *vc = n->ex_icov.as<double>();
     double* pt = n->partials.as<double>();
-#define LGS_LAUNCH(M, D) ndt_derivatives_kernel<M, D><<<dgrid, kDerivThreads, sizeof(DerivSmem), st>>>(src, ns, P, ct, rc, vm, vc, pt, result, counter, one2, mb)
+#define LGS_LAUNCH(M, D) ndt_derivatives_kernel<M, D><<<dgrid, kDerivThreads, sizeof(DerivSmem), st>>>(src, ns, P, ct, rc, vm, vc, pt, counter, one2, mb)
     if (mode == 0 && d7) LGS_LAUNCH(0, true);
     else if (mode == 0) LGS_LAUNCH(0, false);
     else if (mode == 1 && d7) LGS_LAUNCH(1, true);
@@ -1112,7 +1063,7 @@ void lgs_ndt_destroy(lgs_ndt* n) {
                     &n->roll_mcnt, &n->roll_seg, &n->roll_small, &n->roll_poses})
     b->release();
   for (DevBuf* b : {&n->target, &n->source, &n->out_cloud, &n->table, &n->hkeys, &n->recs, &n->ex_idx, &n->ex_n, &n->ex_mean, &n->ex_cov, &n->ex_icov,
-                    &n->small, &n->partials, &n->result, &n->vsums})
+                    &n->small, &n->partials, &n->counter, &n->vsums})
     b->release();
   n->nn.release();
   delete n;
@@ -1298,17 +1249,11 @@ int lgs_ndt_calculate_score(lgs_ndt* n, const float* T16, double* score) {
   fill_offsets(n->search, &P);
   if (!(n->refused || n->n_valid == 0)) {
     const int grid = eval_grid(n->n_source);
-    LGS_TRY(n->partials.reserve(static_cast<size_t>(grid) * kNumAcc * sizeof(double)));
-    if (!n->result.p) {
-      LGS_TRY(n->result.reserve(kNumAcc * sizeof(double) + 64));
-      LGS_CUDA(cudaMemsetAsync(n->result.p, 0, kNumAcc * sizeof(double) + 64, st));
-    }
-    double* result = n->result.as<double>();
-    unsigned* counter = reinterpret_cast<unsigned*>(result + kNumAcc);
+    LGS_TRY(ensure_reduction_buffers(n, grid));
     Mailbox mb;
     LGS_TRY(mailbox_next(ctx, &mb));
     ndt_score_kernel<<<grid, kEvalBlock, 0, st>>>(n->source.as<float4>(), static_cast<int>(n->n_source), P, make_cell_table(n),
-                                                 n->ex_mean.as<double>(), n->ex_icov.as<double>(), n->gauss_d3, n->partials.as<double>(), result, counter, mb);
+                                                 n->ex_mean.as<double>(), n->ex_icov.as<double>(), n->gauss_d3, n->partials.as<double>(), n->counter.as<unsigned>(), mb);
     ctx->launches++;
     LGS_CUDA(cudaGetLastError());
     LGS_TRY(mailbox_wait(ctx, mb, 1, score));
