@@ -466,7 +466,7 @@ typedef struct lgs_batch_params {
   int32_t max_iterations;         /* graph_based_slam.param.yaml */
   double transformation_epsilon;
   double max_correspondence_distance; /* GICP; <= 0 keeps FLT_MAX */
-  int32_t k_correspondences;      /* GICP */
+  int32_t k_correspondences;      /* GICP, GICP_OMP: at most 32; <= 0 keeps 20 */
   float ndt_resolution;           /* NDT */
   double ndt_step_size;
   float submap_leaf;              /* VoxelGrid leaf applied to each submap before setInputTarget (GBS:61: 0.5); <= 0 disables */

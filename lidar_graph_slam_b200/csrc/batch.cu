@@ -6,16 +6,14 @@
 // GPU of the box it was dealt to.
 #include <atomic>
 #include <chrono>
-#include <cstdio>
-#include <cstdlib>
 #include <limits>
 #include <mutex>
 #include <thread>
 #include <vector>
 
 #include "dist.cuh"
-#include "gicp.cuh"
-#include "keyframes.cuh"
+#include "matcher.cuh"
+#include "nn.cuh"
 #include "voxel_common.cuh"
 
 using namespace lgs;
@@ -49,34 +47,53 @@ struct BatchShared {
   std::string err;
 };
 
-// development aid: LGS_BATCH_TRACE=1 prints the host wall time of every stage of every pair (with a stream
-// synchronisation after each stage, so the numbers are not the production timeline)
-struct StageClock {
-  bool on;
-  cudaStream_t st;
-  std::chrono::steady_clock::time_point t0;
-  double ms[6] = {0, 0, 0, 0, 0, 0};
-  explicit StageClock(cudaStream_t s) : on(getenv("LGS_BATCH_TRACE") != nullptr), st(s) {
-    if (on) t0 = std::chrono::steady_clock::now();
+// Every call starts from the library defaults of the method, then the batch's settings.
+MatcherSettings batch_settings(const lgs_batch_params& bp) {
+  MatcherSettings s{};
+  s.k_correspondences = bp.k_correspondences > 0 ? bp.k_correspondences : 20;
+  s.max_optimizer_iterations = bp.max_optimizer_iterations > 0 ? bp.max_optimizer_iterations : 20;
+  s.euclidean_fitness_epsilon = bp.euclidean_fitness_epsilon != 0 ? bp.euclidean_fitness_epsilon : -std::numeric_limits<double>::max();
+  s.ndt_resolution = bp.ndt_resolution > 0 ? bp.ndt_resolution : 1.0f;
+  s.ndt_step_size = bp.ndt_step_size > 0 ? bp.ndt_step_size : 0.1;
+  switch (bp.method) {
+    case LGS_METHOD_GICP:  // fast_gicp.hpp / gicp_settings.hpp
+      s.max_iterations = bp.max_iterations > 0 ? bp.max_iterations : 64;
+      s.transformation_epsilon = bp.transformation_epsilon > 0 ? bp.transformation_epsilon : 5e-4;
+      s.max_correspondence_distance = bp.max_correspondence_distance > 0 ? bp.max_correspondence_distance
+                                                                         : static_cast<double>(std::numeric_limits<float>::max());
+      break;
+    case LGS_METHOD_ICP:  // PCL (GBS:145-148)
+      s.max_iterations = bp.max_iterations > 0 ? bp.max_iterations : 10;
+      s.transformation_epsilon = bp.transformation_epsilon > 0 ? bp.transformation_epsilon : 0.0;
+      s.max_correspondence_distance = bp.max_correspondence_distance > 0 ? bp.max_correspondence_distance : 1.3407807929942596e154;
+      break;
+    case LGS_METHOD_GICP_OMP:  // gicp_omp.h:116-126 (GBS:134-137)
+      s.max_iterations = bp.max_iterations > 0 ? bp.max_iterations : 200;
+      s.transformation_epsilon = bp.transformation_epsilon > 0 ? bp.transformation_epsilon : 5e-4;
+      s.max_correspondence_distance = bp.max_correspondence_distance > 0 ? bp.max_correspondence_distance : 5.0;
+      break;
+    default:  // NDT
+      s.max_iterations = bp.max_iterations > 0 ? bp.max_iterations : 35;
+      s.transformation_epsilon = bp.transformation_epsilon > 0 ? bp.transformation_epsilon : 0.1;
   }
-  void lap(int k) {
-    if (!on) return;
-    cudaStreamSynchronize(st);
-    const auto t1 = std::chrono::steady_clock::now();
-    ms[k] = std::chrono::duration<double, std::milli>(t1 - t0).count();
-    t0 = t1;
-  }
-};
+  return s;
+}
 
-int run_pair(lgs_ctx* ctx, lgs_gicp* gicp, lgs_ndt* ndt, lgs_icp* icp, lgs_gicp_omp* gomp, DevBuf* sub_raw, DevBuf* sub_ds, DevBuf* scan_buf, BatchShared* S, int64_t i) {
+// The checks of the batch's parameters that the four entry points share.  They run before any worker starts, so a
+// refused call verifies no pair and writes no record.
+int check_batch_params(const lgs_batch_params* bp) {
+  LGS_REQUIRE(bp->method >= LGS_METHOD_NDT && bp->method <= LGS_METHOD_GICP_OMP, "unknown method");
+  LGS_REQUIRE(bp->k_correspondences <= kMaxK || (bp->method != LGS_METHOD_GICP && bp->method != LGS_METHOD_GICP_OMP),
+              "k_correspondences must be <= 32 (<= 0 keeps the default)");
+  return LGS_OK;
+}
+
+int run_pair(lgs_ctx* ctx, Matcher& m, DevBuf* sub_raw, DevBuf* sub_ds, DevBuf* scan_buf, BatchShared* S, int64_t i) {
   const lgs_batch_params& bp = *S->bp;
   lgs_align_result& rec = S->records[i];
   memset(&rec, 0, sizeof(rec));
-  StageClock clk(ctx->stream);
   // submap -> (optional) VoxelGrid -> device-resident target
   int64_t n_tgt = 0;
-  const float* scan_dev = nullptr;  // key-frame mode: the scan is a device cloud as well
-  int64_t n_scan_dev = 0;
   if (S->kf) {
     // GBS:297-309: key frames min_id - K .. min_id + K that exist, ascending; GBS:247-251: the scan in the map frame
     std::vector<int32_t> ids;
@@ -90,7 +107,6 @@ int run_pair(lgs_ctx* ctx, lgs_gicp* gicp, lgs_ndt* ndt, lgs_icp* icp, lgs_gicp_
     LGS_TRY(upload_cloud(ctx, S->submaps[i], S->n_submap[i], S->stride, sub_raw));
     n_tgt = S->n_submap[i];
   }
-  clk.lap(0);
   const float* tgt_dev = sub_raw->as<float>();
   if (bp.submap_leaf > 0 && n_tgt > 0) {
     LGS_TRY(sub_ds->reserve(static_cast<size_t>(n_tgt) * 16));
@@ -100,81 +116,22 @@ int run_pair(lgs_ctx* ctx, lgs_gicp* gicp, lgs_ndt* ndt, lgs_icp* icp, lgs_gicp_
     tgt_dev = sub_ds->as<float>();
     n_tgt = info.n_out;
   }
-  clk.lap(1);
-  if (S->kf) {
-    // into the worker's own buffer: setInputTarget may voxelise at once and use every scratch arena of the context
-    LGS_TRY(keyframes_assemble_into(S->kf, ctx, S->scan_ids + i, 1, &ctx->tmp[2], scan_buf, &n_scan_dev));
-    scan_dev = scan_buf->as<float>();
-  }
-  const float* guess = S->guesses ? S->guesses + 16 * i : nullptr;
-  const int32_t pair_id = S->pair_ids ? S->pair_ids[i] : S->pair_id0 + static_cast<int32_t>(i);
+  // key-frame mode: the scan into the worker's own buffer; setInputTarget may voxelise at once and use every scratch
+  // arena of the context
+  int64_t n_scan_dev = 0;
+  if (S->kf) LGS_TRY(keyframes_assemble_into(S->kf, ctx, S->scan_ids + i, 1, &ctx->tmp[2], scan_buf, &n_scan_dev));
+  LGS_TRY(m.set_target_dev(tgt_dev, n_tgt));
+  LGS_TRY(S->kf ? m.set_source_dev(scan_buf->as<float>(), n_scan_dev) : m.set_source(S->scans[i], S->n_scan[i], S->stride));
+  LGS_TRY(m.reset_between_problems());
+  LGS_TRY(m.align(S->guesses ? S->guesses + 16 * i : nullptr, &rec));
   // arms the one-shot record sink of this context: the fitness kernel that follows completes and stores the record
-  auto arm_record = [&]() {
-    rec.pair_id = pair_id;
-    if (S->rec_dev) {
-      ctx->rec_out_proto = rec;
-      ctx->rec_out_dev = S->rec_dev + i;
-    }
-  };
-  const double max_range = bp.fitness_max_range > 0 ? bp.fitness_max_range : std::numeric_limits<double>::max();
-  if (bp.method == LGS_METHOD_GICP) {
-    LGS_TRY(lgs_gicp_set_target_dev(gicp, tgt_dev, n_tgt));
-    clk.lap(2);
-    if (scan_dev)
-      LGS_TRY(lgs_gicp_set_source_dev(gicp, scan_dev, n_scan_dev));
-    else
-      LGS_TRY(lgs_gicp_set_source(gicp, S->scans[i], S->n_scan[i], S->stride));
-    clk.lap(3);
-    LGS_TRY(lgs_gicp_align(gicp, guess, &rec, nullptr));
-    clk.lap(4);
-    arm_record();
-    LGS_TRY(lgs_gicp_fitness(gicp, max_range, &rec.fitness));
-    clk.lap(5);
-  } else if (bp.method == LGS_METHOD_ICP) {
-    LGS_TRY(lgs_icp_set_target_dev(icp, tgt_dev, n_tgt));
-    clk.lap(2);
-    if (scan_dev)
-      LGS_TRY(lgs_icp_set_source_dev(icp, scan_dev, n_scan_dev));
-    else
-      LGS_TRY(lgs_icp_set_source(icp, S->scans[i], S->n_scan[i], S->stride));
-    clk.lap(3);
-    LGS_TRY(lgs_icp_reset_convergence_criteria(icp));  // every pair starts from a fresh criteria object (order independence)
-    LGS_TRY(lgs_icp_align(icp, guess, &rec, nullptr));
-    clk.lap(4);
-    arm_record();
-    LGS_TRY(lgs_icp_fitness(icp, max_range, &rec.fitness));
-    clk.lap(5);
-  } else if (bp.method == LGS_METHOD_GICP_OMP) {
-    LGS_TRY(lgs_gicp_omp_set_target_dev(gomp, tgt_dev, n_tgt));
-    clk.lap(2);
-    if (scan_dev)
-      LGS_TRY(lgs_gicp_omp_set_source_dev(gomp, scan_dev, n_scan_dev));
-    else
-      LGS_TRY(lgs_gicp_omp_set_source(gomp, S->scans[i], S->n_scan[i], S->stride));
-    clk.lap(3);
-    LGS_TRY(lgs_gicp_omp_align(gomp, guess, &rec, nullptr));
-    clk.lap(4);
-    arm_record();
-    LGS_TRY(lgs_gicp_omp_fitness(gomp, max_range, &rec.fitness));
-    clk.lap(5);
-  } else {
-    LGS_TRY(lgs_ndt_set_target_dev(ndt, tgt_dev, n_tgt));
-    clk.lap(2);
-    if (scan_dev)
-      LGS_TRY(lgs_ndt_set_source_dev(ndt, scan_dev, n_scan_dev));
-    else
-      LGS_TRY(lgs_ndt_set_source(ndt, S->scans[i], S->n_scan[i], S->stride));
-    clk.lap(3);
-    LGS_TRY(lgs_ndt_align(ndt, guess, &rec, nullptr));
-    clk.lap(4);
-    arm_record();
-    LGS_TRY(lgs_ndt_fitness(ndt, max_range, &rec.fitness));
-    clk.lap(5);
+  rec.pair_id = S->pair_ids ? S->pair_ids[i] : S->pair_id0 + static_cast<int32_t>(i);
+  if (S->rec_dev) {
+    ctx->rec_out_proto = rec;
+    ctx->rec_out_dev = S->rec_dev + i;
   }
-  if (clk.on)
-    fprintf(stderr, "[lgs batch] pair %lld: upload %.2f  voxelgrid %.2f  set_target %.2f  set_source %.2f  align %.2f  fitness %.2f ms (target %lld pts)\n",
-            static_cast<long long>(i), clk.ms[0], clk.ms[1], clk.ms[2], clk.ms[3], clk.ms[4], clk.ms[5], static_cast<long long>(n_tgt));
-  rec.pair_id = pair_id;
+  const double max_range = bp.fitness_max_range > 0 ? bp.fitness_max_range : std::numeric_limits<double>::max();
+  LGS_TRY(m.fitness(max_range, &rec.fitness));
   return LGS_OK;
 }
 
@@ -184,10 +141,7 @@ int run_pair(lgs_ctx* ctx, lgs_gicp* gicp, lgs_ndt* ndt, lgs_icp* icp, lgs_gicp_
 struct WorkerSlot {
   int device = -1;
   lgs_ctx* ctx = nullptr;
-  lgs_gicp* gicp = nullptr;
-  lgs_ndt* ndt = nullptr;
-  lgs_icp* icp = nullptr;
-  lgs_gicp_omp* gomp = nullptr;
+  Matcher matchers[4];  // by LGS_METHOD_*, created on first use
   DevBuf sub_raw, sub_ds, scan_buf;
   void destroy() {
     if (ctx) {
@@ -197,16 +151,9 @@ struct WorkerSlot {
     sub_raw.release();
     sub_ds.release();
     scan_buf.release();
-    if (gicp) lgs_gicp_destroy(gicp);
-    if (ndt) lgs_ndt_destroy(ndt);
-    if (icp) lgs_icp_destroy(icp);
-    if (gomp) lgs_gicp_omp_destroy(gomp);
+    for (Matcher& m : matchers) m.destroy();
     if (ctx) lgs_ctx_destroy(ctx);
     ctx = nullptr;
-    gicp = nullptr;
-    ndt = nullptr;
-    icp = nullptr;
-    gomp = nullptr;
   }
 };
 
@@ -238,49 +185,13 @@ void worker(BatchShared* S) {
   if (!w->ctx) rc = lgs_ctx_create(S->device, nullptr, &w->ctx);
   if (rc == LGS_OK) w->ctx->polite_wait = true;
   if (rc == LGS_OK) rc = use_device(w->ctx);
-  if (rc == LGS_OK) {
-    if (bp.method == LGS_METHOD_GICP) {
-      if (!w->gicp) rc = lgs_gicp_create(w->ctx, &w->gicp);
-      if (rc == LGS_OK) {
-        // every call starts from the library defaults (fast_gicp.hpp / gicp_settings.hpp), then the batch's settings
-        lgs_gicp_set_correspondence_randomness(w->gicp, bp.k_correspondences > 0 ? bp.k_correspondences : 20);
-        lgs_gicp_set_maximum_iterations(w->gicp, bp.max_iterations > 0 ? bp.max_iterations : 64);
-        lgs_gicp_set_transformation_epsilon(w->gicp, bp.transformation_epsilon > 0 ? bp.transformation_epsilon : 5e-4);
-        lgs_gicp_set_max_correspondence_distance(w->gicp, bp.max_correspondence_distance > 0 ? bp.max_correspondence_distance
-                                                                                              : static_cast<double>(std::numeric_limits<float>::max()));
-      }
-    } else if (bp.method == LGS_METHOD_ICP) {
-      if (!w->icp) rc = lgs_icp_create(w->ctx, &w->icp);
-      if (rc == LGS_OK) {  // PCL defaults, then the batch's settings (GBS:145-148)
-        lgs_icp_set_maximum_iterations(w->icp, bp.max_iterations > 0 ? bp.max_iterations : 10);
-        lgs_icp_set_transformation_epsilon(w->icp, bp.transformation_epsilon > 0 ? bp.transformation_epsilon : 0.0);
-        lgs_icp_set_max_correspondence_distance(w->icp, bp.max_correspondence_distance > 0 ? bp.max_correspondence_distance : 1.3407807929942596e154);
-        lgs_icp_set_euclidean_fitness_epsilon(w->icp, bp.euclidean_fitness_epsilon != 0 ? bp.euclidean_fitness_epsilon : -std::numeric_limits<double>::max());
-        lgs_icp_set_transformation_rotation_epsilon(w->icp, 0.0);
-      }
-    } else if (bp.method == LGS_METHOD_GICP_OMP) {
-      if (!w->gomp) rc = lgs_gicp_omp_create(w->ctx, &w->gomp);
-      if (rc == LGS_OK) {  // gicp_omp.h:116-126 defaults, then the batch's settings (GBS:134-137)
-        lgs_gicp_omp_set_correspondence_randomness(w->gomp, bp.k_correspondences > 0 ? bp.k_correspondences : 20);
-        lgs_gicp_omp_set_maximum_iterations(w->gomp, bp.max_iterations > 0 ? bp.max_iterations : 200);
-        lgs_gicp_omp_set_transformation_epsilon(w->gomp, bp.transformation_epsilon > 0 ? bp.transformation_epsilon : 5e-4);
-        lgs_gicp_omp_set_max_correspondence_distance(w->gomp, bp.max_correspondence_distance > 0 ? bp.max_correspondence_distance : 5.0);
-        lgs_gicp_omp_set_maximum_optimizer_iterations(w->gomp, bp.max_optimizer_iterations > 0 ? bp.max_optimizer_iterations : 20);
-      }
-    } else {
-      if (!w->ndt) rc = lgs_ndt_create(w->ctx, &w->ndt);
-      if (rc == LGS_OK) {
-        lgs_ndt_set_resolution(w->ndt, bp.ndt_resolution > 0 ? bp.ndt_resolution : 1.0f);
-        lgs_ndt_set_step_size(w->ndt, bp.ndt_step_size > 0 ? bp.ndt_step_size : 0.1);
-        lgs_ndt_set_maximum_iterations(w->ndt, bp.max_iterations > 0 ? bp.max_iterations : 35);
-        lgs_ndt_set_transformation_epsilon(w->ndt, bp.transformation_epsilon > 0 ? bp.transformation_epsilon : 0.1);
-      }
-    }
-  }
+  Matcher& m = w->matchers[bp.method];
+  if (rc == LGS_OK && m.method < 0) rc = m.create(w->ctx, bp.method);
+  if (rc == LGS_OK) rc = m.configure(batch_settings(bp));
   while (rc == LGS_OK && !S->failed.load()) {
     const int64_t i = S->next.fetch_add(1);
     if (i >= S->n_pairs) break;
-    rc = run_pair(w->ctx, w->gicp, w->ndt, w->icp, w->gomp, &w->sub_raw, &w->sub_ds, &w->scan_buf, S, i);
+    rc = run_pair(w->ctx, m, &w->sub_raw, &w->sub_ds, &w->scan_buf, S, i);
   }
   if (rc != LGS_OK) {
     std::lock_guard<std::mutex> lk(S->err_mu);
@@ -308,7 +219,7 @@ extern "C" int lgs_batch_align(int device, void* cuda_stream, const lgs_batch_pa
   LGS_NVTX("lgs_batch_align");
   LGS_REQUIRE(params && records, "null argument");
   LGS_REQUIRE(n_pairs >= 0, "negative pair count");
-  LGS_REQUIRE(params->method >= LGS_METHOD_NDT && params->method <= LGS_METHOD_GICP_OMP, "unknown method");
+  LGS_TRY(check_batch_params(params));
   LGS_REQUIRE(n_pairs == 0 || (scans && n_scan && submaps && n_submap), "null pair arrays");
   BatchShared S;
   S.bp = params;
@@ -336,7 +247,7 @@ extern "C" int lgs_batch_align_keyframes(lgs_keyframes* kf, void* cuda_stream, c
   LGS_NVTX("lgs_batch_align_keyframes");
   LGS_REQUIRE(kf && params && records, "null argument");
   LGS_REQUIRE(n_pairs >= 0 && search_key_frame_num >= 0, "negative count");
-  LGS_REQUIRE(params->method >= LGS_METHOD_NDT && params->method <= LGS_METHOD_GICP_OMP, "unknown method");
+  LGS_TRY(check_batch_params(params));
   LGS_REQUIRE(n_pairs == 0 || (scan_ids && center_ids), "null pair arrays");
   const int64_t count = keyframes_count(kf);
   for (int64_t i = 0; i < n_pairs; i++)
@@ -451,7 +362,7 @@ extern "C" int lgs_batch_align_keyframes_dist(lgs_keyframes* kf, lgs_comm* comm,
   LGS_NVTX("lgs_batch_align_keyframes_dist");
   LGS_REQUIRE(kf && comm && params && (records_all || n_pairs == 0), "null argument");
   LGS_REQUIRE(n_pairs >= 0 && n_pairs < (int64_t(1) << 31) && search_key_frame_num >= 0, "count out of range");
-  LGS_REQUIRE(params->method >= LGS_METHOD_NDT && params->method <= LGS_METHOD_GICP_OMP, "unknown method");
+  LGS_TRY(check_batch_params(params));
   LGS_REQUIRE(n_pairs == 0 || (scan_ids && center_ids), "null pair arrays");
   const int64_t count = keyframes_count(kf);
   std::vector<int64_t> sizes(static_cast<size_t>(n_pairs));
@@ -493,7 +404,7 @@ extern "C" int lgs_batch_align_dist(lgs_comm* comm, const lgs_batch_params* para
   LGS_NVTX("lgs_batch_align_dist");
   LGS_REQUIRE(comm && params && (records_all || n_pairs == 0), "null argument");
   LGS_REQUIRE(n_pairs >= 0 && n_pairs < (int64_t(1) << 31), "count out of range");
-  LGS_REQUIRE(params->method >= LGS_METHOD_NDT && params->method <= LGS_METHOD_GICP_OMP, "unknown method");
+  LGS_TRY(check_batch_params(params));
   LGS_REQUIRE(n_pairs == 0 || (scans && n_scan && submaps && n_submap), "null pair arrays");
   std::vector<int64_t> sizes(static_cast<size_t>(n_pairs));
   for (int64_t i = 0; i < n_pairs; i++) sizes[static_cast<size_t>(i)] = n_scan[i] + n_submap[i];

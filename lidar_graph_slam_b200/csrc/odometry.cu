@@ -4,7 +4,7 @@
 //   -> base_from_sensor (transform_cloud, the transform_pcl arithmetic of the key-frame assembly)
 //   -> setInputSource + align(pose after the previous frame) -> key-frame test on the host
 //   -> on a key frame: push into the device key-frame array and rebuild the target from the newest window
-//      (NDT: the incremental lgs_ndt_set_target_keyframes; GICP: assemble + set_target_dev).
+//      (Matcher::set_target_keyframes: incremental for NDT, assemble + set_target_dev for GICP).
 // The host reads only what the loop decides on: the align's record.  A sequence is one problem per GPU (the NDT align is
 // a cooperative launch over every SM), so the sequences of one rank run one after another; lgs_odometry_run_dist deals
 // whole sequences to the ranks and gathers the records once.
@@ -15,7 +15,7 @@
 #include <vector>
 
 #include "dist.cuh"
-#include "keyframes.cuh"
+#include "matcher.cuh"
 #include "voxel_common.cuh"
 
 using namespace lgs;
@@ -83,67 +83,6 @@ int validate(lgs_ctx* ctx, const lgs_odometry_params* params, int32_t n_seq, con
   for (int a = 0; a < 16; a++) r.extrinsic[a] = zero ? ((a % 5) == 0 ? 1.0f : 0.0f) : p.base_from_sensor[a];
   return LGS_OK;
 }
-
-// The registration object of one sequence, created fresh so that no state crosses from one sequence to the next.
-struct Registration {
-  lgs_ctx* ctx;
-  int method;
-  lgs_ndt* ndt = nullptr;
-  lgs_gicp* gicp = nullptr;
-  lgs_gicp_omp* gomp = nullptr;
-  DevBuf target, poses;
-
-  Registration(lgs_ctx* c, int m) : ctx(c), method(m) {}
-  ~Registration() {
-    if (ndt) lgs_ndt_destroy(ndt);
-    if (gicp) lgs_gicp_destroy(gicp);
-    if (gomp) lgs_gicp_omp_destroy(gomp);
-    target.release();
-    poses.release();
-  }
-  int create(const lgs_odometry_params& p) {
-    if (method == LGS_METHOD_NDT) {  // LSM:56-72
-      LGS_TRY(lgs_ndt_create(ctx, &ndt));
-      LGS_TRY(lgs_ndt_set_resolution(ndt, p.ndt_resolution));
-      LGS_TRY(lgs_ndt_set_step_size(ndt, p.ndt_step_size));
-      LGS_TRY(lgs_ndt_set_transformation_epsilon(ndt, p.transformation_epsilon));
-      LGS_TRY(lgs_ndt_set_maximum_iterations(ndt, p.max_iterations));
-    } else if (method == LGS_METHOD_GICP) {  // LSM:38-54
-      LGS_TRY(lgs_gicp_create(ctx, &gicp));
-      LGS_TRY(lgs_gicp_set_correspondence_randomness(gicp, p.k_correspondences));
-      LGS_TRY(lgs_gicp_set_max_correspondence_distance(gicp, p.max_correspondence_distance));
-      LGS_TRY(lgs_gicp_set_transformation_epsilon(gicp, p.transformation_epsilon));
-      LGS_TRY(lgs_gicp_set_maximum_iterations(gicp, p.max_iterations));
-    } else {  // LSM:73-96
-      LGS_TRY(lgs_gicp_omp_create(ctx, &gomp));
-      LGS_TRY(lgs_gicp_omp_set_correspondence_randomness(gomp, p.k_correspondences));
-      LGS_TRY(lgs_gicp_omp_set_max_correspondence_distance(gomp, p.max_correspondence_distance));
-      LGS_TRY(lgs_gicp_omp_set_transformation_epsilon(gomp, p.transformation_epsilon));
-      LGS_TRY(lgs_gicp_omp_set_maximum_iterations(gomp, p.max_iterations));
-      LGS_TRY(lgs_gicp_omp_set_maximum_optimizer_iterations(gomp, p.max_optimizer_iterations));
-    }
-    return LGS_OK;
-  }
-  int set_source(const float4* pts, int64_t n) {
-    const float* f = reinterpret_cast<const float*>(pts);
-    if (ndt) return lgs_ndt_set_source_dev(ndt, f, n);
-    if (gicp) return lgs_gicp_set_source_dev(gicp, f, n);
-    return lgs_gicp_omp_set_source_dev(gomp, f, n);
-  }
-  int align(const float* guess, lgs_align_result* r) {
-    if (ndt) return lgs_ndt_align(ndt, guess, r, nullptr);
-    if (gicp) return lgs_gicp_align(gicp, guess, r, nullptr);
-    return lgs_gicp_omp_align(gomp, guess, r, nullptr);
-  }
-  // LSM:199-212 without caching on identity (Appendix A #9): the target is rebuilt from the window on every change
-  int set_target(lgs_keyframes* kf, const std::vector<int32_t>& ids) {
-    if (ndt) return lgs_ndt_set_target_keyframes(ndt, kf, ids.data(), static_cast<int32_t>(ids.size()), nullptr);
-    int64_t n = 0;
-    LGS_TRY(keyframes_assemble_into(kf, ctx, ids.data(), static_cast<int32_t>(ids.size()), &poses, &target, &n));
-    if (gicp) return lgs_gicp_set_target_dev(gicp, target.as<float>(), n);
-    return lgs_gicp_omp_set_target_dev(gomp, target.as<float>(), n);
-  }
-};
 
 // Where the frames come from.  Device form: the caller's packed clouds.  Host form: two pinned staging buffers and two
 // device buffers on a copy stream; frame k+1 is copied while frame k aligns, ordered by events in both directions.
@@ -311,7 +250,7 @@ struct Driver {
   }
 
   // a key frame (LSM:183-212): the base-frame cloud with pose T, its path length and f64 position, then the target window
-  int add_keyframe(Registration& reg, lgs_keyframes* kf, bool shared_stream, const float* T, double accum, int32_t* id) {
+  int add_keyframe(Matcher& reg, lgs_keyframes* kf, bool shared_stream, const float* T, double accum, int32_t* id) {
     if (!shared_stream) LGS_CUDA(cudaStreamSynchronize(ctx->stream));  // `base` is complete before the array's stream copies it
     LGS_TRY(lgs_keyframes_push_dev(kf, base.as<float>(), base_n, T, id));
     if (!shared_stream) LGS_TRY(keyframes_wait_resident(kf));  // and copied before ctx's stream reuses `base`
@@ -320,7 +259,7 @@ struct Driver {
     LGS_TRY(lgs_keyframes_set_position(kf, *id, pos));
     std::vector<int32_t> ids;
     for (int32_t k = *id; k >= 0 && k > *id - P.p.max_scan_accumulate_num; k--) ids.push_back(k);  // newest first
-    return reg.set_target(kf, ids);
+    return reg.set_target_keyframes(kf, ids);  // LSM:199-212 without caching on identity (Appendix A #9)
   }
 
   int64_t base_n = 0;
@@ -339,8 +278,12 @@ struct Driver {
         if (k) lgs_keyframes_destroy(k);
       }
     } free_scratch{scratch};
-    Registration reg(ctx, P.p.method);  // destroyed before the scratch array its NDT target refers to
-    LGS_TRY(reg.create(P.p));
+    Matcher reg;  // created fresh so that no state crosses from one sequence to the next, and destroyed before the scratch
+                  // array its NDT target refers to
+    LGS_TRY(reg.create(ctx, P.p.method));
+    const lgs_odometry_params& p = P.p;  // NDT LSM:56-72, FastGICP LSM:38-54, pclomp GICP LSM:73-96
+    LGS_TRY(reg.configure({p.max_iterations, p.transformation_epsilon, p.max_correspondence_distance, p.k_correspondences, p.ndt_resolution,
+                           p.ndt_step_size, p.max_optimizer_iterations, 0.0}));
     // the array runs its copies on its own context's stream; with a context of its own it is synchronised around a push
     const bool shared_stream = keyframes_stream(kf) == ctx->stream;
     float T[16], T_kf[16];
@@ -370,7 +313,7 @@ struct Driver {
         r.converged = 1;
         keyframe = true;
       } else {
-        LGS_TRY(reg.set_source(base.as<float4>(), base_n));  // LSM:162
+        LGS_TRY(reg.set_source_dev(base.as<float>(), base_n));  // LSM:162
         lgs_align_result a;
         LGS_TRY(reg.align(T, &a));  // LSM:165, guess = the pose after the previous frame
         timer.mark(2);

@@ -1335,6 +1335,12 @@ def test_batch_loop_closure_from_keyframe_array(api, oracle):
     assert list(a[0].T) == list(b[0].T) and a[0].fitness == b[0].fitness
     with pytest.raises(RuntimeError):
         kf.batch_align([n_kf], [0])
+    # the GICP methods take at most 32 neighbours: a larger k fails the call instead of running with the k a worker had
+    for method in (api.METHOD_GICP, api.METHOD_GICP_OMP):
+        with pytest.raises(RuntimeError, match="k_correspondences"):
+            kf.batch_align(d["scan_ids"], d["center_ids"], search_key_frame_num=K, method=method, k_correspondences=33)
+        with pytest.raises(RuntimeError, match="k_correspondences"):
+            api.batch_align(scans, submaps, method=method, k_correspondences=33)
     # candidate search: key frames along a loop, 2 m apart, the latest one back near the start
     loop = api.KeyFrameArray()
     pts = d["clouds"][0][:100]
